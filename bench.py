@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- scaffolds/s binned (feature build + split search) on N B200s, with roofline and CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaffolds S --samples M --genomes G]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--scaffolds S --samples M --genomes G] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one synthetic metagenome: pack -> windows -> k-mer signature ->
 per-sample coverage -> split search down to the final bins.  At N=1 the workload is BASELINE.json configs[1]
@@ -19,6 +19,9 @@ search is sharded by dimension (abw_search_run_sharded: all-gather of per-cluste
           drop-in command lines of this repo on the same text files (e2e_cli)
 
 `--impl reference` times only that reference arm (rank 0; other ranks exit 0).
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of the resident path handed its caller (rank 0's) as DIR/<name>.npy in
+float64, so that two builds can be compared output for output on the same seeded inputs (see dump_outputs()).
 """
 import argparse
 import gc
@@ -257,6 +260,38 @@ FEATURE_FAMILIES = {
     "coverage": ("k_cov_",),
 }
 
+DUMP_LIMIT_BYTES = 64_000_000
+CLUSTER_FIELDS = ("id", "parent", "ndps", "nscafs", "split", "best.found", "best.dim", "best.value", "best.a", "best.b", "best.legal", "child1", "child2",
+                  "child1_ndps", "child2_ndps", "child1_nscafs", "child2_nscafs", "child1_raw", "child2_raw", "total_size", "scg_unique", "scg_avg",
+                  "gc_avg", "gc_sd", "cvg_avg", "cvg_sd")
+
+
+def cluster_table(recs):
+    """Cluster records as float64 [clusters][CLUSTER_FIELDS] (every integer field stays below 2**53, so the conversion is exact)."""
+    def field(r, name):
+        for part in name.split("."):
+            r = getattr(r, part)
+        return float(r)
+    return np.array([[field(r, f) for f in CLUSTER_FIELDS] for r in recs], dtype=np.float64).reshape(-1, len(CLUSTER_FIELDS))
+
+
+def dump_outputs(directory, arrays, seed=0):
+    """Writes every array as <directory>/<name>.npy in float64, DUMP_LIMIT_BYTES in all.  An array larger than its share is replaced by the rows of a
+    fixed, seeded sample (the same rows for the same shape), whose row numbers go beside it as <name>_rows.npy."""
+    os.makedirs(directory, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // (2 * len(arrays)) - 4096          # room for an array, its row numbers and two .npy headers
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        rows_path = os.path.join(directory, f"{name}_rows.npy")
+        if a.nbytes > share:
+            k = max(1, share // (a.nbytes // a.shape[0]))
+            rows = np.sort(np.random.default_rng(seed).choice(a.shape[0], k, replace=False))
+            np.save(rows_path, rows.astype(np.float64))
+            a = a[rows]
+        elif os.path.exists(rows_path):
+            os.remove(rows_path)
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+
 
 def main():
     ap = argparse.ArgumentParser()
@@ -270,7 +305,10 @@ def main():
     ap.add_argument("--coverage-scale", type=float, default=1.0, help="multiplies the read depth of the synthetic samples (large shapes: thinned reads)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="N > 1: skip the one-off comparison of the sharded search with the single-rank search")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -442,7 +480,7 @@ def main():
         state["exchange_path"] = "peer memory (abw_scatter_columns_milli)" if use_peer else "NCCL all-to-all"
         return dict(full=full, full_ptr=full_ptr, total_rows=total_rows, off=off, cnt=cnt, T_all=T_all, keep_all=keep_all, rows_per_rank=rows_per_rank, local=local64)
 
-    def step(resident, timings=None, on_features=None, keep_exchange=False):
+    def step(resident, timings=None, on_features=None, keep_exchange=False, keep_features=False):
         if resident:
             fb = pipeline.build_features(ctx, d_seq, mg.offsets, d_reads, this_sample=0, seq_on_device=True, reads_on_device=True, nreads=nreads, timings=timings)
         else:
@@ -473,6 +511,7 @@ def main():
             ndps_total = int(res.dp2cluster.size)
         else:
             x = exchange(fb, counts, timings, keep_doubles=keep_exchange)
+            kept = x["keep_all"]
             # dimension-sharded search: this rank sweeps columns [off, off+cnt) of every datapoint
             if isinstance(x["keep_all"], slice):
                 len_kept, mask_kept = lengths_all, masks_all
@@ -502,11 +541,11 @@ def main():
             if fb.milli_inexact():
                 raise SystemExit("bench.py: a feature value is not a multiple of 0.001")
         state.update(ndps=ndps_total, nseg=fb.nseg, ncols=fb.ncols, prof=res.profile, nclusters=len(res.recs), nbins=nbins,
-                     bins=res.scaf2cluster, res=res)
+                     bins=res.scaf2cluster, res=res, kept=kept)
         if timings is not None:                        # window lengths: only needed for the algorithmic byte count of the k-mer kernel
             sg = fb.segments_host()
             state["seg_len"] = sg["seg_end"] - sg["seg_start"] + 1
-        if keep_exchange:
+        if keep_exchange or keep_features:
             state["fb"] = fb
         else:
             fb.close()
@@ -520,7 +559,8 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(resident, steps):
+    def timed(resident, steps, keep_last=False):
+        """keep_last: the feature build of the last step stays open (state["fb"]) for last_step_outputs()."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = ctx.launches
@@ -531,7 +571,7 @@ def main():
         host = []
         for i in range(steps):
             m0, h0 = ctx.arena_misses, time.perf_counter()
-            step(resident)
+            step(resident, keep_features=keep_last and i == steps - 1)
             host.append((round(1000.0 * (time.perf_counter() - h0), 3), ctx.arena_misses - m0))
             marks[i].record(ext)
         e1.record(ext)
@@ -545,6 +585,21 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         state["host_ms_and_driver_allocations_" + ("resident" if resident else "e2e")] = host
         return float(t.item()), ctx.launches - l0, per_step
+
+    def last_step_outputs():
+        """What the last step handed its caller: the feature build (window table, .lrn matrix) and the split search (cluster records, bin of every
+        datapoint and of every scaffold it kept, with the assembly index of those scaffolds).  Copied before the next step reuses the buffers."""
+        fb, res, kept = state.pop("fb"), state["res"], state["kept"]
+        if isinstance(kept, slice):                    # N > 1, no scaffold dropped
+            kept = np.arange(world * nscaf)
+        elif kept.dtype == bool:
+            kept = np.nonzero(kept)[0]
+        sg = fb.segments_host()
+        out = {"windows": np.stack([sg[k].astype(np.float64) for k in ("seg_scaf", "seg_start", "seg_end", "seg_nonN")], axis=1),
+               "features": fb.rows_host(), "clusters": cluster_table(res.recs), "dp2cluster": res.dp2cluster.astype(np.float64),
+               "scaf2cluster": res.scaf2cluster.astype(np.float64), "kept_scaffolds": kept.astype(np.float64)}
+        fb.close()
+        return out
 
     def verify_sharded():
         """Once, outside the timed region: the NCCL-sharded search of this run against the single-rank search of the SAME gathered problem on rank 0 --
@@ -587,12 +642,17 @@ def main():
             raise SystemExit("bench.py: the sharded search differs from the single-rank search")
         step(True)                                     # the verification gathered whole matrices: one more untimed step so that the block caches hold the step's shapes again
     n_warm_samples = len(sampler.rows)                 # samples before this index were taken during the warm-up (same load)
-    ms_res, launches, steps_res = timed(True, args.steps)
+    ms_res, launches, steps_res = timed(True, args.steps, keep_last=bool(args.dump_outputs))
     timed_rows = sampler.rows[n_warm_samples:]
     if len(timed_rows) >= 2:                           # enough samples inside the timed region itself; else keep the warm-up samples (same kernels, same load) as well
         sampler.rows = timed_rows
     clocks = sampler.stop()
     clocks["window"] = "timed region" if len(timed_rows) >= 2 else "warm-up + timed region"
+    if args.dump_outputs:
+        outputs = last_step_outputs()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
+        del outputs
     for _ in range(max(1, args.warmup)):               # warm the host-buffer path (staging buffers enter the context's block cache)
         step(False)
     ms_e2e, _, steps_e2e = timed(False, args.steps)

@@ -14,7 +14,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 EXE = os.path.join(ROOT, "oracle", "_ref", "ref_search_gpu")
 
 
-@pytest.mark.skipif(not os.path.exists(EXE), reason="oracle/_ref/ref_search_gpu is built where /root/reference is mounted and travels with the snapshot")
+@pytest.mark.skipif(not os.path.exists(EXE), reason="oracle/_ref/ref_search_gpu is built by `make -C oracle ref` only where the reference's C++ sources are present")
 @pytest.mark.parametrize("name", ["tiny_clean", "tiny_noisy"])
 @pytest.mark.parametrize("strategy", ["sensspec", "splitscafs"])
 def test_reference_driver_with_gpu_separator_matches_reference(tmp_path, name, strategy):
