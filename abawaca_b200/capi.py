@@ -18,6 +18,7 @@ NKMER = 180
 SENS_SPEC, SPLIT_SCAFS = 0, 1
 LAYOUT_COLMAJOR, LAYOUT_ROWMAJOR, LAYOUT_ROWMAJOR_MILLI32 = 0, 1, 2
 FEAT_TRUNC3, FEAT_RAW = 0, 1
+TEXT_3LF, TEXT_LF = 0, 1         # abw_format_lrn: "%.3lf" (abawaca.lrn), "%lf" (clusters/<id>.lrn)
 
 READ_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4"), ("len", "<u4"), ("flag_nsnps", "<u4")])
 READ8_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4")])      # abw_read8: reads the host parser already filtered
@@ -73,7 +74,7 @@ EXPORTS = [
     "abw_copy_to_device", "abw_copy_to_host", "abw_memset_device", "abw_h2d_async", "abw_wait_h2d", "abw_d2h_async", "abw_search_create", "abw_search_create_from_features", "abw_search_destroy", "abw_search_run",
     "abw_search_set_shard", "abw_search_set_shard_strided", "abw_search_set_max_levels", "abw_search_run_sharded", "abw_search_get_profile", "abw_cluster_scg",
     "abw_names_create", "abw_names_destroy", "abw_parse_sam", "abw_fasta_scan", "abw_fasta_destroy", "abw_fasta_count", "abw_fasta_get", "abw_fasta_pack", "abw_nccl_unique_id", "abw_nccl_collectives_create", "abw_nccl_collectives_destroy", "abw_peer_buffer_create", "abw_peer_buffer_destroy", "abw_peer_group_create", "abw_peer_group_destroy",
-    "abw_scatter_columns_milli", "abw_parse_lrn", "abw_search_set_scaffold_stats",
+    "abw_scatter_columns_milli", "abw_parse_lrn", "abw_gather_rows", "abw_format_lrn", "abw_search_set_scaffold_stats",
 ]
 
 
@@ -152,6 +153,9 @@ def load():
     L.abw_peer_group_destroy.restype = None
     L.abw_scatter_columns_milli.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint64, C.c_size_t, C.c_void_p]
     L.abw_parse_lrn.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+    L.abw_gather_rows.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64]
+    L.abw_format_lrn.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
+                                 C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.abw_search_set_scaffold_stats.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.abw_cluster_scg.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32), C.POINTER(C.c_double)]
     _LIB = L

@@ -491,6 +491,20 @@ __global__ void __launch_bounds__(128) k_lrn_parse(const char* __restrict__ text
 		atomicOr(err, LRN_ERR_FIELDS);                       // "number of dimensions found is ...", ClusterData.cpp:137-141
 }
 
+// one warp per destination row: dst[i][0 .. ncols) = src[rows[i]][0 .. ncols)
+__global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ src, uint64_t ld_src, double* __restrict__ dst, uint64_t ld_dst, uint32_t ncols,
+                                                     const uint64_t* __restrict__ rows, uint64_t nrows)
+{
+	const int lane = threadIdx.x & 31;
+	const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+	for(uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < nrows; i += nwarps) {
+		const double* __restrict__ s = src + rows[i] * ld_src;
+		double* __restrict__ d = dst + i * ld_dst;
+		for(uint32_t c = lane; c < ncols; c += 32)
+			d[c] = s[c];
+	}
+}
+
 }  // namespace
 
 extern "C" {
@@ -801,6 +815,28 @@ int abw_parse_lrn(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_d
 			ABW_CUDA(ctx, abw_sync(ctx));
 		}
 	}
+	return ABW_OK;
+}
+
+int abw_gather_rows(abw_ctx* ctx, const double* d_src, uint64_t ld_src, const uint64_t* rows, int rows_on_device, uint64_t nrows, uint32_t ncols, double* d_dst,
+                    uint64_t ld_dst)
+{
+	if(!ctx || (nrows && (!d_src || !d_dst || !rows)) || ld_dst < ncols)
+		return abw_fail(ctx, ABW_ERR_ARG, "abw_gather_rows: bad argument");
+	ABW_ENTER(ctx);
+	if(nrows == 0 || ncols == 0)
+		return ABW_OK;
+	DevBuf<uint64_t> d_rows;
+	const uint64_t* r = rows;
+	if(!rows_on_device) {
+		ABW_CUDA(ctx, d_rows.alloc(nrows));
+		ABW_CUDA(ctx, cudaMemcpyAsync(d_rows.p, rows, nrows * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+		r = d_rows.p;
+	}
+	const unsigned int blocks = (unsigned int)std::min<uint64_t>(abw_div_up(nrows, 8), (uint64_t)ctx->sm_count * 16);
+	ABW_LAUNCH(ctx, k_gather_rows, blocks, 256, 0, d_src, ld_src, d_dst, ld_dst, ncols, r, nrows);
+	if(!rows_on_device)
+		ABW_CUDA(ctx, abw_sync(ctx));      // the host row list may change once the call returns
 	return ABW_OK;
 }
 

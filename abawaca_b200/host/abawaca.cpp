@@ -3,7 +3,8 @@
 //   the work list :98-197 + ClusterSeparatorBySensitivitySpecificity::separate()  ->  abw_search_create + abw_search_run
 // The loaders below rebuild what ScafDpData (ScafDpData.cpp:11-120), ClusterData (ClusterData.cpp:27-168) and SCGdb
 // (SCGdb.cpp:58-120) build, as flat arrays; the writers reproduce log, summary.txt, dp2cluster.txt, scaf2cluster.txt,
-// final-clusters/<id>.fasta and clusters/<id>.{lrn,scaf-cluster.txt,scaf-stats.txt} from the records the device returns.
+// final-clusters/<id>.fasta and clusters/<id>.{lrn,scaf-cluster.txt,scaf-stats.txt} from the records the device returns; the data lines of
+// clusters/<id>.lrn are printed on the device (abw_format_lrn).
 #include "abw_host.h"
 #include <algorithm>
 #include <cmath>
@@ -132,6 +133,7 @@ struct Model {
 	std::vector<unsigned long> dp_name;
 	std::vector<std::string> dim_names;
 	std::vector<double> values;                 // column major [D][N]
+	double* d_rows = nullptr;                   // the same on the device, row major [N][D] (row = 0-based dp id): what the cluster dumps print
 	std::vector<uint64_t> scgmask;              // [S][W]
 	uint32_t W = 1;
 	int total_num_scgs = 0;
@@ -286,12 +288,13 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 			ABWH_CHECK(ctx, abw_copy_to_host(ctx, rows_rm.data(), d_vals, entry * D * sizeof(double)));
 		}
 		ABWH_CHECK(ctx, abw_device_free(ctx, d_keys));
-		ABWH_CHECK(ctx, abw_device_free(ctx, d_vals));
+		std::vector<uint64_t> row_of_dp(N);
 		for(uint64_t r = 0; r < entry; r++) {
 			auto it = dp_name2id.find((unsigned long)keys[r]);
 			if(it != dp_name2id.end()) {
 				const size_t dp = it->second - 1;
 				seen[dp] = 1;
+				row_of_dp[dp] = r;
 				for(size_t d = 0; d < D; d++)
 					M.values[d * N + dp] = rows_rm[r * D + d];
 			}
@@ -299,6 +302,10 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 		for(size_t i = 0; i < N; i++)
 			if(!seen[i])
 				throw std::invalid_argument("datapoint " + std::to_string(M.dp_name[i]) + " of " + P.names_file + " has no row in " + P.lrn_file);
+		// the rows of the file put into dp order where they already are, for the cluster dumps
+		ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<size_t>(N * D, 1) * sizeof(double), (void**)&M.d_rows));
+		ABWH_CHECK(ctx, abw_gather_rows(ctx, d_vals, D, row_of_dp.data(), 0, N, (uint32_t)D, M.d_rows, D));
+		ABWH_CHECK(ctx, abw_device_free(ctx, d_vals));
 	}
 	// SCG database (SCGdb.cpp:58-120): number of names in scg.list; gene -> SCG, gene = <scaffold>_<non-zero integer>
 	{
@@ -334,29 +341,6 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 }
 
 // size-weighted mean and standard deviation in scaffold-id order (ClusterQuality.cpp:6-27)
-// "%lf" of a value (ClusterWriter.cpp:92-98).  Columns written by abawaca-build are multiples of 0.001: for v == k / 1000.0 with a small integer k the
-// six-decimal rendering is k / 1000 "." k % 1000 "000" (the representation error of v is far below half a unit of the sixth decimal); anything else
-// goes through printf.  The cluster dumps are the host-side throughput ceiling of this program (SURVEY.md section 2, row 16).
-static char* format_lf(char* w, double v)
-{
-	const double k = rint(v * 1000.0);
-	if(k >= 0 && k < 2.0e9 && !std::signbit(v) && k / 1000.0 == v) {
-		const unsigned long ki = (unsigned long)k;
-		unsigned long ip = ki / 1000, fp = ki % 1000;
-		char tmp[16];
-		int n = 0;
-		do { tmp[n++] = (char)('0' + ip % 10); ip /= 10; } while(ip);
-		while(n) *w++ = tmp[--n];
-		*w++ = '.';
-		*w++ = (char)('0' + fp / 100);
-		*w++ = (char)('0' + fp / 10 % 10);
-		*w++ = (char)('0' + fp % 10);
-		*w++ = '0'; *w++ = '0'; *w++ = '0';
-		return w;
-	}
-	return w + sprintf(w, "%lf", v);
-}
-
 static void weighted_stats(const std::vector<std::pair<size_t, double>>& data, double& mean, double& stdev)
 {
 	if(data.empty()) { mean = stdev = -1; return; }
@@ -432,6 +416,12 @@ int main(int argc, const char** argv)
 		std::map<uint32_t, std::vector<uint32_t>> dps_of;      // 0-based datapoints, ascending
 		for(size_t i = 0; i < N; i++)
 			for(uint32_t c = dp2cluster[i]; c != 0; c = parent_of[c]) dps_of[c].push_back((uint32_t)i);
+		// the data lines of the cluster dumps: "<dp+1>" and "\t%lf" per value (ClusterWriter.cpp:81-98), made on the device in pieces of at most LRN_CHUNK bytes
+		const uint64_t LRN_CHUNK = (uint64_t)64 << 20;
+		char* d_text = nullptr;
+		ABWH_CHECK(ctx, abw_device_alloc(ctx, LRN_CHUNK, (void**)&d_text));
+		std::vector<char> text;
+		std::vector<uint64_t> rows;
 		auto write_lrn = [&](uint32_t id, const std::vector<uint32_t>& dps) {
 			FILE* fp = fopen((P.cluster_dir + "/" + std::to_string(id) + ".lrn").c_str(), "w");
 			if(!fp) { std::cerr << "Fatal error: could write to file " << P.cluster_dir << "/" << id << ".lrn" << std::endl << std::endl; exit(-1); }
@@ -442,16 +432,14 @@ int main(int argc, const char** argv)
 			fprintf(fp, "\n%c Key", '%');
 			for(size_t d = 0; d < D; d++) fprintf(fp, "\t%s", M.dim_names[d].c_str());
 			fprintf(fp, "\n");
-			std::vector<char> row(32 + D * 32);
-			for(uint32_t dp : dps) {            // the reference writes these rows in unordered_set order (quirk Q9); here ascending dp id
-				char* w = row.data();
-				w += sprintf(w, "%lu", (unsigned long)(dp + 1));
-				for(size_t d = 0; d < D; d++) {
-					*w++ = '\t';
-					w = format_lf(w, M.values[d * N + dp]);
-				}
-				*w++ = '\n';
-				fwrite(row.data(), 1, (size_t)(w - row.data()), fp);
+			rows.assign(dps.begin(), dps.end());     // the reference writes these rows in unordered_set order (quirk Q9); here ascending dp id
+			for(uint64_t line0 = 0; line0 < rows.size();) {
+				uint64_t done = 0, nbytes = 0;
+				ABWH_CHECK(ctx, abw_format_lrn(ctx, M.d_rows, D, 0, (uint32_t)D, rows.data(), 0, line0, rows.size(), ABW_TEXT_LF, d_text, LRN_CHUNK, &done, &nbytes));
+				text.resize(std::max<size_t>(text.size(), nbytes));
+				ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
+				if(fwrite(text.data(), 1, nbytes, fp) != nbytes) { std::cerr << "Fatal error: could write to file " << P.cluster_dir << "/" << id << ".lrn" << std::endl << std::endl; exit(-1); }
+				line0 += done;
 			}
 			fclose(fp);
 		};
@@ -577,6 +565,8 @@ int main(int argc, const char** argv)
 					    << " copies), %G+C=" << avg_gc << ", coverage=" << avg_cvg << std::endl;
 			}
 		}
+		ABWH_CHECK(ctx, abw_device_free(ctx, d_text));
+		ABWH_CHECK(ctx, abw_device_free(ctx, M.d_rows));
 		milestone("logs, fasta and cluster dumps");
 		// dp2cluster.txt has a row for dp 0 as well (abawaca.cpp:199, quirk Q10)
 		ofs_dp << 0 << "\t0" << std::endl;

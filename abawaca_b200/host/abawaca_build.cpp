@@ -5,11 +5,13 @@
 //   Scaf_segment::Scaf_segment      -> abw_kmer_features
 //   Scaf::add_mapped_read           -> abw_coverage (one call per SAM file, reads in file order)
 //   SAMReader / ReadMapping(line)   -> abw_parse_sam (SAM text goes to the device in 64 MB chunks cut at line boundaries)
-// The text writers stay on the host.  Not ported (out of the hot path, SURVEY.md section 2):
+//   the "%.3lf" rows of abawaca.lrn   -> abw_format_lrn (text made on the device in 64 MB pieces, written with fwrite)
+// The other text writers stay on the host.  Not ported (out of the hot path, SURVEY.md section 2):
 // paired-end link counting (abawaca.links is written empty: `abawaca` only checks that it exists) and the calls to
 // the external gene predictor / SCG script.
 #include "abw_host.h"
 #include <algorithm>
+#include <chrono>
 #include <ctime>
 #include <iostream>
 
@@ -22,6 +24,18 @@ static std::string stamp()
 	char b[32];
 	snprintf(b, sizeof(b), "[%02u:%02u:%02u]\t", t / 3600, (t % 3600) / 60, t % 60);
 	return b;
+}
+
+// ABW_TIMING=1: wall-clock milestones on stderr (CUDA start-up, text in, features, text out)
+static void milestone(const std::string& what)
+{
+	static const bool on = getenv("ABW_TIMING") != nullptr;
+	static auto t0 = std::chrono::steady_clock::now();
+	if(!on)
+		return;
+	const auto t1 = std::chrono::steady_clock::now();
+	fprintf(stderr, "[abw timing] %-28s %8.3f s\n", what.c_str(), std::chrono::duration<double>(t1 - t0).count());
+	t0 = t1;
 }
 
 static void usage(const char* prog)
@@ -55,6 +69,7 @@ static std::vector<std::string> kmer_names()
 
 int main(int argc, const char* argv[])
 {
+	milestone("start");
 	const uint32_t window_size = 2000, max_snps = 15;   // abawaca-build.cpp:436-437
 	if(argc < 5) {
 		usage(argv[0]);
@@ -84,6 +99,7 @@ int main(int argc, const char* argv[])
 			std::cerr << "Error: no usable CUDA device (abawaca_b200 has no CPU path)" << std::endl;
 			return -1;
 		}
+		milestone("abw_ctx_create");
 		// the FASTA text goes to the device as it is: records are indexed there (abw_fasta_scan), the host only reads the names
 		std::string fasta_text;
 		{
@@ -132,6 +148,7 @@ int main(int argc, const char* argv[])
 		abw_segments* sg = nullptr;
 		ABWH_CHECK(ctx, abw_segment(ctx, ss, window_size, &sg));
 		const uint64_t ndps = abw_segments_count(sg);
+		milestone("FASTA");
 
 		if(!directory_exists(out_directory)) {
 			std::string cmd = "mkdir " + out_directory;
@@ -150,6 +167,8 @@ int main(int argc, const char* argv[])
 		ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<uint32_t>(nscaf, 1) * sizeof(uint64_t), (void**)&d_nbps));
 		ABWH_CHECK(ctx, abw_memset_device(ctx, d_nbps, 0, std::max<uint32_t>(nscaf, 1) * sizeof(uint64_t)));
 		ABWH_CHECK(ctx, abw_kmer_features(ctx, ss, sg, ABW_FEAT_TRUNC3, 1, d_rows, ld, 0));
+		ABWH_CHECK(ctx, abw_ctx_synchronize(ctx));
+		milestone("k-mer");
 
 		// the scaffold names as a device-side table: SAM text is parsed on the device (abw_parse_sam)
 		abw_names* names = nullptr;
@@ -211,6 +230,7 @@ int main(int argc, const char* argv[])
 			fclose(fp);
 			ABWH_CHECK(ctx, abw_coverage(ctx, sg, d_reads, nreads, 1, max_snps, ABW_FEAT_TRUNC3, d_rows, ld, (uint32_t)(179 + j), is_this_sample? d_nbps : nullptr));
 			ABWH_CHECK(ctx, abw_device_free(ctx, d_reads));
+			milestone("SAM " + std::to_string(j));
 			if(is_this_sample) {
 				FILE* fl = fopen(links_file.c_str(), "w");     // scaffold-end links are not computed (SURVEY.md section 2, row 5); the file must exist
 				if(fl) fclose(fl);
@@ -218,16 +238,14 @@ int main(int argc, const char* argv[])
 		}
 		abw_names_destroy(names);
 
-		// fetch everything the three text files need
-		std::vector<double> rows((size_t)ndps * ld);
+		// fetch what .names and .info need (the matrix stays on the device: abw_format_lrn prints it)
 		std::vector<uint32_t> seg_scaf(ndps);
 		std::vector<uint64_t> seg_start(ndps), seg_end(ndps), seg_nonN(ndps), nbps(nscaf), nN(nscaf), nGC(nscaf);
-		if(ndps)
-			ABWH_CHECK(ctx, abw_copy_to_host(ctx, rows.data(), d_rows, rows.size() * sizeof(double)));
 		ABWH_CHECK(ctx, abw_segments_get(ctx, sg, nullptr, seg_scaf.data(), seg_start.data(), seg_end.data(), seg_nonN.data()));
 		if(nscaf)
 			ABWH_CHECK(ctx, abw_copy_to_host(ctx, nbps.data(), d_nbps, nscaf * sizeof(uint64_t)));
 		ABWH_CHECK(ctx, abw_seqset_stats(ctx, ss, nN.data(), nGC.data()));
+		milestone("fetch");
 
 		FILE* fout = fopen(names_file.c_str(), "w");
 		FILE* flrn = fopen(lrn_file.c_str(), "w");
@@ -245,6 +263,23 @@ int main(int argc, const char* argv[])
 		for(size_t d = 1; d < kn.size(); d++) fprintf(flrn, "\t%s", kn[d].c_str());
 		for(auto& sf : sam_files) fprintf(flrn, "\t%s", sf.c_str());
 		fprintf(flrn, "\n");
+		{
+			// the data lines: "<g+1>" and "\t%.3lf" per value, made on the device in pieces of at most LRN_CHUNK bytes
+			const uint64_t LRN_CHUNK = (uint64_t)64 << 20;
+			char* d_text = nullptr;
+			ABWH_CHECK(ctx, abw_device_alloc(ctx, LRN_CHUNK, (void**)&d_text));
+			std::vector<char> text(LRN_CHUNK);
+			for(uint64_t line0 = 0; line0 < ndps;) {
+				uint64_t done = 0, nbytes = 0;
+				ABWH_CHECK(ctx, abw_format_lrn(ctx, d_rows, ld, 0, (uint32_t)ld, nullptr, 0, line0, ndps, ABW_TEXT_3LF, d_text, LRN_CHUNK, &done, &nbytes));
+				ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
+				if(fwrite(text.data(), 1, nbytes, flrn) != nbytes) { std::cerr << "Could not write to " << lrn_file << std::endl << std::endl; return -1; }
+				line0 += done;
+			}
+			ABWH_CHECK(ctx, abw_device_free(ctx, d_text));
+		}
+		fclose(flrn);
+		milestone(".lrn");
 		uint64_t g = 0;
 		for(uint32_t s = 0; s < nscaf; s++) {
 			const std::string& id = scaf_name[s];
@@ -259,15 +294,11 @@ int main(int argc, const char* argv[])
 				k++;
 				fprintf(fout, "%lu\t%s_%lu\t%s:(%lu, %lu), %lu/%lu non-Ns bps\n", (unsigned long)(g + 1), id.c_str(), k, id.c_str(), (unsigned long)seg_start[g],
 				        (unsigned long)seg_end[g], (unsigned long)seg_nonN[g], (unsigned long)(seg_end[g] - seg_start[g] + 1));
-				fprintf(flrn, "%lu", (unsigned long)(g + 1));
-				for(uint64_t c = 0; c < ld; c++)
-					fprintf(flrn, "\t%.3lf", rows[g * ld + c]);
-				fprintf(flrn, "\n");
 			}
 		}
 		fclose(fout);
-		fclose(flrn);
 		fclose(finfo);
+		milestone(".names, .info");
 
 		std::cerr << stamp() << "Predicting genes and SCGs (skipped: external tools are not part of this build; pass -c <gene2scg> to abawaca)" << std::endl;
 		size_t l = assembly_file.rfind('/');
@@ -295,6 +326,7 @@ int main(int argc, const char* argv[])
 		abw_segments_destroy(sg);
 		abw_seqset_destroy(ss);
 		abw_ctx_destroy(ctx);
+		milestone("teardown");
 		std::cerr << stamp() << "Finished successfully" << std::endl;
 	}
 	catch(std::exception& e) {

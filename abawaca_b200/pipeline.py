@@ -75,6 +75,32 @@ def parse_lrn_rows(ctx, text, D):
     return keys, d_vals, int(n.value)
 
 
+def format_lrn_rows(ctx, d_values, ld, ncols, rows=None, nlines=None, fmt=capi.TEXT_3LF, col0=0, cap=64 << 20, rows_on_device=False) -> bytes:
+    """.lrn data lines of a row-major device matrix (abw_format_lrn): line i is "<r+1>\\t<v_0>...\\n" with r = rows[i] (None: r = i, nlines lines).
+    rows: uint64 numpy array, or a device pointer with rows_on_device.  The text is made in pieces of at most `cap` bytes and concatenated."""
+    if rows is not None and not rows_on_device:
+        rows = np.ascontiguousarray(rows, dtype=np.uint64)
+        nlines = rows.size if nlines is None else nlines
+    if nlines is None:
+        raise ValueError("format_lrn_rows: nlines is required unless rows is a host array")
+    d_text = ctx.alloc(max(cap, 1))
+    out, line0 = [], 0
+    done, nbytes = C.c_uint64(), C.c_uint64()
+    try:
+        while True:                  # at least one call, so that an empty range goes through abw_format_lrn too
+            ctx.check(ctx.lib.abw_format_lrn(ctx.h, C.c_void_p(d_values), ld, col0, ncols, None if rows is None else (C.c_void_p(rows) if rows_on_device else capi._p(rows)),
+                                             1 if rows_on_device else 0, line0, nlines, fmt, C.c_void_p(d_text), cap, C.byref(done), C.byref(nbytes)))
+            buf = np.empty(int(nbytes.value), dtype=np.uint8)
+            ctx.to_host(buf, d_text)
+            out.append(buf.tobytes())
+            line0 += int(done.value)
+            if line0 >= nlines:
+                break
+    finally:
+        ctx.free(d_text)
+    return b"".join(out)
+
+
 def fasta_to_seqset(ctx, text):
     """FASTA text (bytes) -> (seqset handle, names in scaffold order, lengths): records indexed on the device (abw_fasta_scan), the first record of
     every name kept, scaffolds in byte-wise name order (abawaca-build.cpp:482-490), sequences packed by abw_fasta_pack."""

@@ -193,6 +193,25 @@ int      abw_fasta_pack(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_orde
  * abw_search_create as it is (ABW_LAYOUT_ROWMAJOR, values_on_device, h_row_of_dp built from the keys).  Decimal values take the exact
  * one-operation conversion on the device; the rare others (more than 19 digits, exponents beyond +-22, inf/nan) are converted with the host's atof. */
 int abw_parse_lrn(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_device, uint32_t D, uint64_t* d_keys, double* d_values, uint64_t cap_rows, uint64_t* nrows);
+/* Row i of d_dst (row stride ld_dst) = the first ncols values of row rows[i] of d_src (row stride ld_src), for i < nrows; both matrices row-major
+ * doubles in device memory, rows in host memory (rows_on_device = 0) or device memory.  E.g. the rows abw_parse_lrn read, in file order, put
+ * into datapoint order.  Enqueued on the context stream. */
+int abw_gather_rows(abw_ctx* ctx, const double* d_src, uint64_t ld_src, const uint64_t* rows, int rows_on_device, uint64_t nrows, uint32_t ncols, double* d_dst,
+                    uint64_t ld_dst);
+
+/* ---- matrix -> .lrn data lines on the device (the counterpart of abw_parse_lrn) ---------------------------------------------------------------
+ * Replaces the per-value printf of the .lrn writers: abawaca-build's abawaca.lrn ("\t%.3lf", abawaca-build.cpp:603) and ClusterEsomWriter's
+ * clusters/<id>.lrn ("\t%lf", ClusterWriter.cpp:81-98).  Line i (line0 <= i < nlines) is "<r+1>\t<v_0>\t...\t<v_{ncols-1}>\n" with r = rows[i]
+ * (rows == NULL: r = i) and v_c = d_values[r * ld + col0 + c] (row-major doubles, device memory); rows is device memory when rows_on_device != 0.
+ * Every value is byte-identical to what the C library's printf writes for the format: ties round to even, the sign of zero is kept, inf / nan
+ * are "inf", "-inf", "nan", "-nan".  The longest run of whole lines from line0 on that fits `cap` bytes is written to d_text (device memory);
+ * *nlines_done / *nbytes say how many lines and bytes that is, and the caller continues with line0 + *nlines_done.  If line line0 alone does not
+ * fit, nothing is written, *nbytes holds its size and ABW_ERR_ARG is returned.  d_text may start at any byte address.  Values of magnitude >= 2^64 / 10^decimals and non-finite values
+ * are printed by the host's C library; all others on the device. */
+#define ABW_TEXT_3LF 0   /* "%.3lf": abawaca.lrn */
+#define ABW_TEXT_LF  1   /* "%lf":   clusters/<id>.lrn */
+int abw_format_lrn(abw_ctx* ctx, const double* d_values, uint64_t ld, uint32_t col0, uint32_t ncols, const uint64_t* rows, int rows_on_device,
+                   uint64_t line0, uint64_t nlines, int fmt, char* d_text, uint64_t cap, uint64_t* nlines_done, uint64_t* nbytes);
 
 /* device memory helpers so that hosts without a CUDA runtime binding can drive the ABI */
 int abw_device_alloc(abw_ctx* ctx, size_t bytes, void** d_out);
