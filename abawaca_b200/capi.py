@@ -22,7 +22,8 @@ TEXT_3LF, TEXT_LF = 0, 1         # abw_format_lrn: "%.3lf" (abawaca.lrn), "%lf" 
 
 READ_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4"), ("len", "<u4"), ("flag_nsnps", "<u4")])
 READ8_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4")])      # abw_read8: reads the host parser already filtered
-READS_FULL, READS_COMPACT = 0, 1
+READ_RUN_DTYPE = np.dtype([("scaf", "<u4"), ("count", "<u4")])   # abw_read_run: `count` consecutive reads on scaffold `scaf` (sorted format)
+READS_FULL, READS_COMPACT, READS_SORTED = 0, 1, 2
 
 
 class AbwError(RuntimeError):
@@ -50,7 +51,8 @@ class ClusterRec(C.Structure):
 
 class Sample(C.Structure):
     """abw_sample"""
-    _fields_ = [("reads", C.c_void_p), ("nreads", C.c_uint64), ("format", C.c_int32), ("len", C.c_uint32), ("len16", C.c_void_p), ("h2d_ticket", C.c_uint64)]
+    _fields_ = [("reads", C.c_void_p), ("nreads", C.c_uint64), ("format", C.c_int32), ("len", C.c_uint32), ("len16", C.c_void_p), ("h2d_ticket", C.c_uint64),
+                ("runs", C.c_void_p), ("nruns", C.c_uint64), ("exc", C.c_void_p), ("nexc", C.c_uint64)]
 
 
 class SearchProfile(C.Structure):

@@ -261,7 +261,7 @@ void abw_arena_free(abw_ctx* ctx, void* p)
 
 extern "C" {
 
-const char* abw_version(void) { return "abawaca_b200 0.1 (sm_100a)"; }
+const char* abw_version(void) { return "abawaca_b200 0.2 (sm_100a)"; }
 
 void abw_default_params(abw_params* p)
 {

@@ -13,6 +13,7 @@
 //                           sorted stably by (sample, window) in one radix sort and summed in SAM order by one thread per window.
 // ABW_FEAT_RAW (un-truncated doubles) sends every pair through pass 2.
 // Two record formats: abw_read (16 bytes, filter applied here) and abw_read8 (8 bytes: reads the host parser already filtered, SURVEY.md section 8b(4)).
+// Samples of coordinate-sorted reads (ABW_READS_SORTED, about 2 bytes per read) are decoded into abw_read8 records first (readcodec.cu).
 #include "features.cuh"
 #include <algorithm>
 
@@ -656,11 +657,18 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 	for(uint32_t s0 = 0; s0 < nsamples; s0 += group) {
 		const uint32_t ns = std::min(group, nsamples - s0);
 		std::vector<ReadSrc> srcs(ns);
+		// sorted samples are decoded into compact records, which pass 2 reads again: they live until the end of the group
+		std::vector<DevBuf<abw_read8>> decoded(ns);
 		uint32_t total_tiles = 0, max_tiles = 0;
 		for(uint32_t j = 0; j < ns; j++) {
 			const abw_sample& sm = samples[s0 + j];
 			ReadSrc& r = srcs[j];
 			r.p = sm.reads; r.n = sm.nreads; r.len16 = sm.len16; r.len = sm.len; r.fmt = sm.format;
+			if(sm.format == ABW_READS_SORTED) {
+				ABW_CUDA(ctx, decoded[j].alloc(sm.nreads));
+				r.p = decoded[j].p;
+				r.fmt = ABW_READS_COMPACT;
+			}
 			r.tile0 = total_tiles;
 			r.ntiles = abw_div_up(sm.nreads, COV_TILE);
 			total_tiles += r.ntiles;
@@ -676,6 +684,9 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 		if(all) {
 			for(uint32_t j = 0; j < ns; j++)
 				ABW_CHECK(abw_wait_h2d(ctx, samples[s0 + j].h2d_ticket));
+			for(uint32_t j = 0; j < ns; j++)
+				if(samples[s0 + j].format == ABW_READS_SORTED)
+					ABW_CHECK(abw_decode_sorted_reads(ctx, samples[s0 + j], decoded[j].p));
 			ABW_LAUNCH(ctx, k_cov_zero_columns, abw_div_up(g->nseg * ns, 256), 256, 0, d_rows, g->nseg, ld, col0 + s0, ns);
 			ABW_CHECK(coverage_pairs(ctx, g, d_srcs.p, ns, max_tiles, total_tiles, max_snps, kind, d_rows, ld, col0 + s0, true, nullptr, nwords, nullptr, nullptr,
 			                         (unsigned long long*)d_scaf_nbps, nbps_local));
@@ -689,6 +700,8 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 		ABW_CUDA(ctx, cudaMemsetAsync(nflagged.p, 0, sizeof(uint32_t) * ns, ctx->stream));
 		for(uint32_t j = 0; j < ns; j++) {
 			ABW_CHECK(abw_wait_h2d(ctx, samples[s0 + j].h2d_ticket));           // the sample's records may still be on their way (abw_h2d_async)
+			if(samples[s0 + j].format == ABW_READS_SORTED)
+				ABW_CHECK(abw_decode_sorted_reads(ctx, samples[s0 + j], decoded[j].p));
 			if(srcs[j].ntiles == 0)
 				continue;
 			if((int)j == nbps_local)
@@ -725,8 +738,16 @@ int abw_coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* h_
 		const abw_sample& sm = h_samples[j];
 		if(!sm.reads && sm.nreads)
 			return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage_batch: null read records");
-		if(sm.format != ABW_READS_FULL && sm.format != ABW_READS_COMPACT)
+		if(sm.format != ABW_READS_FULL && sm.format != ABW_READS_COMPACT && sm.format != ABW_READS_SORTED)
 			return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage_batch: unknown record format");
+		if(sm.format == ABW_READS_SORTED) {
+			if((!sm.runs && sm.nruns) || (!sm.exc && sm.nexc))
+				return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage_batch: null runs or escape array");
+			if(sm.nexc > sm.nreads)
+				return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage_batch: more escapes than reads");
+			if(sm.nruns >= (1ull << 32))
+				return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage_batch: 2^32 runs or more");
+		}
 		if(sm.nreads >= (1ull << 32))
 			return abw_fail(ctx, ABW_ERR_UNSUPPORTED, "abw_coverage: more than 2^32-1 reads per sample; split the sample");
 	}
@@ -747,7 +768,7 @@ int abw_coverage(abw_ctx* ctx, const abw_segments* g, const abw_read* reads, uin
 		return abw_fail(ctx, ABW_ERR_ARG, "abw_coverage: unknown kind");
 	ABW_ENTER(ctx);
 	DevBuf<abw_read> d_reads;
-	abw_sample sm;
+	abw_sample sm{};
 	sm.reads = reads; sm.nreads = nreads; sm.format = ABW_READS_FULL; sm.len = 0; sm.len16 = nullptr; sm.h2d_ticket = 0;
 	if(!reads_on_device && nreads) {
 		ABW_CUDA(ctx, d_reads.alloc(nreads));

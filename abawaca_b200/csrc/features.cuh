@@ -23,3 +23,6 @@ struct abw_segments {
 
 // scaf_info.w of a scaffold whose windows are all nbps characters long (no N): coverage then needs no window table for its reads
 constexpr uint32_t COV_REGULAR = 0x80000000u;
+
+// readcodec.cu: enqueues the decode of an ABW_READS_SORTED sample (arrays checked by abw_coverage_batch) into d_out[sm.nreads] on the context stream
+int abw_decode_sorted_reads(abw_ctx* ctx, const abw_sample& sm, abw_read8* d_out);

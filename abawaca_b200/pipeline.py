@@ -255,31 +255,67 @@ class FeatureBuild:
 
 
 class ReadSample:
-    """One sample's read records for build_features: either abw_read records (READ_DTYPE, the device applies the filter of abawaca-build.cpp:546-550)
-    or compact abw_read8 records of the reads that passed it on the host (compact_reads), as host arrays or as device pointers."""
+    """One sample's read records for build_features: either abw_read records (READ_DTYPE, the device applies the filter of abawaca-build.cpp:546-550),
+    compact abw_read8 records of the reads that passed it on the host (compact_reads), or the same reads coordinate-sorted in about 2 bytes each
+    (sorted_reads: uint16 deltas in `recs`, plus `runs` and `exc`), as host arrays or as device pointers (d_recs, d_runs, d_exc with nruns, nexc)."""
 
-    def __init__(self, fmt, n, recs=None, length=0, len16=None, d_recs=None, d_len16=None):
+    def __init__(self, fmt, n, recs=None, length=0, len16=None, d_recs=None, d_len16=None, runs=None, exc=None, d_runs=None, d_exc=None, nruns=0, nexc=0):
         self.fmt, self.n, self.recs, self.length, self.len16, self.d_recs, self.d_len16 = fmt, int(n), recs, int(length), len16, d_recs, d_len16
+        self.runs, self.exc, self.d_runs, self.d_exc = runs, exc, d_runs, d_exc
+        self.nruns = int(runs.size) if runs is not None else int(nruns)
+        self.nexc = int(exc.size) if exc is not None else int(nexc)
 
     @property
     def nbytes(self):
-        return self.n * (16 if self.fmt == capi.READS_FULL else 8) + (2 * self.n if (self.len16 is not None or self.d_len16) else 0)
+        per_read = {capi.READS_FULL: 16, capi.READS_COMPACT: 8, capi.READS_SORTED: 2}[self.fmt]
+        return self.n * per_read + (2 * self.n if (self.len16 is not None or self.d_len16) else 0) + 8 * self.nruns + 4 * self.nexc
+
+
+def _host_filter(r, nscaf, max_snps):
+    """the read filter of abawaca-build.cpp:546-550 (mapped, not a secondary alignment, at most max_snps mismatches, scaffold known), file order kept"""
+    flag, nsnps = r["flag_nsnps"] & 0xFFFF, r["flag_nsnps"] >> 16
+    return r[((flag & 0x104) == 0) & (nsnps <= max_snps) & (r["scaf"] < nscaf)]
+
+
+def _lengths(lens):
+    """(one length for the sample, None) when all reads are that long, else (0, uint16 per-read lengths)"""
+    if lens.size == 0 or bool((lens == lens[0]).all()):
+        return (int(lens[0]) if lens.size else 0), None
+    if int(lens.max()) > 65535:
+        raise ValueError("reads longer than 65535 bases need the full record format")
+    return 0, lens.astype(np.uint16)
 
 
 def compact_reads(r, nscaf, max_snps=15) -> ReadSample:
     """What a host-side SAM parser hands over when it applies the read filter itself (abawaca-build.cpp:546-550: mapped, not a secondary alignment,
     at most max_snps mismatches, scaffold known; SURVEY.md section 8b(4)): 8-byte records in SAM order, one length for the sample or uint16 lengths."""
-    flag, nsnps = r["flag_nsnps"] & 0xFFFF, r["flag_nsnps"] >> 16
-    ok = ((flag & 0x104) == 0) & (nsnps <= max_snps) & (r["scaf"] < nscaf)
-    rr = r[ok]
+    rr = _host_filter(r, nscaf, max_snps)
     out = np.empty(rr.size, dtype=capi.READ8_DTYPE)
     out["scaf"], out["pos0"] = rr["scaf"], rr["pos0"]
-    lens = rr["len"]
-    if lens.size == 0 or bool((lens == lens[0]).all()):
-        return ReadSample(capi.READS_COMPACT, out.size, out, int(lens[0]) if lens.size else 0)
-    if int(lens.max()) > 65535:
-        raise ValueError("reads longer than 65535 bases need the full record format")
-    return ReadSample(capi.READS_COMPACT, out.size, out, 0, lens.astype(np.uint16))
+    length, len16 = _lengths(rr["len"])
+    return ReadSample(capi.READS_COMPACT, out.size, out, length, len16)
+
+
+def sorted_reads(r, nscaf, max_snps=15) -> ReadSample:
+    """The reads of compact_reads, in the same order, in the ABW_READS_SORTED format (include/abawaca_b200.h): runs of consecutive reads on one
+    scaffold, a uint16 position delta per read (0xFFFF: the position is the next entry of `exc`).  About 2 bytes per read when the SAM file is
+    coordinate sorted; any order is encoded losslessly."""
+    rr = _host_filter(r, nscaf, max_snps)
+    n = rr.size
+    scaf = rr["scaf"].astype(np.uint32)
+    pos = rr["pos0"].astype(np.int64)
+    starts = np.flatnonzero(np.concatenate(([n > 0], scaf[1:] != scaf[:-1])))
+    runs = np.empty(starts.size, dtype=capi.READ_RUN_DTYPE)
+    runs["scaf"] = scaf[starts]
+    runs["count"] = np.diff(np.append(starts, n))
+    prev = np.empty(n, dtype=np.int64)
+    prev[1:] = pos[:-1]
+    prev[starts] = 0
+    diff = pos - prev
+    esc = (diff < 0) | (diff >= 0xFFFF)
+    delta = np.where(esc, 0xFFFF, diff).astype(np.uint16)
+    length, len16 = _lengths(rr["len"])
+    return ReadSample(capi.READS_SORTED, n, delta, length, len16, runs=runs, exc=pos[esc].astype(np.uint32))
 
 
 def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params=None, kind=capi.FEAT_TRUNC3, skip_A=True,
@@ -317,27 +353,28 @@ def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params
         staged.append(d_seq)
         t_seq = ctx.h2d_async(d_seq, seq)                  # enqueue every host->device copy up front on the copy stream (inputs should be pinned)
         seq, seq_on_device = d_seq, True
-    dev = []                                               # (records, len16) device pointers per sample
+    dev = []                                               # (records, len16, runs, exc) device pointers per sample
     for j, sm in enumerate(samples):
         if sm.d_recs is not None:
-            dev.append((sm.d_recs, sm.d_len16))
+            dev.append((sm.d_recs, sm.d_len16, sm.d_runs, sm.d_exc))
             continue
-        recs = np.ascontiguousarray(sm.recs)
-        d = ctx.alloc(max(recs.nbytes, 16))
-        staged.append(d)
-        d16 = None
-        if sm.len16 is not None:
-            d16 = ctx.alloc(max(sm.len16.nbytes, 16))
-            staged.append(d16)
-        if overlap_h2d:
-            if sm.len16 is not None and sm.n:
-                ctx.h2d_async(d16, sm.len16)
-            tickets[j] = ctx.h2d_async(d, recs) if sm.n else 0   # copies of one stream complete in order: the later ticket covers both
-        elif sm.n:
-            ctx.to_device(d, recs)
-            if sm.len16 is not None:
-                ctx.to_device(d16, sm.len16)
-        dev.append((d, d16))
+        arrays = [np.ascontiguousarray(a) if a is not None else None for a in (sm.recs, sm.len16, sm.runs, sm.exc)]
+        ptrs = []
+        for a in arrays:
+            d = None
+            if a is not None:
+                d = ctx.alloc(max(a.nbytes, 16))
+                staged.append(d)
+            ptrs.append(d)
+        # records last: copies of one stream complete in order, so the ticket of the records covers the sample's other arrays too
+        for a, d in list(zip(arrays, ptrs))[1:] + [(arrays[0], ptrs[0])]:
+            if a is None or a.size == 0:
+                continue
+            if overlap_h2d:
+                tickets[j] = ctx.h2d_async(d, a)
+            else:
+                ctx.to_device(d, a)
+        dev.append(tuple(ptrs))
     if t_seq:
         ctx.wait_h2d(t_seq)
     if seqset is not None:
@@ -371,6 +408,8 @@ def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params
         arr = (capi.Sample * len(samples))()
         for j, sm in enumerate(samples):
             arr[j].reads, arr[j].nreads, arr[j].format, arr[j].len, arr[j].len16, arr[j].h2d_ticket = dev[j][0], sm.n, sm.fmt, sm.length, dev[j][1], tickets[j]
+            if sm.fmt == capi.READS_SORTED:
+                arr[j].runs, arr[j].nruns, arr[j].exc, arr[j].nexc = dev[j][2], sm.nruns, dev[j][3], sm.nexc
         ctx.check(L.abw_coverage_batch(ctx.h, segs, arr, len(samples), p.max_snps, kind, C.c_void_p(d_rows), ncols, nk,
                                        this_sample if this_sample is not None else -1, C.c_void_p(d_nbps)))
     ctx.synchronize()

@@ -124,7 +124,7 @@ int abw_kmer_features(abw_ctx* ctx, const abw_seqset* s, const abw_segments* g, 
 int abw_coverage(abw_ctx* ctx, const abw_segments* g, const abw_read* reads, uint64_t nreads, int reads_on_device, uint32_t max_snps,
                  int kind, double* d_rows, uint64_t ld, uint32_t col, uint64_t* d_scaf_nbps);
 
-/* Several samples in one call, in either record format.  ABW_READS_FULL: abw_read records, the read filter (:546-550) is applied on the device.
+/* Several samples in one call, in any of the record formats.  ABW_READS_FULL: abw_read records, the read filter (:546-550) is applied on the device.
  * ABW_READS_COMPACT: abw_read8 records of the reads that PASSED that filter on the host (SURVEY.md section 8b(4): the host parser may pre-filter), in SAM
  * order, 8 bytes instead of 16 over the host link; every read is `len` bases long unless len16 gives per-read lengths (reads longer than 65535 bases
  * need the full format).  Record arrays (and len16) are DEVICE memory; h2d_ticket (0: none) is the abw_h2d_async ticket they depend on -- the call
@@ -138,13 +138,32 @@ typedef struct {
 } abw_read8;
 #define ABW_READS_FULL    0
 #define ABW_READS_COMPACT 1
+/* ABW_READS_SORTED: the reads of ABW_READS_COMPACT (host-filtered, in SAM order) in about 2 bytes per read when the SAM file is coordinate sorted.
+ * The reads are cut into runs of one scaffold each, runs[nruns]: `count` consecutive reads on scaffold `scaf` (a scaffold may appear in several runs,
+ * in any order; a count may be 0).  `reads` points to uint16_t delta[nreads]: read i's pos0 is prev + delta[i], prev being the pos0 of read i - 1 when
+ * that read is in the same run and 0 for the first read of a run.  delta 0xFFFF is an escape: pos0 is then exc[k], k = number of escapes before read i
+ * (an encoder escapes every difference that is negative or >= 0xFFFF).  Lengths as in the compact format (len, or len16).  Nothing is reordered, so
+ * the result is that of the compact records of the same reads.  The arrays may still be in flight behind h2d_ticket, so malformed contents are dealt
+ * with on the device: reads past the sum of the counts, reads of runs with scaf >= nscaf and escapes with k >= nexc are skipped (an escaped read that
+ * is skipped counts as pos0 0 for the read after it); counts past nreads are ignored.  Decoded into 8-byte records in device memory of the context
+ * that live until the call returns. */
+#define ABW_READS_SORTED  2
 typedef struct {
-	const void*     reads;       /* abw_read[nreads] or abw_read8[nreads], device memory */
+	uint32_t scaf;        /* 0-based scaffold index */
+	uint32_t count;       /* consecutive reads on it */
+} abw_read_run;
+typedef struct {
+	const void*     reads;       /* abw_read[nreads], abw_read8[nreads] or uint16_t delta[nreads], device memory */
 	uint64_t        nreads;
 	int32_t         format;
-	uint32_t        len;         /* compact: read length when len16 is NULL */
-	const uint16_t* len16;       /* compact, optional: per-read lengths, device memory */
+	uint32_t        len;         /* compact, sorted: read length when len16 is NULL */
+	const uint16_t* len16;       /* compact, sorted, optional: per-read lengths, device memory */
 	uint64_t        h2d_ticket;
+	/* sorted only (zero for the other formats): device memory, nruns < 2^32, nexc <= nreads */
+	const abw_read_run* runs;
+	uint64_t        nruns;
+	const uint32_t* exc;         /* escaped positions in read order */
+	uint64_t        nexc;
 } abw_sample;
 int abw_coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* h_samples, uint32_t nsamples, uint32_t max_snps, int kind, double* d_rows, uint64_t ld,
                        uint32_t col0, int32_t this_sample, uint64_t* d_scaf_nbps);
