@@ -44,6 +44,7 @@ struct abw_ctx {
 	size_t scan_cap = 0;
 	uint32_t scan_epoch = 0;
 	uint64_t scan_tickets = 0;
+	uint32_t* scan_failed = nullptr;          // mapped pinned word: set by a prefix sum whose look-back wait gave up, reported and cleared by abw_sync
 };
 
 // Small uploads (descriptors, job lists, tile tables) go through pinned memory so that cudaMemcpyAsync really is asynchronous.
@@ -59,6 +60,7 @@ cudaError_t abw_stage_upload(abw_ctx* ctx, void* d_dst, const void* h_src, size_
 // abw_fetch lets a kernel write the result into mapped pinned memory, from where abw_sync (cudaStreamSynchronize + copy-out) hands it to the
 // caller's buffer.  ABW_SMALL_COPIES=memcpy selects plain cudaMemcpyAsync (the round-1 behaviour).  Every device->host result of an entry point
 // is requested with abw_fetch and every wait on the context stream is abw_sync; ABW_ENTER drops requests an earlier, failed call may have left behind.
+// abw_sync also fails (cudaErrorTimeout) when a prefix sum enqueued since the previous abw_sync gave up a look-back wait: its results are wrong.
 bool abw_small_copies_by_kernel();
 cudaError_t abw_fetch(abw_ctx* ctx, void* h_dst, const void* d_src, size_t bytes);
 cudaError_t abw_sync(abw_ctx* ctx);
@@ -158,6 +160,90 @@ struct DevBuf {
 };
 
 static inline unsigned int abw_div_up(uint64_t a, uint64_t b) { return (unsigned int)((a + b - 1) / b); }
+
+// ---- decoupled look-back, shared by every one-pass kernel (k_scan_onepass, k_flip_prefix, k_sweep_split_scafs, k_sweep_ss, k_partition2) ----
+// A tile publishes its aggregate, walks back over its predecessors until it meets a published inclusive prefix, and publishes its own.
+// Published words carry the epoch of the launch (or search level) that wrote them: words of earlier epochs read as empty, so the arrays are not
+// cleared between launches.
+constexpr uint32_t LB_EMPTY = 0, LB_AGG = 1, LB_PREFIX = 2;
+constexpr uint32_t LB_SPIN_LIMIT = 1u << 28;      // a bug must not hang the GPU: give up, flag the error, produce garbage that the host rejects
+
+__device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t* p) { return *reinterpret_cast<const volatile uint32_t*>(p); }
+__device__ __forceinline__ void st_volatile_u32(uint32_t* p, uint32_t v) { *reinterpret_cast<volatile uint32_t*>(p) = v; }
+__device__ __forceinline__ unsigned long long ld_volatile_u64(const unsigned long long* p) { return *reinterpret_cast<const volatile unsigned long long*>(p); }
+__device__ __forceinline__ void st_volatile_u64(unsigned long long* p, unsigned long long v) { *reinterpret_cast<volatile unsigned long long*>(p) = v; }
+
+// Packed layout: one 64-bit word, payload in bits 0-55, epoch (6 bits) in 56-61, state in 62-63.  One store publishes value and state together.
+__device__ __forceinline__ unsigned long long lb_pack(unsigned long long payload, uint32_t st, uint32_t epoch)
+{
+	return payload | ((unsigned long long)(epoch & 63u) << 56) | ((unsigned long long)st << 62);
+}
+__device__ __forceinline__ uint32_t lb_packed_state(unsigned long long v, uint32_t epoch)
+{
+	return (((uint32_t)(v >> 56) & 63u) == (epoch & 63u))? (uint32_t)(v >> 62) : LB_EMPTY;
+}
+
+// Split layout: a u32 status word (epoch << 2) | state, the value in a slot of its own.  The writer stores the value (st.cg), then publishes the
+// state; the reader, once the walk has seen the states, fences and reads the values with ld.cg (lb_split_value).
+__device__ __forceinline__ void lb_split_publish(uint32_t* status, uint32_t st, uint32_t epoch)
+{
+	__threadfence();
+	st_volatile_u32(status, (epoch << 2) | st);
+}
+__device__ __forceinline__ uint32_t lb_split_state(uint32_t raw, uint32_t epoch) { return ((raw >> 2) == epoch)? (raw & 3u) : LB_EMPTY; }
+// value of predecessor i for a sum: its aggregate below the prefix, its inclusive prefix at it, zero where the lane does not take part
+template <typename T, typename Slot, typename LdCg>
+__device__ __forceinline__ T lb_split_value(uint64_t i, bool take, bool at_prefix, const Slot* aggs, const Slot* prefixes, LdCg ld_cg)
+{
+	__threadfence();
+	T v{};
+	if(take)
+		v = at_prefix? ld_cg(prefixes + i) : ld_cg(aggs + i);
+	return v;
+}
+
+// The walk of one warp over the predecessors w-1, w-2, ..., w-npred of tile w (npred > 0), 32 per window: lane l of a window reads the word of
+// predecessor i = base - l, so higher lanes are earlier tiles.  Once every predecessor of the window up to its nearest published prefix has
+// published, fold(word, i, take, first_prefix) runs on all lanes: first_prefix is the lane of that prefix (32: the window has none and the walk
+// goes on), take is true on the lanes that hold a predecessor up to and including it.  Returns false when a wait exceeded LB_SPIN_LIMIT.
+template <typename Load, typename State, typename Fold>
+__device__ __forceinline__ bool lb_walk(uint64_t w, uint32_t npred, Load load, State state, Fold fold)
+{
+	const uint32_t lane = threadIdx.x & 31;
+	uint64_t base = w - 1;
+	uint32_t remaining = npred;
+	bool done = false, failed = false;
+	while(!done && !failed) {
+		const uint32_t cnt = min(32u, remaining);
+		decltype(load(base)) v{};
+		uint32_t first_prefix, spins = 0;
+		while(true) {
+			if(lane < cnt)
+				v = load(base - lane);
+			const uint32_t st = state(v);
+			const uint32_t pm = __ballot_sync(0xffffffffu, lane < cnt && st == LB_PREFIX);
+			const uint32_t em = __ballot_sync(0xffffffffu, lane < cnt && st == LB_EMPTY);
+			first_prefix = pm? (uint32_t)(__ffs(pm) - 1) : 32u;
+			const uint32_t need = (first_prefix >= 32u)? 0xFFFFFFFFu : ((2u << first_prefix) - 1u);
+			if((em & need) == 0)
+				break;
+			if(++spins >= LB_SPIN_LIMIT) {
+				failed = true;
+				break;
+			}
+		}
+		if(failed)
+			break;
+		fold(v, base - lane, lane < cnt && lane <= first_prefix, first_prefix);
+		if(first_prefix < 32u)
+			done = true;
+		else {
+			base -= 32;
+			remaining -= 32;
+		}
+	}
+	return !failed;
+}
 
 // ---- device-wide primitives implemented in scan_sort.cu -------------------------------------------
 // exclusive prefix sum of n uint64 values (in place allowed); d_total (may be null) receives the sum

@@ -186,7 +186,11 @@ cudaError_t abw_fetch(abw_ctx* ctx, void* h_dst, const void* d_src, size_t bytes
 
 cudaError_t abw_sync(abw_ctx* ctx)
 {
-	const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+	cudaError_t e = cudaStreamSynchronize(ctx->stream);
+	if(e == cudaSuccess && *ctx->scan_failed) {
+		*ctx->scan_failed = 0;
+		e = cudaErrorTimeout;
+	}
 	if(e == cudaSuccess)
 		for(const abw_ctx::Fetch& f : ctx->pending)
 			memcpy(f.h_dst, f.slot, f.bytes);
@@ -296,10 +300,12 @@ int abw_ctx_create(int device, abw_ctx** out)
 	abw_ctx* c = new abw_ctx();
 	c->device = device;
 	if(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
-	   cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess) {
+	   cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess ||
+	   cudaHostAlloc((void**)&c->scan_failed, sizeof(uint32_t), cudaHostAllocMapped) != cudaSuccess) {
 		delete c;
 		return ABW_ERR_CUDA;
 	}
+	*c->scan_failed = 0;
 	cudaDeviceProp prop;
 	if(cudaGetDeviceProperties(&prop, device) == cudaSuccess)
 		c->sm_count = prop.multiProcessorCount;
@@ -374,6 +380,9 @@ void abw_ctx_destroy(abw_ctx* ctx)
 	if(ctx->scan_scratch)
 		cudaFree(ctx->scan_scratch);
 	ctx->scan_scratch = nullptr;
+	if(ctx->scan_failed)
+		cudaFreeHost(ctx->scan_failed);
+	ctx->scan_failed = nullptr;
 	for(cudaEvent_t e : ctx->copy_events)
 		cudaEventDestroy(e);
 	if(ctx->side_stream) {

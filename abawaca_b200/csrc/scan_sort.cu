@@ -50,11 +50,12 @@ __device__ __forceinline__ uint64_t block_excl_scan_u64(uint64_t v, uint64_t* to
 // a tile publishes its sum, looks back over its predecessors until it meets a published inclusive prefix, publishes its own and writes its values.
 // The per-context scratch (status words, sums, prefixes, ticket) is never cleared between scans: status words carry the number of the scan that wrote
 // them (epoch), and the ticket counter keeps running -- the host knows how many tickets every scan draws (its number of CTAs = tiles).
-constexpr uint32_t SC_EMPTY = 0, SC_AGG = 1, SC_PREFIX = 2;
+// A look-back wait that gives up sets *failed (mapped pinned memory of the context), which abw_sync reports.
 template <typename Tin>
 __global__ void __launch_bounds__(SCAN_THREADS) k_scan_onepass(const Tin* __restrict__ in, uint64_t* __restrict__ out, uint64_t n, uint64_t* __restrict__ total_out,
                                                               unsigned long long* __restrict__ ticket, unsigned long long ticket_base, uint32_t epoch,
-                                                              uint32_t* __restrict__ status, unsigned long long* __restrict__ aggs, unsigned long long* __restrict__ prefixes)
+                                                              uint32_t* __restrict__ status, unsigned long long* __restrict__ aggs, unsigned long long* __restrict__ prefixes,
+                                                              uint32_t* __restrict__ failed)
 {
 	__shared__ uint64_t sm[33];
 	__shared__ unsigned long long sm_tile, sm_carry;
@@ -78,49 +79,23 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_onepass(const Tin* __rest
 		if(tile > 0) {
 			if(lane == 0) {
 				__stcg(&aggs[tile], (unsigned long long)total);
-				__threadfence();
-				*reinterpret_cast<volatile uint32_t*>(&status[tile]) = (epoch << 2) | SC_AGG;
+				lb_split_publish(&status[tile], LB_AGG, epoch);
 			}
-			uint64_t probe = tile - 1;
-			uint64_t remaining = tile;
-			bool done = false;
-			while(!done) {
-				const uint32_t cnt = (uint32_t)min((uint64_t)32, remaining);
-				uint32_t st, first_prefix;
-				while(true) {
-					uint32_t raw = ((uint32_t)lane < cnt)? *reinterpret_cast<const volatile uint32_t*>(&status[probe - lane]) : ((epoch << 2) | SC_AGG);
-					st = ((raw >> 2) == epoch)? (raw & 3u) : SC_EMPTY;
-					const uint32_t pm = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == SC_PREFIX);
-					const uint32_t em = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == SC_EMPTY);
-					first_prefix = pm? (uint32_t)(__ffs(pm) - 1) : 32u;
-					const uint32_t need = (first_prefix >= 32u)? 0xFFFFFFFFu : ((2u << first_prefix) - 1u);
-					if((em & need) == 0)
-						break;
-				}
-				__threadfence();
-				unsigned long long x = 0;
-				if((uint32_t)lane < cnt) {
-					if((uint32_t)lane < first_prefix)
-						x = __ldcg(&aggs[probe - lane]);
-					else if((uint32_t)lane == first_prefix)
-						x = __ldcg(&prefixes[probe - lane]);
-				}
+			const bool ok = lb_walk(tile, (uint32_t)tile, [&](uint64_t i) { return ld_volatile_u32(&status[i]); }, [&](uint32_t raw) { return lb_split_state(raw, epoch); },
+			                        [&](uint32_t, uint64_t i, bool take, uint32_t first_prefix) {
+				unsigned long long x = lb_split_value<unsigned long long>(i, take, (uint32_t)lane == first_prefix, aggs, prefixes,
+				                                                          [](const unsigned long long* p) { return __ldcg(p); });
 #pragma unroll
 				for(int o = 16; o > 0; o >>= 1)
 					x += __shfl_xor_sync(0xffffffffu, x, o);
 				carry += x;
-				if(first_prefix < 32u)
-					done = true;
-				else {
-					probe -= 32;
-					remaining -= 32;
-				}
-			}
+			});
+			if(!ok && lane == 0)
+				*failed = 1u;
 		}
 		if(lane == 0) {
 			__stcg(&prefixes[tile], carry + (unsigned long long)total);
-			__threadfence();
-			*reinterpret_cast<volatile uint32_t*>(&status[tile]) = (epoch << 2) | SC_PREFIX;
+			lb_split_publish(&status[tile], LB_PREFIX, epoch);
 			sm_carry = carry;
 			if(total_out != nullptr && tile == gridDim.x - 1)
 				*total_out = carry + total;
@@ -170,7 +145,7 @@ int scan_impl(abw_ctx* ctx, const Tin* d_in, uint64_t* d_out, uint64_t n, uint64
 		ctx->scan_tickets = 0;
 	}
 	ABW_LAUNCH(ctx, k_scan_onepass<Tin>, nblocks, SCAN_THREADS, 0, d_in, d_out, n, d_total, ticket, (unsigned long long)ctx->scan_tickets, ctx->scan_epoch, status, aggs,
-	           prefixes);
+	           prefixes, ctx->scan_failed);
 	ctx->scan_tickets += nblocks;
 	return ABW_OK;
 }

@@ -174,14 +174,6 @@ struct __align__(16) AggSlot { Agg v; unsigned long long pad; };   // 32 bytes
 
 // status words carry the epoch (level number + 1) of the search level that wrote them: words of earlier levels read as empty, so the look-back arrays are
 // cleared once per search and not once per level (nothing in a level depends on a host-side memset of a size only the device knows)
-constexpr uint32_t LB_EMPTY = 0, LB_AGG = 1, LB_PREFIX = 2;
-__device__ __forceinline__ uint32_t lb_state(uint32_t raw, uint32_t epoch) { return ((raw >> 2) == epoch)? (raw & 3u) : LB_EMPTY; }
-constexpr uint32_t LB_SPIN_LIMIT = 1u << 28;      // a bug must not hang the GPU: give up, flag the error, produce garbage that the host rejects
-
-__device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t* p) { return *reinterpret_cast<const volatile uint32_t*>(p); }
-__device__ __forceinline__ void st_volatile_u32(uint32_t* p, uint32_t v) { *reinterpret_cast<volatile uint32_t*>(p) = v; }
-__device__ __forceinline__ unsigned long long ld_volatile_u64(const unsigned long long* p) { return *reinterpret_cast<const volatile unsigned long long*>(p); }
-__device__ __forceinline__ void st_volatile_u64(unsigned long long* p, unsigned long long v) { *reinterpret_cast<volatile unsigned long long*>(p) = v; }
 __device__ __forceinline__ Agg ld_cg_agg(const AggSlot* p)
 {
 	const uint4* q = reinterpret_cast<const uint4*>(p);
@@ -196,113 +188,56 @@ __device__ __forceinline__ void st_cg_agg(AggSlot* p, const Agg& v)
 	__stcg(q + 1, make_uint4((uint32_t)v.e, (uint32_t)(v.e >> 32), 0u, 0u));
 }
 
-// Decoupled look-back of warp 0 over the earlier tiles of a segment (items w - tile .. w - 1): publishes this tile's aggregate, walks back
-// 32 predecessors at a time until it meets a published inclusive prefix, publishes its own inclusive prefix and returns the exclusive one.
+// Decoupled look-back of warp 0 over the earlier tiles of a segment (items w - tile .. w - 1), split layout: publishes this tile's aggregate, walks
+// back to the nearest published inclusive prefix, publishes its own inclusive prefix and returns the exclusive one.
 __device__ __forceinline__ Agg agg_lookback(uint64_t w, uint32_t tile, const Agg& total, uint32_t* __restrict__ status, AggSlot* __restrict__ aggs,
                                             AggSlot* __restrict__ prefixes, uint32_t epoch, uint32_t* __restrict__ error_flag)
 {
-	const int ln = threadIdx.x;
+	const int ln = threadIdx.x & 31;
 	Agg carry = agg_zero();
-	if(tile == 0) {
+	if(tile > 0) {
 		if(ln == 0) {
-			st_cg_agg(&prefixes[w], total);
-			__threadfence();
-			st_volatile_u32(&status[w], (epoch << 2) | LB_PREFIX);
+			st_cg_agg(&aggs[w], total);
+			lb_split_publish(&status[w], LB_AGG, epoch);
 		}
-		return carry;
-	}
-	if(ln == 0) {
-		st_cg_agg(&aggs[w], total);
-		__threadfence();
-		st_volatile_u32(&status[w], (epoch << 2) | LB_AGG);
-	}
-	uint64_t base = w - 1;              // nearest predecessor; lane l looks at base - l
-	uint32_t remaining = tile;          // predecessors left in this segment (tile 0 always ends the walk with a prefix)
-	bool done = false, failed = false;
-	while(!done && !failed) {
-		const uint32_t cnt = min(32u, remaining);
-		uint32_t st, first_prefix, spins = 0;
-		while(true) {
-			st = ((uint32_t)ln < cnt)? lb_state(ld_volatile_u32(&status[base - ln]), epoch) : LB_AGG;
-			const uint32_t pm = __ballot_sync(0xffffffffu, (uint32_t)ln < cnt && st == LB_PREFIX);
-			const uint32_t em = __ballot_sync(0xffffffffu, (uint32_t)ln < cnt && st == LB_EMPTY);
-			first_prefix = pm? (uint32_t)(__ffs(pm) - 1) : 32u;
-			const uint32_t need = (first_prefix >= 32u)? 0xFFFFFFFFu : ((2u << first_prefix) - 1u);
-			if((em & need) == 0)
-				break;
-			if(++spins >= LB_SPIN_LIMIT) {
-				failed = true;
-				break;
-			}
-		}
-		if(failed)
-			break;
-		__threadfence();
-		Agg v = agg_zero();
-		if((uint32_t)ln < cnt) {
-			if((uint32_t)ln < first_prefix)
-				v = ld_cg_agg(&aggs[base - ln]);
-			else if((uint32_t)ln == first_prefix)
-				v = ld_cg_agg(&prefixes[base - ln]);
-		}
+		const bool ok = lb_walk(w, tile, [&](uint64_t i) { return ld_volatile_u32(&status[i]); }, [&](uint32_t raw) { return lb_split_state(raw, epoch); },
+		                        [&](uint32_t, uint64_t i, bool take, uint32_t first_prefix) {
+			Agg v = lb_split_value<Agg>(i, take, (uint32_t)ln == first_prefix, aggs, prefixes, ld_cg_agg);
 #pragma unroll
-		for(int o = 16; o > 0; o >>= 1) {
-			Agg t2;
-			t2.a = __shfl_xor_sync(0xffffffffu, v.a, o); t2.b = __shfl_xor_sync(0xffffffffu, v.b, o);
-			t2.c = __shfl_xor_sync(0xffffffffu, v.c, o); t2.d = __shfl_xor_sync(0xffffffffu, v.d, o);
-			t2.e = __shfl_xor_sync(0xffffffffu, v.e, o);
-			v = agg_add(v, t2);
-		}
-		carry = agg_add(carry, v);
-		if(first_prefix < 32u)
-			done = true;
-		else {
-			base -= 32;
-			remaining -= 32;
-		}
+			for(int o = 16; o > 0; o >>= 1) {
+				Agg t2;
+				t2.a = __shfl_xor_sync(0xffffffffu, v.a, o); t2.b = __shfl_xor_sync(0xffffffffu, v.b, o);
+				t2.c = __shfl_xor_sync(0xffffffffu, v.c, o); t2.d = __shfl_xor_sync(0xffffffffu, v.d, o);
+				t2.e = __shfl_xor_sync(0xffffffffu, v.e, o);
+				v = agg_add(v, t2);
+			}
+			carry = agg_add(carry, v);
+		});
+		if(!ok && ln == 0)
+			atomicExch(error_flag, 1u);
 	}
-	if(failed && ln == 0)
-		atomicExch(error_flag, 1u);
 	if(ln == 0) {
 		st_cg_agg(&prefixes[w], agg_add(carry, total));
-		__threadfence();
-		st_volatile_u32(&status[w], (epoch << 2) | LB_PREFIX);
+		lb_split_publish(&status[w], LB_PREFIX, epoch);
 	}
 	return carry;
 }
 
-// per-element contribution to the running sums (see the table in DESIGN.md section 3)
-template <int STRATEGY>
+// per-element contribution to the running sums of the split-scafs sweep (see the table in DESIGN.md section 3)
+// a: ndps_in_scafs_that_belong of side 1, b: scafs_in of side 1, c: decrease of ndps_in_scafs_that_belong of side 2, d: decrease of scafs_in of side 2
 __device__ __forceinline__ Agg contribution(uint32_t el, bool in_range, const ScafRow* __restrict__ rows, double fraction_in)
 {
 	const uint32_t cls = (el >> EL_CLASS_SHIFT) & 3u, aux = (el >> EL_AUX_SHIFT) & 3u;
 	Agg x = agg_zero();
-	if(STRATEGY == ABW_SENS_SPEC) {
-		// a: TP1 (dps of side 1 whose scaffold is assigned to side 1), b: total_dps_for_assigned_scafs of side 1,
-		// c: dps in the cluster of the scaffolds assigned to side 1, d: SCG-carrying scaffolds flipped, e: their length
-		if(cls == 2u)
-			x.a = 1;
-		else if(cls == 1u) {
-			const uint4 r = __ldg(reinterpret_cast<const uint4*>(rows + (el & EL_SCAF_MASK)));   // {T, n, len}
-			x.a = r.x / 2 + 1;          // the flip element brings itself and the floor(T/2) earlier dps of the scaffold (...Specificity.cpp:41-57)
-			x.b = r.x;
-			x.c = r.y;
-			x.d = aux & 1u;
-			x.e = (unsigned long long)r.z | ((unsigned long long)r.w << 32);
-		}
-	}
-	else {
-		// a: ndps_in_scafs_that_belong of side 1, b: scafs_in of side 1, c: decrease of ndps_in_scafs_that_belong of side 2, d: decrease of scafs_in of side 2
-		if(cls == 2u)
-			x.a = 1;
-		if(aux == 0u && in_range)
-			x.c = 1;
-		if(cls == 1u || aux == 1u) {
-			const uint4 r = __ldg(reinterpret_cast<const uint4*>(rows + (el & EL_SCAF_MASK)));
-			const uint32_t r1 = (uint32_t)ceil(__dmul_rn(fraction_in, (double)r.x));
-			if(cls == 1u) { x.a = r1; x.b = 1; }
-			if(aux == 1u) { x.c = r1; x.d = 1; }
-		}
+	if(cls == 2u)
+		x.a = 1;
+	if(aux == 0u && in_range)
+		x.c = 1;
+	if(cls == 1u || aux == 1u) {
+		const uint4 r = __ldg(reinterpret_cast<const uint4*>(rows + (el & EL_SCAF_MASK)));
+		const uint32_t r1 = (uint32_t)ceil(__dmul_rn(fraction_in, (double)r.x));
+		if(cls == 1u) { x.a = r1; x.b = 1; }
+		if(aux == 1u) { x.c = r1; x.d = 1; }
 	}
 	return x;
 }
@@ -337,18 +272,17 @@ __device__ __forceinline__ void block_best_out(CandRec best, uint32_t d, CandRec
 		out[w] = best;
 }
 
-template <int STRATEGY>
-__global__ void __launch_bounds__(SW_THREADS, 3) k_sweep(const uint32_t* __restrict__ E, uint64_t N, const LevelCluster* __restrict__ clusters, uint32_t D,
-                                                        LevelCtl* __restrict__ ctl, const uint2* __restrict__ tile_tab, const ScafRow* __restrict__ rows,
-                                                        const uint8_t* __restrict__ pass_tab, SweepParams prm, uint32_t epoch, uint32_t* __restrict__ status,
-                                                        AggSlot* __restrict__ aggs, AggSlot* __restrict__ prefixes, CandRec* __restrict__ out)
+__global__ void __launch_bounds__(SW_THREADS, 3) k_sweep_split_scafs(const uint32_t* __restrict__ E, uint64_t N, const LevelCluster* __restrict__ clusters, uint32_t D,
+                                                                    LevelCtl* __restrict__ ctl, const uint2* __restrict__ tile_tab, const ScafRow* __restrict__ rows,
+                                                                    SweepParams prm, uint32_t epoch, uint32_t* __restrict__ status, AggSlot* __restrict__ aggs,
+                                                                    AggSlot* __restrict__ prefixes, CandRec* __restrict__ out)
 {
 	__shared__ Agg sm_agg[SW_THREADS / 32 + 1];
 	__shared__ CandRec sm_best[SW_THREADS / 32];
 	__shared__ unsigned long long sm_w;
 	__shared__ Agg sm_carry;
 	const uint32_t TT = ctl->TT;
-	const uint64_t items = (uint64_t)TT * D, tab_stride = ctl->tab_total;
+	const uint64_t items = (uint64_t)TT * D;
 	// work items are (dimension, tile-table entry), entry fastest: the tiles of a (cluster, dimension) segment are consecutive items.  CTAs take items
 	// through a ticket until none is left, so an item only ever waits for items taken earlier by CTAs that are running (forward progress).
 	while(true) {
@@ -363,11 +297,10 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep(const uint32_t* __restr
 		const uint32_t c = te.x, tile = te.y;
 		const ClusterDesc cl = clusters[c].d;
 		const uint32_t* __restrict__ seg = E + (uint64_t)d * N + cl.off;
-		const uint8_t* __restrict__ tab = (STRATEGY == ABW_SENS_SPEC)? pass_tab + (uint64_t)d * tab_stride + cl.tabOff : nullptr;
 		const uint32_t n = cl.n;
 		CandRec best;
 		best.found = 0; best.k1 = 0; best.k2 = 0; best.p = 0; best.i0 = best.i1 = best.i2 = 0; best.dim0 = d;
-		if(STRATEGY == ABW_SPLIT_SCAFS && !cl.ss_ok) {        // uniform over the tiles of the cluster: nobody waits for these items
+		if(!cl.ss_ok) {        // uniform over the tiles of the cluster: nobody waits for these items
 			if(threadIdx.x == 0)
 				out[w] = best;
 			__syncthreads();
@@ -393,7 +326,7 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep(const uint32_t* __restr
 		Agg tsum = agg_zero();
 #pragma unroll
 		for(int j = 0; j < SW_ITEMS; j++)
-			tsum = agg_add(tsum, contribution<STRATEGY>(el[j], i0 + j < n, rows, prm.fraction_in));
+			tsum = agg_add(tsum, contribution(el[j], i0 + j < n, rows, prm.fraction_in));
 		Agg total;
 		Agg ex = block_excl_scan_agg(tsum, total, sm_agg);
 		// decoupled look-back over the earlier tiles of this (cluster, dimension)
@@ -409,47 +342,23 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep(const uint32_t* __restr
 		for(int j = 0; j < SW_ITEMS; j++) {
 			const uint32_t p = i0 + j;
 			if((el[j] & EL_BOUNDARY) && p < n && p >= prm.thr && n - p >= prm.thr) {
-				if(STRATEGY == ABW_SENS_SPEC) {
-					// ...Specificity.cpp:146-161 with TP1/FP1/TP2/FP2 written as prefix sums
-					uint32_t TP, tot, u;
-					if(p < n - p) { TP = ex.a; tot = ex.b; u = p; }
-					else { TP = (n - p) - (ex.c - ex.a); tot = cl.totT - ex.b; u = n - p; }
-					if(tot != 0) {
-						const float fTP = (float)TP;
-						if(fTP >= prm.prune * (float)tot && fTP >= prm.prune * (float)u) {
-							const double sens = __ddiv_rn((double)(int)TP, (double)(int)tot), spec = __ddiv_rn((double)(int)TP, (double)(int)u);
-							const double score = __dmul_rn(sens, spec);
-							if(score >= prm.min_score && (!best.found || score > best.k1)) {
-								const uint8_t pt = tab[ex.d];
-								bool ok = (pt == 1);
-								if(pt == 2)
-									ok = (ex.e >= prm.scg_min_size) && (cl.totLen - ex.e >= prm.scg_min_size);
-								if(ok) {
-									best.found = 1; best.k1 = score; best.p = p; best.i0 = TP; best.i1 = tot; best.i2 = u;
-								}
-							}
-						}
-					}
-				}
-				else {
-					// ...SplitScafs.cpp:131-154
-					const uint32_t belong1 = ex.a, in1 = ex.b, belong2 = n - ex.c, in2 = cl.U - ex.d;
-					if(belong1 >= prm.thr && belong2 >= prm.thr) {
-						const uint32_t separated = cl.U - in1 - in2;
-						const uint32_t in_small = (p < n - p)? in1 : in2, in_large = (p < n - p)? in2 : in1;
-						const double ratio = __ddiv_rn((double)separated, (double)(int)in_small);
-						double csr = __ddiv_rn((double)(int)in_small, (double)(int)in_large);
-						if(csr < 1)
-							csr = __ddiv_rn(1.0, csr);
-						if(!best.found || ratio < best.k1 || (ratio == best.k1 && csr < best.k2)) {
-							best.found = 1; best.k1 = ratio; best.k2 = csr; best.p = p; best.i0 = separated; best.i1 = in_small; best.i2 = in_large;
-						}
+				// ...SplitScafs.cpp:131-154
+				const uint32_t belong1 = ex.a, in1 = ex.b, belong2 = n - ex.c, in2 = cl.U - ex.d;
+				if(belong1 >= prm.thr && belong2 >= prm.thr) {
+					const uint32_t separated = cl.U - in1 - in2;
+					const uint32_t in_small = (p < n - p)? in1 : in2, in_large = (p < n - p)? in2 : in1;
+					const double ratio = __ddiv_rn((double)separated, (double)(int)in_small);
+					double csr = __ddiv_rn((double)(int)in_small, (double)(int)in_large);
+					if(csr < 1)
+						csr = __ddiv_rn(1.0, csr);
+					if(!best.found || ratio < best.k1 || (ratio == best.k1 && csr < best.k2)) {
+						best.found = 1; best.k1 = ratio; best.k2 = csr; best.p = p; best.i0 = separated; best.i1 = in_small; best.i2 = in_large;
 					}
 				}
 			}
-			ex = agg_add(ex, contribution<STRATEGY>(el[j], i0 + j < n, rows, prm.fraction_in));
+			ex = agg_add(ex, contribution(el[j], i0 + j < n, rows, prm.fraction_in));
 		}
-		block_best_out<STRATEGY>(best, d, sm_best, out, w);
+		block_best_out<ABW_SPLIT_SCAFS>(best, d, sm_best, out, w);
 		__syncthreads();
 	}
 }
@@ -465,15 +374,8 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep(const uint32_t* __restr
 // ---------------------------------------------------------------------------------------------------
 constexpr int SW_WARP_CHUNK = 32 * 32;            // elements per warp: 32 rows of 32
 
-// look-back word of the sweep: two counts below 2^28 (a problem holds fewer than 2^28 datapoints), the epoch of the level (6 bits) and the state
-__device__ __forceinline__ unsigned long long cnt_pack(uint32_t nf, uint32_t nc, uint32_t st, uint32_t epoch)
-{
-	return (unsigned long long)nf | ((unsigned long long)nc << 28) | ((unsigned long long)(epoch & 63u) << 56) | ((unsigned long long)st << 62);
-}
-__device__ __forceinline__ uint32_t cnt_state(unsigned long long v, uint32_t epoch)
-{
-	return (((uint32_t)(v >> 56) & 63u) == (epoch & 63u))? (uint32_t)(v >> 62) : LB_EMPTY;
-}
+// payload of the sweep's packed look-back word (lb_pack): two counts below 2^28 (a problem holds fewer than 2^28 datapoints)
+__device__ __forceinline__ unsigned long long cnt_payload(uint32_t nf, uint32_t nc) { return (unsigned long long)nf | ((unsigned long long)nc << 28); }
 
 // Tables of a level, per (cluster, dimension), indexed by the number k of flip elements already passed:
 //   F8[k-1]  = sums over the first k flips: x = T/2+1 (TP brought by the flips), y = T;  FC[k-1] = n (only kept when some scaffold has n < T)
@@ -683,48 +585,18 @@ __global__ void __launch_bounds__(SW_THREADS, ABW_SWEEP_CTAS) k_sweep_ss(const u
 			uint32_t cF = 0, cC = 0;
 			if(tile > 0) {
 				if(lane == 0)
-					st_volatile_u64(&lookback[w], cnt_pack(totF, totC, LB_AGG, epoch));
-				uint64_t base = w - 1;
-				uint32_t remaining = tile;
-				bool done = false, failed = false;
-				while(!done && !failed) {
-					const uint32_t cnt = min(32u, remaining);
-					unsigned long long v;
-					uint32_t first_prefix, spins = 0;
-					while(true) {
-						v = ((uint32_t)lane < cnt)? ld_volatile_u64(&lookback[base - lane]) : cnt_pack(0, 0, LB_AGG, epoch);
-						const uint32_t st = cnt_state(v, epoch);
-						const uint32_t pm = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == LB_PREFIX);
-						const uint32_t em = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == LB_EMPTY);
-						first_prefix = pm? (uint32_t)(__ffs(pm) - 1) : 32u;
-						const uint32_t need = (first_prefix >= 32u)? 0xFFFFFFFFu : ((2u << first_prefix) - 1u);
-						if((em & need) == 0)
-							break;
-						if(++spins >= LB_SPIN_LIMIT) {
-							failed = true;
-							break;
-						}
-					}
-					if(failed)
-						break;
-					const bool take = (uint32_t)lane < cnt && (uint32_t)lane <= first_prefix;
-					uint32_t vf = take? (uint32_t)(v & 0xFFFFFFFull) : 0u, vc = take? (uint32_t)((v >> 28) & 0xFFFFFFFull) : 0u;
-					vf = __reduce_add_sync(0xffffffffu, vf);
-					vc = __reduce_add_sync(0xffffffffu, vc);
-					cF += vf;
-					cC += vc;
-					if(first_prefix < 32u)
-						done = true;
-					else {
-						base -= 32;
-						remaining -= 32;
-					}
-				}
-				if(failed && lane == 0)
+					st_volatile_u64(&lookback[w], lb_pack(cnt_payload(totF, totC), LB_AGG, epoch));
+				const bool ok = lb_walk(w, tile, [&](uint64_t i) { return ld_volatile_u64(&lookback[i]); },
+				                        [&](unsigned long long v) { return lb_packed_state(v, epoch); },
+				                        [&](unsigned long long v, uint64_t, bool take, uint32_t) {
+					cF += __reduce_add_sync(0xffffffffu, take? (uint32_t)(v & 0xFFFFFFFull) : 0u);
+					cC += __reduce_add_sync(0xffffffffu, take? (uint32_t)((v >> 28) & 0xFFFFFFFull) : 0u);
+				});
+				if(!ok && lane == 0)
 					atomicExch(&ctl->error, 1u);
 			}
 			if(lane == 0) {
-				st_volatile_u64(&lookback[w], cnt_pack(cF + totF, cC + totC, LB_PREFIX, epoch));
+				st_volatile_u64(&lookback[w], lb_pack(cnt_payload(cF + totF, cC + totC), LB_PREFIX, epoch));
 				sm_carry[0] = cF;
 				sm_carry[1] = cC;
 			}
@@ -1610,11 +1482,8 @@ __device__ __forceinline__ uint32_t ht_compose(uint32_t first, uint32_t then)
 // pending state (bit 0: child 1, bit 1: child 2) after a run with summary ht entered in `state`
 __device__ __forceinline__ uint32_t ht_apply(uint32_t ht, uint32_t state) { return ((ht >> 2) | (state & ~ht)) & 3u; }
 
-// look-back word of the partition: count of child-1 elements, summary bits, the epoch of the level (6 bits), state
-__device__ __forceinline__ unsigned long long lb2_pack(uint32_t cnt, uint32_t ht, uint32_t st, uint32_t epoch)
-{
-	return (unsigned long long)cnt | ((unsigned long long)ht << 32) | ((unsigned long long)(epoch & 63u) << 56) | ((unsigned long long)st << 62);
-}
+// payload of the partition's packed look-back word (lb_pack): count of child-1 elements, summary bits (an inclusive prefix has the pending state there)
+__device__ __forceinline__ unsigned long long lb2_payload(uint32_t cnt, uint32_t ht) { return (unsigned long long)cnt | ((unsigned long long)ht << 32); }
 
 struct PartPlans {
 	const uint32_t* in[4];
@@ -1622,7 +1491,7 @@ struct PartPlans {
 	uint64_t        stride[4];
 };
 
-// resident CTAs per SM of the three look-back kernels, measured on B200 (cfg2, 13 levels; registers are capped accordingly and a few values spill):
+// resident CTAs per SM of the three look-back kernels of a sens/spec search level, measured on B200 (cfg2, 13 levels; registers are capped accordingly and a few values spill):
 //   k_partition2 3 -> 4: 1625 -> 1500 us;  k_sweep_ss 4 -> 5 -> 6: 1222 -> 1159 -> 1135 us;  k_flip_prefix 4 -> 5 -> 6: 1150 -> 1088 -> 1217 us
 #ifndef ABW_PART_CTAS
 #define ABW_PART_CTAS 4
@@ -1727,34 +1596,13 @@ __global__ void __launch_bounds__(SW_THREADS, ABW_PART_CTAS) k_partition2(const 
 			uint32_t carry_cnt = 0, carry_state = 3u;          // the first element of each child gets its boundary flag set
 			if(tile > 0) {
 				if(lane == 0)
-					st_volatile_u64(&lookback[w], lb2_pack(rc, rh, LB_AGG, epoch));
-				uint32_t acc = 0;                               // summary of the tiles between the probe window and this tile
-				uint64_t base = w - 1;
-				uint32_t remaining = tile;
-				bool done = false, failed = false;
-				while(!done && !failed) {
-					const uint32_t cnt = min(32u, remaining);
-					unsigned long long v;
-					uint32_t first_prefix, spins = 0;
-					while(true) {
-						v = ((uint32_t)lane < cnt)? ld_volatile_u64(&lookback[base - lane]) : lb2_pack(0, 0, LB_AGG, epoch);
-						const uint32_t st = cnt_state(v, epoch);
-						const uint32_t pm = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == LB_PREFIX);
-						const uint32_t em = __ballot_sync(0xffffffffu, (uint32_t)lane < cnt && st == LB_EMPTY);
-						first_prefix = pm? (uint32_t)(__ffs(pm) - 1) : 32u;
-						const uint32_t need = (first_prefix >= 32u)? 0xFFFFFFFFu : ((2u << first_prefix) - 1u);
-						if((em & need) == 0)
-							break;
-						if(++spins >= LB_SPIN_LIMIT) {
-							failed = true;
-							break;
-						}
-					}
-					if(failed)
-						break;
-					const bool take = (uint32_t)lane < cnt && (uint32_t)lane <= first_prefix;
+					st_volatile_u64(&lookback[w], lb_pack(lb2_payload(rc, rh), LB_AGG, epoch));
+				uint32_t acc = 0;                               // summary of the tiles between the window and this tile
+				const bool ok = lb_walk(w, tile, [&](uint64_t i) { return ld_volatile_u64(&lookback[i]); },
+				                        [&](unsigned long long v) { return lb_packed_state(v, epoch); },
+				                        [&](unsigned long long v, uint64_t, bool take, uint32_t first_prefix) {
 					carry_cnt += __reduce_add_sync(0xffffffffu, take? (uint32_t)v : 0u);
-					// summaries compose in tile order: lane l holds tile base - l, i.e. higher lanes are EARLIER tiles.  Suffix-compose towards lane 0.
+					// summaries compose in tile order and higher lanes are EARLIER tiles: suffix-compose towards lane 0
 					uint32_t h = (take && (uint32_t)lane != first_prefix)? ((uint32_t)(v >> 32) & 0xFu) : 0u;      // identity for lanes that do not take part
 #pragma unroll
 					for(int o = 1; o < 32; o <<= 1) {
@@ -1766,19 +1614,15 @@ __global__ void __launch_bounds__(SW_THREADS, ABW_PART_CTAS) k_partition2(const 
 					if(first_prefix < 32u) {
 						const uint32_t state_at_prefix = (uint32_t)(__shfl_sync(0xffffffffu, v, (int)first_prefix) >> 32) & 3u;
 						carry_state = ht_apply(acc, ht_apply(window, state_at_prefix));
-						done = true;
 					}
-					else {
+					else
 						acc = ht_compose(window, acc);
-						base -= 32;
-						remaining -= 32;
-					}
-				}
-				if(failed && lane == 0)
+				});
+				if(!ok && lane == 0)
 					atomicExch(&ctl->error, 1u);
 			}
 			if(lane == 0)
-				st_volatile_u64(&lookback[w], lb2_pack(carry_cnt + rc, ht_apply(rh, carry_state), LB_PREFIX, epoch));
+				st_volatile_u64(&lookback[w], lb_pack(lb2_payload(carry_cnt + rc, ht_apply(rh, carry_state)), LB_PREFIX, epoch));
 			if(lane < SW_THREADS / 32) {
 				sm_cnt[lane] = carry_cnt + wc;                  // child-1 elements before warp `lane`
 				sm_ht[lane] = ht_apply(wh, carry_state);        // pending state when warp `lane` starts
@@ -2795,7 +2639,7 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 			           Sf, d_tab.p, sp, ep_sweep, d_lookback.p, d_cand.p);
 		}
 		else
-			ABW_LAUNCH(ctx, k_sweep<ABW_SPLIT_SCAFS>, g_sweep, SW_THREADS, 0, s->E[cur].p, N, d_cl[cur].p, D, d_ctl.p, d_tile_tab.p, s->rows.p, (const uint8_t*)nullptr, sp,
+			ABW_LAUNCH(ctx, k_sweep_split_scafs, g_sweep, SW_THREADS, 0, s->E[cur].p, N, d_cl[cur].p, D, d_ctl.p, d_tile_tab.p, s->rows.p, sp,
 			           ep_sweep, d_status.p, d_aggs.p, d_prefixes.p, d_cand.p);
 		s->prof.sweep_ms += tm.stop();
 		tm.start();
@@ -2950,7 +2794,7 @@ int abw_search_create(abw_ctx* ctx, const double* values, int values_on_device, 
 		return abw_fail(ctx, ABW_ERR_ARG, "abw_search_create: empty problem");
 	if(W > SCG_WMAX)
 		return abw_fail(ctx, ABW_ERR_UNSUPPORTED, "abw_search_create: at most 512 distinct SCG names (W <= 8)");
-	if(N >= (1ull << 28) || S >= (1u << EL_SCAF_BITS))       // the look-back words of the sweep carry two 28-bit counts (cnt_pack)
+	if(N >= (1ull << 28) || S >= (1u << EL_SCAF_BITS))       // the look-back words of the sweep carry two 28-bit counts (cnt_payload)
 		return abw_fail(ctx, ABW_ERR_UNSUPPORTED, "abw_search_create: at most 2^28-1 datapoints and 2^27-1 scaffolds per device");
 	if(!h_row_of_dp)
 		nrows = N;

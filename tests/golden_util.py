@@ -141,3 +141,46 @@ def coverage_edge_workload(seed=7, nscaf=160, nsamples=3, depth=40, cover_all_n=
         extra["scaf"], extra["pos0"], extra["len"] = len(lens) - 1, [0, 250], 300
         reads[-1] = np.concatenate([reads[-1], extra])
     return seq, offsets, reads
+
+
+def _random_problem(rng, S, D, partial=False, ties=True, scg=True, nclus=3):
+    """Seeded random split-search problem of S scaffolds (T in 2..8 datapoints each, n = T unless partial) in D dimensions around nclus centres."""
+    T = rng.integers(2, 9, S).astype(np.uint32)
+    n = T.copy()
+    if partial:
+        drop = rng.random(S) < 0.3
+        n = np.where(drop, np.maximum(1, T - rng.integers(1, 4, S)), T).astype(np.uint32)
+    dp2scaf = np.repeat(np.arange(S, dtype=np.uint32), n)
+    N = dp2scaf.size
+    grp = rng.integers(0, nclus, S)
+    centers = rng.normal(0, 1.0, (nclus, D))
+    vals = centers[grp[dp2scaf]].T + rng.normal(0, 0.35, (D, N))
+    if ties:
+        vals = np.round(vals, 1)             # heavy ties, negative values and +-0.0
+        vals[vals == 0] = np.where(rng.random((vals == 0).sum()) < 0.5, 0.0, -0.0)
+    length = rng.integers(2000, 400000, S).astype(np.uint64)
+    W = 2
+    mask = np.zeros((S, W), dtype=np.uint64)
+    if scg:
+        for g in range(70):
+            for c in range(nclus):
+                if rng.random() < 0.8:
+                    cand = np.nonzero(grp == c)[0]
+                    if cand.size:
+                        s = cand[rng.integers(0, cand.size)]
+                        mask[s, g // 64] |= np.uint64(1) << np.uint64(g % 64)
+    return np.ascontiguousarray(vals), dp2scaf, T, length, mask
+
+
+def assert_search_matches_oracle(orecs, odp, osc, res):
+    """A device search (pipeline.search) gives every cluster record, dp2cluster and scaf2cluster of the oracle's run (abwo.Search.run)."""
+    assert len(orecs) == len(res.recs)
+    for o, r in zip(orecs, res.recs):
+        assert (o.id, o.parent, o.ndps, o.nscafs, o.split) == (r.id, r.parent, r.ndps, r.nscafs, r.split)
+        assert (o.best.found, o.best.dim, o.best.value, o.best.a, o.best.legal) == (r.best.found, r.best.dim, r.best.value, r.best.a, r.best.legal), (o.id, o.best.b, r.best.b)
+        assert o.best.b == r.best.b
+        assert (o.child1, o.child2, o.child1_ndps, o.child2_ndps, o.child1_nscafs, o.child2_nscafs, o.child1_raw, o.child2_raw) == \
+               (r.child1, r.child2, r.child1_ndps, r.child2_ndps, r.child1_nscafs, r.child2_nscafs, r.child1_raw, r.child2_raw)
+        assert (o.total_size, o.scg_unique, o.scg_avg) == (r.total_size, r.scg_unique, r.scg_avg)
+    assert odp.tolist() == res.dp2cluster.tolist()
+    assert osc.tolist() == res.scaf2cluster.tolist()
