@@ -28,10 +28,9 @@ struct abw_ctx {
 	// device blocks freed by this context, kept for reuse (see abw_arena_alloc): capacity -> block
 	std::multimap<size_t, void*> free_blocks;
 	std::map<void*, size_t> block_cap;                         // capacity of every block obtained through the arena, cached or in use
-	// pinned staging for the many small host->device uploads of a search level: two halves used alternately (see abw_stage_flip)
+	// pinned staging for small host->device uploads (abw_upload_small), free again after every abw_sync
 	unsigned char* h_stage = nullptr;
-	size_t stage_half = 0, stage_used = 0;
-	int stage_side = 0;
+	size_t stage_cap = 0, stage_used = 0;
 	// small device->host results fetched by a kernel into mapped pinned memory instead of through the copy engine (abw_fetch, abw_sync)
 	struct Fetch { void* h_dst; const unsigned char* slot; size_t bytes; };
 	unsigned char* h_bounce = nullptr;
@@ -47,26 +46,21 @@ struct abw_ctx {
 	uint32_t* scan_failed = nullptr;          // mapped pinned word: set by a prefix sum whose look-back wait gave up, reported and cleared by abw_sync
 };
 
-// Small uploads (descriptors, job lists, tile tables) go through pinned memory so that cudaMemcpyAsync really is asynchronous.
-// abw_stage_flip switches to the other half; the caller guarantees that the copies enqueued two flips ago have completed
-// (the split search synchronises at least once per level and flips once per level).
-void abw_stage_flip(abw_ctx* ctx);
-cudaError_t abw_stage_upload(abw_ctx* ctx, void* d_dst, const void* h_src, size_t bytes);
-
 // Small transfers and the copy engines.  Copies of one direction execute in the order they were issued, whatever their stream: an 8-byte
 // cudaMemcpyAsync on the compute stream waits for every bulk copy (read records in, .lrn matrix out) that was enqueued before it on the copy
 // stream, and the kernels behind it wait too -- measured: end-to-end step = H2D + resident step + D2H, no overlap at all (DESIGN.md section 5).
-// Therefore the small transfers bypass the engines: abw_stage_upload lets a kernel read the pinned staging slot, and
-// abw_fetch lets a kernel write the result into mapped pinned memory, from where abw_sync (cudaStreamSynchronize + copy-out) hands it to the
-// caller's buffer.  ABW_SMALL_COPIES=memcpy selects plain cudaMemcpyAsync (the round-1 behaviour).  Every device->host result of an entry point
-// is requested with abw_fetch and every wait on the context stream is abw_sync; ABW_ENTER drops requests an earlier, failed call may have left behind.
+// Therefore the small transfers bypass the engines, in both directions through pinned memory and a copy kernel on the context stream:
+//  * abw_upload_small (descriptors, job lists, tile tables) copies h_src into the pinned staging area, from where a kernel reads it.  An upload that
+//    does not fit, or any upload when the pinned allocation failed, is a cudaMemcpyAsync from h_src.
+//  * abw_fetch has a kernel write the result into mapped pinned memory, from where abw_sync (cudaStreamSynchronize + copy-out) hands it to the
+//    caller's buffer.
+// Every device->host result of an entry point is requested with abw_fetch and every wait on the context stream is abw_sync.  Once abw_sync has drained
+// the stream, no copy kernel reads or writes a slot any more, so abw_sync makes the whole staging area and bounce buffer free again; ABW_ENTER
+// drops fetch requests an earlier, failed call may have left behind.
 // abw_sync also fails (cudaErrorTimeout) when a prefix sum enqueued since the previous abw_sync gave up a look-back wait: its results are wrong.
-bool abw_small_copies_by_kernel();
+cudaError_t abw_upload_small(abw_ctx* ctx, void* d_dst, const void* h_src, size_t bytes);
 cudaError_t abw_fetch(abw_ctx* ctx, void* h_dst, const void* d_src, size_t bytes);
 cudaError_t abw_sync(abw_ctx* ctx);
-// host->device upload of a small array on the context stream: cudaMemcpyAsync by default, through the pinned staging area and a kernel (cudaMemcpyAsync with
-// ABW_SMALL_COPIES=memcpy) (the caller waits for the stream before it changes h_src or returns)
-cudaError_t abw_upload_small(abw_ctx* ctx, void* d_dst, const void* h_src, size_t bytes);
 
 inline int abw_fail(abw_ctx* ctx, int code, const std::string& msg)
 {

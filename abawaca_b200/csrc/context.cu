@@ -122,19 +122,6 @@ cudaError_t abw_arena_alloc(abw_ctx* ctx, size_t bytes, void** out)
 	return cudaSuccess;
 }
 
-void abw_stage_flip(abw_ctx* ctx)
-{
-	ctx->stage_side ^= 1;
-	ctx->stage_used = 0;
-}
-
-bool abw_small_copies_by_kernel()
-{
-	// default since round 2 (GPU suite green with it, end-to-end step 72.7 -> 63.9 ms); ABW_SMALL_COPIES=memcpy selects plain cudaMemcpyAsync
-	static const bool on = [] { const char* e = getenv("ABW_SMALL_COPIES"); return !(e && strcmp(e, "memcpy") == 0); }();
-	return on;
-}
-
 // bytes from src to dst, one of them mapped pinned host memory; word-wise when both are 4-byte aligned
 __global__ void k_copy_small(unsigned char* __restrict__ dst, const unsigned char* __restrict__ src, size_t bytes)
 {
@@ -164,7 +151,7 @@ cudaError_t abw_fetch(abw_ctx* ctx, void* h_dst, const void* d_src, size_t bytes
 {
 	if(bytes == 0)
 		return cudaSuccess;
-	if(abw_small_copies_by_kernel() && bytes <= ((size_t)256 << 10)) {
+	if(bytes <= ((size_t)256 << 10)) {
 		if(!ctx->h_bounce) {
 			ctx->bounce_cap = (size_t)2 << 20;
 			if(cudaHostAlloc((void**)&ctx->h_bounce, ctx->bounce_cap, cudaHostAllocMapped) != cudaSuccess) {
@@ -196,40 +183,30 @@ cudaError_t abw_sync(abw_ctx* ctx)
 			memcpy(f.h_dst, f.slot, f.bytes);
 	ctx->pending.clear();
 	ctx->bounce_used = 0;
+	ctx->stage_used = 0;
 	return e;
-}
-
-cudaError_t abw_stage_upload(abw_ctx* ctx, void* d_dst, const void* h_src, size_t bytes)
-{
-	if(bytes == 0)
-		return cudaSuccess;
-	if(!ctx->h_stage) {
-		ctx->stage_half = (size_t)4 << 20;
-		if(cudaMallocHost((void**)&ctx->h_stage, 2 * ctx->stage_half) != cudaSuccess) {
-			cudaGetLastError();
-			ctx->h_stage = nullptr;
-			ctx->stage_half = 0;
-		}
-	}
-	const size_t need = (bytes + 255) & ~(size_t)255;
-	if(ctx->h_stage && ctx->stage_used + need <= ctx->stage_half) {
-		unsigned char* slot = ctx->h_stage + (size_t)ctx->stage_side * ctx->stage_half + ctx->stage_used;
-		memcpy(slot, h_src, bytes);
-		ctx->stage_used += need;
-		if(abw_small_copies_by_kernel())
-			return copy_small(ctx, d_dst, slot, bytes);        // pinned memory is mapped into the device's address space (unified addressing)
-		return cudaMemcpyAsync(d_dst, slot, bytes, cudaMemcpyHostToDevice, ctx->stream);
-	}
-	return cudaMemcpyAsync(d_dst, h_src, bytes, cudaMemcpyHostToDevice, ctx->stream);      // too large for the staging half: the driver stages it
 }
 
 cudaError_t abw_upload_small(abw_ctx* ctx, void* d_dst, const void* h_src, size_t bytes)
 {
 	if(bytes == 0)
 		return cudaSuccess;
-	if(abw_small_copies_by_kernel())
-		return abw_stage_upload(ctx, d_dst, h_src, bytes);     // falls back to cudaMemcpyAsync when the staging half is full
-	return cudaMemcpyAsync(d_dst, h_src, bytes, cudaMemcpyHostToDevice, ctx->stream);
+	if(!ctx->h_stage) {
+		ctx->stage_cap = (size_t)4 << 20;
+		if(cudaMallocHost((void**)&ctx->h_stage, ctx->stage_cap) != cudaSuccess) {
+			cudaGetLastError();
+			ctx->h_stage = nullptr;
+			ctx->stage_cap = 0;
+		}
+	}
+	const size_t need = (bytes + 255) & ~(size_t)255;
+	if(ctx->h_stage && ctx->stage_used + need <= ctx->stage_cap) {
+		unsigned char* slot = ctx->h_stage + ctx->stage_used;
+		memcpy(slot, h_src, bytes);
+		ctx->stage_used += need;
+		return copy_small(ctx, d_dst, slot, bytes);            // pinned memory is mapped into the device's address space (unified addressing)
+	}
+	return cudaMemcpyAsync(d_dst, h_src, bytes, cudaMemcpyHostToDevice, ctx->stream);      // does not fit the staging area: the driver stages it
 }
 
 void abw_arena_free(abw_ctx* ctx, void* p)

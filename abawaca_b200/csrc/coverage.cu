@@ -583,7 +583,7 @@ __global__ void k_cov_zero_columns(double* __restrict__ rows, uint64_t nseg, uin
 }
 
 // pass 2 for the samples [0, ns) of a group whose ReadSrc records are at d_srcs
-int coverage_pairs(abw_ctx* ctx, const abw_segments* g, const ReadSrc* d_srcs, uint32_t ns, uint32_t max_tiles, uint32_t total_tiles, uint32_t max_snps, int kind,
+int coverage_pairs(abw_ctx* ctx, const abw_segments* g, const ReadSrc* d_srcs, uint32_t ns, uint32_t total_tiles, uint32_t max_snps, int kind,
                    double* d_rows, uint64_t ld, uint32_t col0, bool all, const uint32_t* flags, uint32_t nwords, const uint32_t* nflagged, const uint2* tile_range,
                    unsigned long long* d_scaf_nbps, int nbps_sample)
 {
@@ -600,7 +600,6 @@ int coverage_pairs(abw_ctx* ctx, const abw_segments* g, const ReadSrc* d_srcs, u
 	ABW_CUDA(ctx, cudaMemsetAsync(nlist.p, 0, sizeof(uint32_t), ctx->stream));
 	ABW_LAUNCH(ctx, k_cov_tile_filter, abw_div_up(total_tiles, 256), 256, 0, d_srcs, ns, total_tiles, flags, nwords, nflagged, tile_range, all? 1 : 0, tile_counts.p, list.p,
 	           nlist.p);
-	(void)max_tiles;
 	const unsigned int grid = std::min<unsigned int>(total_tiles, 8u * (unsigned)ctx->sm_count);
 	if(all)
 		ABW_LAUNCH(ctx, (k_cov_pairs<false, true>), grid, COV_THREADS, 0, d_srcs, max_snps, g->nscaf, g->scaf_info.p, g->seg_end.p, g->nseg, flags, nwords,
@@ -633,10 +632,8 @@ int coverage_pairs(abw_ctx* ctx, const abw_segments* g, const ReadSrc* d_srcs, u
 	// (sample, window) ids are dense: every bit below nbits is taken as varying, no inspection pass
 	ABW_CHECK(abw_radix_sort_pairs_u32(ctx, keys.p, keys_tmp.p, vals.p, vals_tmp.p, npairs, 1, npairs, -nbits));
 	const unsigned int blocks = abw_div_up(npairs, 128);
-	if(kind == ABW_FEAT_TRUNC3 && !all)
+	if(kind == ABW_FEAT_TRUNC3)
 		ABW_LAUNCH(ctx, (k_cov_accumulate<ABW_FEAT_TRUNC3, 16>), blocks, 128, 0, keys.p, vals.p, npairs, g->nseg, g->seg_start.p, g->seg_end.p, d_rows, ld, col0);
-	else if(kind == ABW_FEAT_TRUNC3)
-		ABW_LAUNCH(ctx, (k_cov_accumulate<ABW_FEAT_TRUNC3, 8>), blocks, 128, 0, keys.p, vals.p, npairs, g->nseg, g->seg_start.p, g->seg_end.p, d_rows, ld, col0);
 	else
 		ABW_LAUNCH(ctx, (k_cov_accumulate<ABW_FEAT_RAW, 8>), blocks, 128, 0, keys.p, vals.p, npairs, g->nseg, g->seg_start.p, g->seg_end.p, d_rows, ld, col0);
 	return ABW_OK;
@@ -647,9 +644,7 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 {
 	if(nsamples == 0 || g->nseg == 0)
 		return ABW_OK;
-	// ABW_COVERAGE_SORT_ALL=1: every read through the sort also for three-decimal output (the first formulation; the tests compare the two)
-	static const bool sort_all = [] { const char* e = getenv("ABW_COVERAGE_SORT_ALL"); return e && *e && *e != '0'; }();
-	const bool all = (kind != ABW_FEAT_TRUNC3) || sort_all;
+	const bool all = (kind == ABW_FEAT_RAW);
 	const uint32_t nwords = (uint32_t)((g->nseg + 31) / 32);
 	// samples are processed in groups: (sample, window) keys must fit 32 bits and the integer sums a few GB
 	const uint64_t by_key = std::max<uint64_t>(1, ((1ull << 32) - 1) / g->nseg), by_mem = std::max<uint64_t>(1, (4ull << 30) / (8 * g->nseg));
@@ -659,7 +654,7 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 		std::vector<ReadSrc> srcs(ns);
 		// sorted samples are decoded into compact records, which pass 2 reads again: they live until the end of the group
 		std::vector<DevBuf<abw_read8>> decoded(ns);
-		uint32_t total_tiles = 0, max_tiles = 0;
+		uint32_t total_tiles = 0;
 		for(uint32_t j = 0; j < ns; j++) {
 			const abw_sample& sm = samples[s0 + j];
 			ReadSrc& r = srcs[j];
@@ -672,7 +667,6 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 			r.tile0 = total_tiles;
 			r.ntiles = abw_div_up(sm.nreads, COV_TILE);
 			total_tiles += r.ntiles;
-			max_tiles = std::max(max_tiles, r.ntiles);
 		}
 		DevBuf<ReadSrc> d_srcs;
 		DevBuf<unsigned long long> sum_ov;
@@ -688,7 +682,7 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 				if(samples[s0 + j].format == ABW_READS_SORTED)
 					ABW_CHECK(abw_decode_sorted_reads(ctx, samples[s0 + j], decoded[j].p));
 			ABW_LAUNCH(ctx, k_cov_zero_columns, abw_div_up(g->nseg * ns, 256), 256, 0, d_rows, g->nseg, ld, col0 + s0, ns);
-			ABW_CHECK(coverage_pairs(ctx, g, d_srcs.p, ns, max_tiles, total_tiles, max_snps, kind, d_rows, ld, col0 + s0, true, nullptr, nwords, nullptr, nullptr,
+			ABW_CHECK(coverage_pairs(ctx, g, d_srcs.p, ns, total_tiles, max_snps, kind, d_rows, ld, col0 + s0, true, nullptr, nwords, nullptr, nullptr,
 			                         (unsigned long long*)d_scaf_nbps, nbps_local));
 			continue;
 		}
@@ -713,7 +707,7 @@ int coverage_batch(abw_ctx* ctx, const abw_segments* g, const abw_sample* sample
 		}
 		ABW_LAUNCH(ctx, k_cov_quotient, dim3(abw_div_up(g->nseg, 256), ns), 256, 0, sum_ov.p, g->nseg, g->seg_start.p, g->seg_end.p, d_rows, ld, col0 + s0, flags.p, nwords,
 		           nflagged.p);
-		ABW_CHECK(coverage_pairs(ctx, g, d_srcs.p, ns, max_tiles, total_tiles, max_snps, kind, d_rows, ld, col0 + s0, false, flags.p, nwords, nflagged.p, tile_range.p,
+		ABW_CHECK(coverage_pairs(ctx, g, d_srcs.p, ns, total_tiles, max_snps, kind, d_rows, ld, col0 + s0, false, flags.p, nwords, nflagged.p, tile_range.p,
 		                         nullptr, -1));
 	}
 	return ABW_OK;

@@ -513,8 +513,6 @@ static int pack_impl(abw_ctx* ctx, abw_seqset* s, const char* ascii, int ascii_o
 		src = d_ascii.p;
 		readable = bytes + 64;
 	}
-	if(abw_small_copies_by_kernel())
-		abw_stage_flip(ctx);                                   // this call waits for the stream before it returns: the half used two flips ago is free
 	ABW_CUDA(ctx, d_off.alloc((size_t)nscaf + 1));
 	ABW_CUDA(ctx, abw_upload_small(ctx, d_off.p, h_offsets, sizeof(uint64_t) * ((size_t)nscaf + 1)));
 	ABW_CUDA(ctx, s->len.alloc(nscaf));

@@ -85,8 +85,8 @@ struct LevelCtl {
 
 // what the host polls (mapped pinned memory): written by k_level_decide at the end of every level
 struct LevelProgress {
-	volatile uint32_t levels_done, done, nrec, error;
-	volatile uint32_t ticks, done_at, pad0, pad1;     // see LevelCtl; done_at is written before ticks
+	volatile uint32_t levels_done, done, error;
+	volatile uint32_t ticks, done_at;                 // see LevelCtl; done_at is written before ticks
 	volatile uint32_t c_next[16];                     // c_next[t & 15]: clusters of the level that follows the t-th executed level (t = 0, 1, ...)
 };
 
@@ -387,10 +387,10 @@ constexpr int FP_TILE = SW_THREADS * FP_ITEMS;
 // The per-scaffold records of a tile are staged in shared memory (coalesced list reads, the gathers of all eight entries of a thread in flight,
 // 16-byte slots swizzled so that both the strided stores and the blocked loads are conflict free) instead of living in registers across the
 // scan and the look-back: 40 registers instead of 128, six CTAs per SM instead of two.
-#ifndef ABW_FLIP_CTAS
-#define ABW_FLIP_CTAS 5
-#endif
-__global__ void __launch_bounds__(SW_THREADS, ABW_FLIP_CTAS) k_flip_prefix(const uint32_t* __restrict__ flip_list, uint64_t Sf, const LevelCluster* __restrict__ clusters, uint32_t D,
+// Resident CTAs per SM of the three look-back kernels of a sens/spec search level, measured on B200 (cfg2, 13 levels; registers are capped accordingly and a few values spill):
+//   k_partition2 3 -> 4: 1625 -> 1500 us;  k_sweep_ss 4 -> 5 -> 6: 1222 -> 1159 -> 1135 us;  k_flip_prefix 4 -> 5 -> 6: 1150 -> 1088 -> 1217 us
+constexpr int FLIP_CTAS = 5, SWEEP_CTAS = 6, PART_CTAS = 4;
+__global__ void __launch_bounds__(SW_THREADS, FLIP_CTAS) k_flip_prefix(const uint32_t* __restrict__ flip_list, uint64_t Sf, const LevelCluster* __restrict__ clusters, uint32_t D,
                                                               LevelCtl* __restrict__ ctl, const uint2* __restrict__ ftile_tab, const uint4* __restrict__ frow,
                                                               uint32_t epoch, uint32_t* __restrict__ status, AggSlot* __restrict__ aggs,
                                                               AggSlot* __restrict__ prefixes, uint2* __restrict__ F8, uint32_t* __restrict__ FC, uint32_t* __restrict__ scg_k,
@@ -503,10 +503,7 @@ __global__ void __launch_bounds__(SW_THREADS, ABW_FLIP_CTAS) k_flip_prefix(const
 	}
 }
 
-#ifndef ABW_SWEEP_CTAS
-#define ABW_SWEEP_CTAS 6
-#endif
-__global__ void __launch_bounds__(SW_THREADS, ABW_SWEEP_CTAS) k_sweep_ss(const uint32_t* __restrict__ E, uint64_t N, const LevelCluster* __restrict__ clusters, uint32_t D,
+__global__ void __launch_bounds__(SW_THREADS, SWEEP_CTAS) k_sweep_ss(const uint32_t* __restrict__ E, uint64_t N, const LevelCluster* __restrict__ clusters, uint32_t D,
                                                            LevelCtl* __restrict__ ctl, const uint2* __restrict__ tile_tab, const uint2* __restrict__ F8,
                                                            const uint32_t* __restrict__ FC, const uint32_t* __restrict__ scg_k, uint64_t Kstride,
                                                            const uint2* __restrict__ klohi, uint32_t Cstride, uint64_t Sf, const uint8_t* __restrict__ pass_tab,
@@ -1331,7 +1328,6 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_decide(const LevelBufs B, 
 		ctl->ticks++;
 		if(ctl->done && !ctl->done_at)
 			ctl->done_at = ctl->ticks;
-		B.prog->nrec = ctl->nrec;
 		B.prog->error = ctl->error;
 		B.prog->done = ctl->done;
 		B.prog->done_at = ctl->done_at;
@@ -1343,12 +1339,12 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_decide(const LevelBufs B, 
 }
 
 // pending clusters become bins without being evaluated (abw_search_set_max_levels): the children of the last level that was run
-__global__ void __launch_bounds__(LV_THREADS) k_pending_jobs(const LevelBufs B, int cur, uint32_t Cpend_from_P, uint32_t W)
+__global__ void __launch_bounds__(LV_THREADS) k_pending_jobs(const LevelBufs B, int cur, uint32_t W)
 {
 	__shared__ uint32_t sm[33];
 	LevelCtl* const ctl = B.ctl;
 	const LevelCluster* __restrict__ cls = B.cl[cur];
-	const uint32_t Tn = Cpend_from_P? 2 * ctl->P : ctl->C;
+	const uint32_t Tn = 2 * ctl->P;
 	for(uint32_t i = threadIdx.x; i < Tn; i += LV_THREADS) {
 		TermJob tj;
 		tj.sOff = cls[i].d.sOff; tj.ns = cls[i].d.ns; tj.id = cls[i].id; tj.rec = 0xFFFFFFFFu;
@@ -1491,12 +1487,7 @@ struct PartPlans {
 	uint64_t        stride[4];
 };
 
-// resident CTAs per SM of the three look-back kernels of a sens/spec search level, measured on B200 (cfg2, 13 levels; registers are capped accordingly and a few values spill):
-//   k_partition2 3 -> 4: 1625 -> 1500 us;  k_sweep_ss 4 -> 5 -> 6: 1222 -> 1159 -> 1135 us;  k_flip_prefix 4 -> 5 -> 6: 1150 -> 1088 -> 1217 us
-#ifndef ABW_PART_CTAS
-#define ABW_PART_CTAS 4
-#endif
-__global__ void __launch_bounds__(SW_THREADS, ABW_PART_CTAS) k_partition2(const PartPlans plans, LevelCtl* __restrict__ ctl, const PartJob* __restrict__ jobs_all,
+__global__ void __launch_bounds__(SW_THREADS, PART_CTAS) k_partition2(const PartPlans plans, LevelCtl* __restrict__ ctl, const PartJob* __restrict__ jobs_all,
                                                              const uint2* __restrict__ tab_all, const uint8_t* __restrict__ side, const uint8_t* __restrict__ new_assigned,
                                                              uint8_t* __restrict__ assigned, uint32_t epoch, unsigned long long* __restrict__ lookback)
 {
@@ -2124,15 +2115,6 @@ struct Trace {
 	}
 };
 
-template <typename T>
-int upload(abw_ctx* ctx, DevBuf<T>& buf, const std::vector<T>& h)
-{
-	ABW_CUDA(ctx, buf.alloc(h.size()));
-	if(!h.empty())
-		ABW_CUDA(ctx, cudaMemcpyAsync(buf.p, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice, ctx->stream));
-	return ABW_OK;
-}
-
 // The part of abw_search_create that starts from device arrays: s->vsrc (the matrix), d_T, d_len, s->scgmask, s->dp2scaf (when the caller gave one).
 // One host wait for the whole build when all dimensions fit one chunk of sort scratch: per-scaffold tables, their validation, the root statistics, the number
 // of SCG-carrying scaffolds and the key statistics of the first chunk are fetched together.
@@ -2519,7 +2501,7 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 		ABW_CUDA(ctx, cudaHostAlloc((void**)&ctx->h_prog, 256, cudaHostAllocMapped));
 	}
 	LevelProgress* const h_prog = reinterpret_cast<LevelProgress*>(ctx->h_prog);
-	h_prog->levels_done = 0; h_prog->done = 0; h_prog->nrec = 0; h_prog->error = 0; h_prog->ticks = 0; h_prog->done_at = 0;
+	h_prog->levels_done = 0; h_prog->done = 0; h_prog->error = 0; h_prog->ticks = 0; h_prog->done_at = 0;
 
 	// ---- root cluster and control block
 	{
@@ -2550,12 +2532,11 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 		std::vector<uint2> tt(c0.TT), ft(std::max<uint32_t>(c0.FPT, 1));
 		for(uint32_t t = 0; t < c0.TT; t++) tt[t] = make_uint2(0, t);
 		for(uint32_t t = 0; t < c0.FPT; t++) ft[t] = make_uint2(0, t);
-		abw_stage_flip(ctx);
-		ABW_CUDA(ctx, abw_stage_upload(ctx, d_cl[0].p, &root, sizeof(root)));
-		ABW_CUDA(ctx, abw_stage_upload(ctx, d_ctl.p, &c0, sizeof(c0)));
-		ABW_CUDA(ctx, abw_stage_upload(ctx, d_tile_tab.p, tt.data(), sizeof(uint2) * c0.TT));
+		ABW_CUDA(ctx, abw_upload_small(ctx, d_cl[0].p, &root, sizeof(root)));
+		ABW_CUDA(ctx, abw_upload_small(ctx, d_ctl.p, &c0, sizeof(c0)));
+		ABW_CUDA(ctx, abw_upload_small(ctx, d_tile_tab.p, tt.data(), sizeof(uint2) * c0.TT));
 		if(c0.FPT)
-			ABW_CUDA(ctx, abw_stage_upload(ctx, d_fp_tab.p, ft.data(), sizeof(uint2) * c0.FPT));
+			ABW_CUDA(ctx, abw_upload_small(ctx, d_fp_tab.p, ft.data(), sizeof(uint2) * c0.FPT));
 	}
 	LevelBufs B;
 	memset(&B, 0, sizeof(B));
@@ -2571,16 +2552,15 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 
 	// grids: CTAs walk the work items of a level, whatever their number turns out to be
 	const unsigned int sms = (unsigned int)ctx->sm_count;
-	const unsigned int g_sweep = (unsigned int)std::min<uint64_t>(items_max, (uint64_t)sms * ABW_SWEEP_CTAS), g_fp = (unsigned int)std::min<uint64_t>(std::max<uint64_t>(fp_items_max, 1), (uint64_t)sms * ABW_FLIP_CTAS);
-	const unsigned int g_part = (unsigned int)std::min<uint64_t>(part_items_max, (uint64_t)sms * ABW_PART_CTAS), g_small = sms * 4;
+	const unsigned int g_sweep = (unsigned int)std::min<uint64_t>(items_max, (uint64_t)sms * SWEEP_CTAS), g_fp = (unsigned int)std::min<uint64_t>(std::max<uint64_t>(fp_items_max, 1), (uint64_t)sms * FLIP_CTAS);
+	const unsigned int g_part = (unsigned int)std::min<uint64_t>(part_items_max, (uint64_t)sms * PART_CTAS), g_small = sms * 4;
 
 	// levels the host may run ahead of the device.  A sharded search must make the same number of collective calls on every rank, so there the decision
 	// to enqueue level l is a function of device state that is final when it is read: level l is enqueued iff the search had not ended by level
 	// l - lead (every rank waits until that level has been reported, then reads done_at, which is written once).  That enqueues lead - 1 empty levels
 	// (kernels that find no work, collectives over zeroes) after the last one, on every rank alike, and hides the host's round trip behind the
-	// kernels of lead - 1 levels.  ABW_SHARD_LEAD overrides (1 = wait for every level's verdict, the first formulation).
-	static const uint32_t shard_lead = [] { const char* e = getenv("ABW_SHARD_LEAD"); const int v = e? atoi(e) : 3; return (uint32_t)std::min(std::max(v, 1), 8); }();
-	const uint32_t lead = (world > 1)? shard_lead : 6u;
+	// kernels of lead - 1 levels.
+	const uint32_t lead = (world > 1)? 3u : 6u;
 	// side stream for k_finalize_terminal (not while kernels are timed one by one); its destructor makes the main stream wait, so that no buffer of this
 	// call returns to the block cache while a side kernel may still use it
 	struct SideStream {
@@ -2595,7 +2575,7 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 		}
 		~SideStream() { join(); }
 	} side{ctx};
-	if(!ctx->profiling && !getenv("ABW_NO_SIDE_STREAM")) {
+	if(!ctx->profiling) {
 		if(!ctx->side_stream) {
 			ABW_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->side_stream, cudaStreamNonBlocking));
 			ABW_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming));
@@ -2752,7 +2732,7 @@ int search_run(abw_ctx* ctx, abw_search* s, const abw_collectives* coll, abw_clu
 		return abw_fail(ctx, ABW_ERR_CUDA, "abw_search_run: internal error, a look-back wait timed out");
 	if(!h_ctl.done && max_levels > 0 && h_ctl.level >= max_levels && h_ctl.P > 0) {
 		// level limit reached: the pending clusters (the children written by the last level) are reported as bins (their ids) without being evaluated
-		ABW_LAUNCH(ctx, k_pending_jobs, 1, LV_THREADS, 0, B, cur, 1u, W);
+		ABW_LAUNCH(ctx, k_pending_jobs, 1, LV_THREADS, 0, B, cur, W);
 		ABW_LAUNCH(ctx, k_finalize_terminal, g_small, 128, 0, s->scaf_list[cur].p, B, s->rows.p, s->assigned.p, s->scgmask.p, W, s->scaf_member.p, s->scaf_final.p,
 		           (const double*)nullptr, (const double*)nullptr);
 	}
