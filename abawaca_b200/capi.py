@@ -24,6 +24,8 @@ READ_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4"), ("len", "<u4"), ("flag_
 READ8_DTYPE = np.dtype([("scaf", "<u4"), ("pos0", "<u4")])      # abw_read8: reads the host parser already filtered
 READ_RUN_DTYPE = np.dtype([("scaf", "<u4"), ("count", "<u4")])   # abw_read_run: `count` consecutive reads on scaffold `scaf` (sorted format)
 READS_FULL, READS_COMPACT, READS_SORTED = 0, 1, 2
+BASE_RUN_DTYPE = np.dtype([("scaf", "<u4"), ("start", "<u4"), ("len", "<u4"), ("kind", "<u4")])   # abw_base_run
+BASE_N, BASE_OTHER = 0, 1
 
 
 class AbwError(RuntimeError):
@@ -55,6 +57,12 @@ class Sample(C.Structure):
                 ("runs", C.c_void_p), ("nruns", C.c_uint64), ("exc", C.c_void_p), ("nexc", C.c_uint64)]
 
 
+class TwoBitAssembly(C.Structure):
+    """abw_2bit_assembly"""
+    _fields_ = [("codes", C.c_void_p), ("nbytes", C.c_uint64), ("h_byte_off", C.c_void_p), ("h_len", C.c_void_p), ("runs", C.c_void_p), ("nruns", C.c_uint64),
+                ("h2d_ticket", C.c_uint64)]
+
+
 class SearchProfile(C.Structure):
     _fields_ = [("build_ms", C.c_float), ("sweep_ms", C.c_float), ("partition_ms", C.c_float), ("other_ms", C.c_float),
                 ("sweep_elements", C.c_uint64), ("partition_elements", C.c_uint64), ("levels", C.c_uint32), ("sweep_launches", C.c_uint32)]
@@ -77,6 +85,7 @@ EXPORTS = [
     "abw_search_set_shard", "abw_search_set_shard_strided", "abw_search_set_max_levels", "abw_search_run_sharded", "abw_search_get_profile", "abw_cluster_scg",
     "abw_names_create", "abw_names_destroy", "abw_parse_sam", "abw_fasta_scan", "abw_fasta_destroy", "abw_fasta_count", "abw_fasta_get", "abw_fasta_pack", "abw_nccl_unique_id", "abw_nccl_collectives_create", "abw_nccl_collectives_destroy", "abw_peer_buffer_create", "abw_peer_buffer_destroy", "abw_peer_group_create", "abw_peer_group_destroy",
     "abw_scatter_columns_milli", "abw_parse_lrn", "abw_gather_rows", "abw_format_lrn", "abw_search_set_scaffold_stats",
+    "abw_pack_2bit", "abw_twobit_scan", "abw_twobit_destroy", "abw_twobit_count", "abw_twobit_get", "abw_twobit_decode", "abw_twobit_pack",
 ]
 
 
@@ -145,6 +154,15 @@ def load():
     L.abw_fasta_count.restype = C.c_uint64
     L.abw_fasta_get.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.abw_fasta_pack.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
+    L.abw_pack_2bit.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
+    L.abw_twobit_scan.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_void_p)]
+    L.abw_twobit_destroy.argtypes = [C.c_void_p]
+    L.abw_twobit_destroy.restype = None
+    L.abw_twobit_count.argtypes = [C.c_void_p]
+    L.abw_twobit_count.restype = C.c_uint64
+    L.abw_twobit_get.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.abw_twobit_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
+    L.abw_twobit_pack.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
     L.abw_nccl_unique_id.argtypes = [C.c_void_p, C.c_void_p]
     L.abw_nccl_collectives_create.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     L.abw_nccl_collectives_destroy.argtypes = [C.c_void_p]

@@ -202,7 +202,15 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 		}
 	}
 	// assembly
-	M.fasta = read_fasta(P.fasta_file);
+	{
+		std::string bytes = read_file(P.fasta_file);
+		if(is_twobit(bytes))
+			M.fasta = read_twobit(ctx, P.fasta_file, bytes);
+		else {
+			std::string().swap(bytes);
+			M.fasta = read_fasta(P.fasta_file);
+		}
+	}
 	M.scaf_seq.assign(M.S(), nullptr);
 	M.scaf_cvg.assign(M.S(), 0);
 	for(auto& r : M.fasta) {

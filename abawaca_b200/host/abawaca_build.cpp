@@ -1,6 +1,7 @@
 // abawaca-build (B200): same command line and same output files as the reference program
 // (/root/reference/src/abawaca-build.cpp main, :434-634), with the feature stage on the device:
-//   SeqIORead_fasta::next_seq       -> abw_fasta_scan / abw_fasta_pack (the FASTA text goes to the device as it is)
+//   SeqIORead_fasta::next_seq       -> abw_fasta_scan / abw_fasta_pack (the FASTA text goes to the device as it is), or for a UCSC .2bit
+//                                      file abw_twobit_scan / abw_twobit_pack (the file goes to the device as it is)
 //   Scaf::Scaf                      -> abw_segment
 //   Scaf_segment::Scaf_segment      -> abw_kmer_features
 //   Scaf::add_mapped_read           -> abw_coverage (one call per SAM file, reads in file order)
@@ -100,33 +101,27 @@ int main(int argc, const char* argv[])
 			return -1;
 		}
 		milestone("abw_ctx_create");
-		// the FASTA text goes to the device as it is: records are indexed there (abw_fasta_scan), the host only reads the names
-		std::string fasta_text;
-		{
-			FILE* fp = fopen(assembly_file.c_str(), "rb");
-			if(!fp)
-				throw std::runtime_error("Failed to open file " + assembly_file);
-			fseek(fp, 0, SEEK_END);
-			const long sz = ftell(fp);
-			rewind(fp);
-			fasta_text.resize((size_t)std::max<long>(sz, 0));
-			if(sz > 0 && fread(&fasta_text[0], 1, (size_t)sz, fp) != (size_t)sz)
-				throw std::runtime_error("Failed to read file " + assembly_file);
-			fclose(fp);
-		}
+		// The assembly goes to the device as it is: FASTA text (records indexed there, abw_fasta_scan) or a UCSC .2bit file (decoded there,
+		// abw_twobit_pack).  The host only reads the names.
+		std::string file_bytes = read_file(assembly_file);
+		const bool twobit = is_twobit(file_bytes);
 		abw_fasta* fa = nullptr;
-		if(abw_fasta_scan(ctx, fasta_text.data(), fasta_text.size(), 0, &fa) != ABW_OK)
+		abw_twobit* tb = nullptr;
+		if(twobit? abw_twobit_scan(ctx, file_bytes.data(), file_bytes.size(), &tb) != ABW_OK : abw_fasta_scan(ctx, file_bytes.data(), file_bytes.size(), 0, &fa) != ABW_OK)
 			throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + assembly_file + ")");
-		const uint64_t nrec = abw_fasta_count(fa);
+		const uint64_t nrec = twobit? abw_twobit_count(tb) : abw_fasta_count(fa);
 		std::vector<uint64_t> id_off(nrec), rec_len(nrec);
 		std::vector<uint32_t> id_len(nrec);
-		ABWH_CHECK(ctx, abw_fasta_get(ctx, fa, id_off.data(), id_len.data(), rec_len.data()));
+		if(twobit)
+			ABWH_CHECK(ctx, abw_twobit_get(ctx, tb, id_off.data(), id_len.data(), rec_len.data()));
+		else
+			ABWH_CHECK(ctx, abw_fasta_get(ctx, fa, id_off.data(), id_len.data(), rec_len.data()));
 		// scaffolds in name order; the first record of a name wins (std::map::insert, abawaca-build.cpp:482-490)
 		std::map<std::string, size_t> by_name;
 		for(size_t i = 0; i < nrec; i++) {
 			if(rec_len[i] == 0)
-				std::cerr << "Warning: sequence " << fasta_text.substr(id_off[i], id_len[i]) << " is empty" << std::endl;      // SeqIORead_fasta.h:99-101
-			by_name.insert(std::make_pair(fasta_text.substr(id_off[i], id_len[i]), i));
+				std::cerr << "Warning: sequence " << file_bytes.substr(id_off[i], id_len[i]) << " is empty" << std::endl;      // SeqIORead_fasta.h:99-101
+			by_name.insert(std::make_pair(file_bytes.substr(id_off[i], id_len[i]), i));
 		}
 		const uint32_t nscaf = (uint32_t)by_name.size();
 		std::vector<std::string> scaf_name;
@@ -138,9 +133,21 @@ int main(int argc, const char* argv[])
 			order.push_back((uint32_t)kv.second);
 		}
 		abw_seqset* ss = nullptr;
-		int rc = abw_fasta_pack(ctx, fa, order.data(), nscaf, &ss);
-		abw_fasta_destroy(fa);
-		std::string().swap(fasta_text);
+		int rc;
+		if(twobit) {
+			void* d_file = nullptr;
+			ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<size_t>(file_bytes.size(), 1), &d_file));
+			ABWH_CHECK(ctx, abw_copy_to_device(ctx, d_file, file_bytes.data(), file_bytes.size()));
+			rc = abw_twobit_pack(ctx, tb, d_file, 0, order.data(), nscaf, &ss);
+			ABWH_CHECK(ctx, abw_ctx_synchronize(ctx));
+			ABWH_CHECK(ctx, abw_device_free(ctx, d_file));
+			abw_twobit_destroy(tb);
+		}
+		else {
+			rc = abw_fasta_pack(ctx, fa, order.data(), nscaf, &ss);
+			abw_fasta_destroy(fa);
+		}
+		std::string().swap(file_bytes);
 		if(rc != ABW_OK) {
 			std::cerr << "Fatal error, attempted to initialize DNAString with illegal string: " << abw_last_error(ctx) << std::endl;
 			return -1;

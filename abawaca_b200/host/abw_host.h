@@ -65,6 +65,55 @@ inline std::vector<FastaRecord> read_fasta(const std::string& path)
 	return out;
 }
 
+inline std::string read_file(const std::string& path)
+{
+	std::string text;
+	FILE* fp = fopen(path.c_str(), "rb");
+	if(!fp)
+		throw std::runtime_error("Failed to open file " + path);
+	fseek(fp, 0, SEEK_END);
+	const long sz = ftell(fp);
+	rewind(fp);
+	text.resize((size_t)(sz > 0? sz : 0));
+	if(sz > 0 && fread(&text[0], 1, (size_t)sz, fp) != (size_t)sz) {
+		fclose(fp);
+		throw std::runtime_error("Failed to read file " + path);
+	}
+	fclose(fp);
+	return text;
+}
+
+// a UCSC .2bit file starts with the signature 0x1A412743 in the byte order of the file
+inline bool is_twobit(const std::string& bytes)
+{
+	if(bytes.size() < 4)
+		return false;
+	const unsigned char* b = (const unsigned char*)bytes.data();
+	return (b[0] == 0x43 && b[1] == 0x27 && b[2] == 0x41 && b[3] == 0x1A) || (b[0] == 0x1A && b[1] == 0x41 && b[2] == 0x27 && b[3] == 0x43);
+}
+
+// the records of a .2bit file as twoBitToFa prints them (abw_twobit_scan / _get / _decode), with an empty description
+inline std::vector<FastaRecord> read_twobit(abw_ctx* ctx, const std::string& path, const std::string& bytes)
+{
+	abw_twobit* t = nullptr;
+	if(abw_twobit_scan(ctx, bytes.data(), bytes.size(), &t) != ABW_OK)
+		throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + path + ")");
+	const uint64_t n = abw_twobit_count(t);
+	std::vector<uint64_t> name_off(n), len(n);
+	std::vector<uint32_t> name_len(n);
+	std::vector<FastaRecord> out(n);
+	int rc = abw_twobit_get(ctx, t, name_off.data(), name_len.data(), len.data());
+	for(uint64_t i = 0; i < n && rc == ABW_OK; i++) {
+		out[i].id = bytes.substr(name_off[i], name_len[i]);
+		out[i].seq.resize(len[i]);
+		rc = abw_twobit_decode(ctx, t, i, bytes.data(), &out[i].seq[0]);
+	}
+	abw_twobit_destroy(t);
+	if(rc != ABW_OK)
+		throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + path + ")");
+	return out;
+}
+
 inline bool directory_exists(const std::string& d)
 {
 	struct stat st;

@@ -44,6 +44,46 @@ def read_fasta(path):
     return names, [b"".join(s) for s in seqs]
 
 
+def _blocks(mask):
+    """(starts, sizes) of the maximal runs of True in a bool array"""
+    d = np.diff(np.concatenate(([0], mask.view(np.int8), [0])))
+    starts = np.flatnonzero(d == 1)
+    return starts.astype(np.uint32), (np.flatnonzero(d == -1) - starts).astype(np.uint32)
+
+
+def write_twobit(path, names, seqs, version=0, big_endian=False):
+    """A UCSC .2bit file of the sequences (bytes), as faToTwoBit writes one: A/C/G/T of either case packed 2 bits per base (T=0 C=1 A=2 G=3, first
+    base in the high bits), every other character an N block (the format cannot carry IUPAC codes), lower-case letters mask blocks.
+    version 1 has 64-bit record offsets; big_endian writes every word byte-swapped."""
+    e = ">" if big_endian else "<"
+    code = np.zeros(256, dtype=np.uint8)
+    is_acgt = np.zeros(256, dtype=bool)
+    for i, c in enumerate(b"TCAG"):
+        code[c] = code[c | 0x20] = i
+        is_acgt[c] = is_acgt[c | 0x20] = True
+    records = []
+    for s in seqs:
+        a = np.frombuffer(s, dtype=np.uint8)
+        ns, nz = _blocks(~is_acgt[a])
+        ms, mz = _blocks((a >= ord("a")) & (a <= ord("z")))
+        c = code[a]
+        c = np.concatenate((c, np.zeros((-c.size) % 4, dtype=np.uint8))).reshape(-1, 4)
+        dna = ((c[:, 0] << 6) | (c[:, 1] << 4) | (c[:, 2] << 2) | c[:, 3]).astype(np.uint8).tobytes()
+        u32 = lambda x: np.asarray(x, dtype=e + "u4").tobytes()       # noqa: E731
+        records.append(u32([a.size, ns.size]) + u32(ns) + u32(nz) + u32([ms.size]) + u32(ms) + u32(mz) + u32([0]) + dna)
+    osz = 8 if version else 4
+    index_size = sum(1 + len(n.encode()) + osz for n in names)
+    off = 16 + index_size
+    with open(path, "wb") as f:
+        f.write(np.asarray([0x1A412743, version, len(names), 0], dtype=e + "u4").tobytes())
+        for n, r in zip(names, records):
+            nb = n.encode()
+            f.write(bytes([len(nb)]) + nb + np.asarray([off], dtype=e + ("u8" if version else "u4")).tobytes())
+            off += len(r)
+        for r in records:
+            f.write(r)
+
+
 def write_lrn(path, rows, sample_names, dp_names=None):
     """abawaca-build.cpp:579-606. rows: [ndps][179 + nsamples] truncated values."""
     ndps, ncols = rows.shape

@@ -127,6 +127,112 @@ def fasta_to_seqset(ctx, text):
         L.abw_fasta_destroy(f)
 
 
+def twobit_to_seqset(ctx, data):
+    """UCSC .2bit file image (bytes) -> (seqset handle, names in scaffold order, lengths), the counterpart of fasta_to_seqset: header and records
+    parsed by abw_twobit_scan, the first record of every name kept, scaffolds in byte-wise name order, the file copied to the device once as it is
+    and decoded there (abw_twobit_pack)."""
+    L = ctx.lib
+    arr = np.frombuffer(data, dtype=np.uint8)
+    t = C.c_void_p()
+    ctx.check(L.abw_twobit_scan(ctx.h, capi._p(arr) if arr.size else None, arr.size, C.byref(t)))
+    d_file = None
+    try:
+        n = int(L.abw_twobit_count(t))
+        name_off = np.zeros(n, dtype=np.uint64)
+        name_len = np.zeros(n, dtype=np.uint32)
+        seq_len = np.zeros(n, dtype=np.uint64)
+        ctx.check(L.abw_twobit_get(ctx.h, t, capi._p(name_off), capi._p(name_len), capi._p(seq_len)))
+        first = {}
+        for i in range(n):
+            first.setdefault(bytes(data[int(name_off[i]):int(name_off[i]) + int(name_len[i])]), i)
+        names = sorted(first)
+        order = np.array([first[k] for k in names], dtype=np.uint32)
+        d_file = ctx.alloc(max(arr.size, 1))
+        if arr.size:
+            ctx.to_device(d_file, arr)
+        ss = C.c_void_p()
+        ctx.check(L.abw_twobit_pack(ctx.h, t, C.c_void_p(d_file), 0, capi._p(order), order.size, C.byref(ss)))
+        ctx.synchronize()
+        return ss, [k.decode() for k in names], seq_len[order]
+    finally:
+        if d_file is not None:
+            ctx.free(d_file)
+        L.abw_twobit_destroy(t)
+
+
+class PackedAssembly:
+    """An assembly in 2 bits per base (abw_2bit_assembly): UCSC-order codes with every scaffold starting at a byte of its own, plus runs of the
+    characters that are not A/C/G/T (capi.BASE_RUN_DTYPE, kind BASE_N for 'N', BASE_OTHER for the rest)."""
+
+    def __init__(self, codes, byte_off, lengths, runs):
+        self.codes, self.byte_off, self.lengths, self.runs = codes, byte_off, lengths, runs
+
+    @property
+    def nscaf(self):
+        return int(self.lengths.size)
+
+    @property
+    def nbytes(self):
+        """what crosses the host link: codes and runs"""
+        return int(self.codes.nbytes + self.runs.nbytes)
+
+
+_UCSC_CODE = np.zeros(256, dtype=np.uint8)           # T=0 C=1 A=2 G=3, either case; 0 for every other byte
+_BASE_CLASS = np.full(256, 2, dtype=np.uint8)          # 0: A/C/G/T (either case), 1: 'N', 2: any other byte (quirk Q2)
+for _i, _c in enumerate(b"TCAG"):
+    _UCSC_CODE[_c] = _UCSC_CODE[_c | 0x20] = _i
+    _BASE_CLASS[_c] = _BASE_CLASS[_c | 0x20] = 0
+_BASE_CLASS[ord("N")] = 1
+
+
+def packed_assembly(seq, offsets) -> PackedAssembly:
+    """ASCII scaffolds (uint8 text, offsets [nscaf+1] delimit them) -> PackedAssembly, lossless with respect to abw_pack_sequences: A/C/G/T of
+    either case become codes, maximal runs of 'N' and of any other character become runs.  Raises ValueError on a lower-case 'n', which the
+    reference throws on (String.cpp:47-49) and which the encoding cannot carry."""
+    seq = np.ascontiguousarray(seq, dtype=np.uint8)
+    offsets = np.ascontiguousarray(offsets, dtype=np.uint64).astype(np.int64)
+    lengths = np.diff(offsets)
+    if (lengths < 0).any():
+        raise ValueError("offsets must be non-decreasing")
+    seq = seq[offsets[0]:offsets[-1]] if offsets.size else seq[:0]
+    offsets = offsets - (offsets[0] if offsets.size else 0)
+    nscaf = lengths.size
+    # every scaffold padded to whole bytes: insert (-len) % 4 zero codes after it
+    pad = (-lengths) % 4
+    codes = np.insert(_UCSC_CODE[seq], np.repeat(offsets[1:], pad), 0) if pad.any() else _UCSC_CODE[seq]
+    q = codes.reshape(-1, 4)
+    packed = (q[:, 0] << 6) | (q[:, 1] << 4) | (q[:, 2] << 2) | q[:, 3]
+    byte_off = np.zeros(nscaf, dtype=np.uint64)
+    if nscaf > 1:
+        byte_off[1:] = np.cumsum((lengths + 3) // 4)[:-1]
+    # runs: maximal stretches of one non-ACGT class inside one scaffold
+    cls = _BASE_CLASS[seq]
+    nz = np.flatnonzero(cls)
+    if nz.size and (seq[nz] == ord("n")).any():
+        raise ValueError("lower-case 'n' in a sequence: the reference throws Illegal_DNAString (String.cpp:47-49)")
+    scaf = np.searchsorted(offsets, nz, side="right") - 1
+    c = cls[nz]
+    new = np.ones(nz.size, dtype=bool)
+    if nz.size > 1:
+        new[1:] = (nz[1:] != nz[:-1] + 1) | (c[1:] != c[:-1]) | (scaf[1:] != scaf[:-1])
+    first = np.flatnonzero(new)
+    runs = np.empty(first.size, dtype=capi.BASE_RUN_DTYPE)
+    runs["scaf"] = scaf[first]
+    runs["start"] = nz[first] - offsets[scaf[first]]
+    runs["len"] = np.diff(np.append(first, nz.size))
+    runs["kind"] = np.where(c[first] == 1, capi.BASE_N, capi.BASE_OTHER)
+    return PackedAssembly(np.ascontiguousarray(packed, dtype=np.uint8), byte_off, lengths.astype(np.uint64), runs)
+
+
+def pack_2bit(ctx, pa: PackedAssembly, d_codes, d_runs, ticket=0):
+    """abw_pack_2bit of a PackedAssembly whose codes and runs are in device memory already (possibly still in flight behind `ticket`)"""
+    desc = capi.TwoBitAssembly(d_codes, pa.codes.nbytes, capi._p(pa.byte_off).value, capi._p(pa.lengths).value, d_runs if pa.runs.size else None,
+                               pa.runs.size, ticket)
+    ss = C.c_void_p()
+    ctx.check(ctx.lib.abw_pack_2bit(ctx.h, C.byref(desc), pa.nscaf, C.byref(ss)))
+    return ss
+
+
 class FeatureBuild:
     """Device-resident result of the feature stage; `rows_host()` fetches the .lrn matrix."""
 
@@ -320,13 +426,19 @@ def sorted_reads(r, nscaf, max_snps=15) -> ReadSample:
 
 def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params=None, kind=capi.FEAT_TRUNC3, skip_A=True,
                    seq_on_device=False, reads_on_device=False, nreads=None, timings=None, overlap_h2d=False, seqset=None, per_sample_calls=False) -> FeatureBuild:
-    """seq: uint8 ASCII (numpy array, or a device pointer int when seq_on_device); offsets: uint64 [nscaf+1];
+    """seq: uint8 ASCII (numpy array, or a device pointer int when seq_on_device), or a PackedAssembly (offsets is then ignored and may be None);
+    offsets: uint64 [nscaf+1];
     reads: per sample a structured array (capi.READ_DTYPE), a ReadSample, or a device pointer of abw_read records (reads_on_device, with nreads).
     All samples go through ONE abw_coverage_batch call (per_sample_calls=True: one abw_coverage call per sample, full records only)."""
     L = ctx.lib
     p = params or capi.default_params()
-    offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-    nscaf = offsets.size - 1
+    packed = isinstance(seq, PackedAssembly)
+    if packed:
+        offsets = None
+        nscaf = seq.nscaf
+    else:
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        nscaf = offsets.size - 1
     t_last = [time.perf_counter()]
 
     def lap(name):
@@ -347,7 +459,21 @@ def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params
     staged = []
     tickets = [0] * len(samples)
     t_seq = 0
-    if not seq_on_device and seqset is None and overlap_h2d:
+    d_2bit = None
+    if packed and seqset is None:
+        # codes and runs behind one ticket: copies of one stream complete in order, so the ticket of the codes covers the runs
+        d_codes = ctx.alloc(max(seq.codes.nbytes, 16))
+        d_runs = ctx.alloc(max(seq.runs.nbytes, 16))
+        staged += [d_codes, d_runs]
+        for a, d in ((seq.runs, d_runs), (seq.codes, d_codes)):
+            if a.size == 0:
+                continue
+            if overlap_h2d:
+                t_seq = ctx.h2d_async(d, a)
+            else:
+                ctx.to_device(d, a)
+        d_2bit = (d_codes, d_runs)
+    elif not seq_on_device and seqset is None and overlap_h2d:
         seq = np.ascontiguousarray(seq, dtype=np.uint8)
         d_seq = ctx.alloc(seq.nbytes + 64)
         staged.append(d_seq)
@@ -375,10 +501,12 @@ def build_features(ctx: capi.Context, seq, offsets, reads, this_sample=0, params
             else:
                 ctx.to_device(d, a)
         dev.append(tuple(ptrs))
-    if t_seq:
+    if t_seq and not packed:
         ctx.wait_h2d(t_seq)
     if seqset is not None:
         pass                                               # packed elsewhere (fasta_to_seqset); offsets only carry the scaffold count
+    elif packed:
+        seqset = pack_2bit(ctx, seq, d_2bit[0], d_2bit[1], t_seq)      # waits for the ticket on the device, not on the host
     elif seq_on_device:
         seqset = C.c_void_p()
         ctx.check(L.abw_pack_sequences(ctx.h, C.c_void_p(seq), 1, capi._p(offsets), nscaf, C.byref(seqset)))

@@ -205,6 +205,53 @@ uint64_t abw_fasta_count(const abw_fasta* f);
 int      abw_fasta_get(abw_ctx* ctx, const abw_fasta* f, uint64_t* h_id_off, uint32_t* h_id_len, uint64_t* h_seq_len);
 int      abw_fasta_pack(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_order, uint32_t nout, abw_seqset** out);
 
+/* ---- assembly in 2 bits per base -> packed assembly on the device ----------------------------------------------------------
+ * The codes are those of a UCSC .2bit file: T=0 C=1 A=2 G=3, four bases per byte, the first base in the HIGH bits of its byte; every scaffold
+ * starts at a byte of its own (at any byte address).  Characters other than A/C/G/T (either case) are described by runs: kind ABW_BASE_N for the
+ * literal 'N', ABW_BASE_OTHER for any other character (quirk Q2: a base for windowing that breaks k-mers); the code under a run is ignored.
+ * abw_pack_2bit builds the abw_seqset abw_pack_sequences makes from the ASCII text the encoding stands for, bit for bit (packed, valid, nmask,
+ * Bio::Ns and the C+G count).  Upper/lower case is not part of the encoding, so a lower-case 'n' cannot be reported here: encoders refuse it.
+ * Checked on the host (ABW_ERR_ARG): h_byte_off[s] + ceil(h_len[s] / 4) <= nbytes and h_len[s] < 2^32.  The runs may still be in flight behind
+ * h2d_ticket, so their contents are dealt with on the device: a run with scaf >= nscaf or start >= the scaffold's length is skipped, a run that
+ * reaches past the scaffold's end is clipped, a position under any N run is N whatever other runs cover it, and a kind other than ABW_BASE_N
+ * counts as ABW_BASE_OTHER.  The call waits for h2d_ticket on the device and returns once its work is enqueued; codes and runs must stay alive
+ * until later work on the context has consumed the result (e.g. until abw_ctx_synchronize). */
+#define ABW_BASE_N     0   /* the literal 'N': nmask bit set, valid bit clear */
+#define ABW_BASE_OTHER 1   /* any other non-ACGT character: valid bit clear */
+typedef struct {
+	uint32_t scaf;        /* 0-based scaffold index */
+	uint32_t start;       /* 0-based first position in the scaffold */
+	uint32_t len;         /* positions */
+	uint32_t kind;        /* ABW_BASE_N or ABW_BASE_OTHER */
+} abw_base_run;
+typedef struct {
+	const uint8_t*      codes;        /* device: 2-bit codes in the UCSC .2bit layout */
+	uint64_t            nbytes;       /* readable bytes at codes */
+	const uint64_t*     h_byte_off;   /* host [nscaf]: byte of codes where scaffold s starts */
+	const uint64_t*     h_len;        /* host [nscaf]: bases of scaffold s, < 2^32 */
+	const abw_base_run* runs;         /* device [nruns], may be NULL when nruns is 0 */
+	uint64_t            nruns;
+	uint64_t            h2d_ticket;   /* 0: none; codes and runs may still be in flight behind it (abw_h2d_async) */
+} abw_2bit_assembly;
+int abw_pack_2bit(abw_ctx* ctx, const abw_2bit_assembly* in, uint32_t nscaf, abw_seqset** out);
+
+/* UCSC .2bit files, the counterpart of abw_fasta_*.  abw_twobit_scan parses header, index and record headers of the file image h_file[nbytes] on the
+ * host: versions 0 (32-bit offsets) and 1 (64-bit offsets), either byte order (the signature 0x1A412743 read byte-swapped marks a big-endian file).
+ * ABW_ERR_ARG for a malformed file: truncated, an offset or block outside the file or the sequence, blocks unsorted or overlapping, an empty name.
+ * abw_twobit_get returns per record, in file order, where its name lies in the file, the name's length and the sequence length.
+ * abw_twobit_decode writes record `record` as twoBitToFa prints its sequence: upper case, lower case under mask blocks, 'N' (or 'n' under a mask
+ * block) under N blocks; h_out has room for the sequence length.
+ * abw_twobit_pack packs the records h_order[0 .. nout) (abawaca-build keeps the first record of every name, in name order) from d_file, the same
+ * file image in device memory (possibly still in flight behind h2d_ticket), through abw_pack_2bit.  ABW_ERR_ILLEGAL_DNA when a selected record has
+ * an N block that overlaps a mask block: that is a lower-case 'n' in its FASTA, which the reference throws on (String.cpp:47-49). */
+typedef struct abw_twobit abw_twobit;
+int      abw_twobit_scan(abw_ctx* ctx, const void* h_file, uint64_t nbytes, abw_twobit** out);
+void     abw_twobit_destroy(abw_twobit* t);
+uint64_t abw_twobit_count(const abw_twobit* t);
+int      abw_twobit_get(abw_ctx* ctx, const abw_twobit* t, uint64_t* h_name_off, uint32_t* h_name_len, uint64_t* h_seq_len);
+int      abw_twobit_decode(abw_ctx* ctx, const abw_twobit* t, uint64_t record, const void* h_file, char* h_out);
+int      abw_twobit_pack(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, const uint32_t* h_order, uint32_t nout, abw_seqset** out);
+
 /* ---- .lrn data lines -> matrix on the device ---------------------------------------------------------------------------------
  * Replaces the datapoint loop of ClusterData::ClusterData (ClusterData.cpp:110-168) for the text after the four header lines: every line that is
  * not empty and does not start with '%' is "<key>\t<v1>\t...\t<vD>"; keys are read with atoi, values with atof (:151,159).  Row r of the
