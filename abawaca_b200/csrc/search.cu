@@ -2959,11 +2959,16 @@ int abw_cluster_scg(abw_ctx* ctx, const abw_search* s, const uint32_t* h_scafs, 
 	for(uint32_t i = 0; i < nscafs; i++)
 		if(h_scafs[i] >= s->S)
 			return abw_fail(ctx, ABW_ERR_ARG, "abw_cluster_scg: scaffold index out of range");
+	// the reference walks a std::set of scaffolds: a scaffold listed twice counts once
+	std::vector<uint32_t> set(h_scafs, h_scafs + nscafs);
+	std::sort(set.begin(), set.end());
+	set.erase(std::unique(set.begin(), set.end()), set.end());
+	nscafs = (uint32_t)set.size();
 	ABW_CUDA(ctx, d_list.alloc(nscafs));
 	ABW_CUDA(ctx, d_st.alloc(1));
 	ABW_CUDA(ctx, d_un.alloc(s->W));
 	if(nscafs)
-		ABW_CUDA(ctx, cudaMemcpyAsync(d_list.p, h_scafs, sizeof(uint32_t) * nscafs, cudaMemcpyHostToDevice, ctx->stream));
+		ABW_CUDA(ctx, cudaMemcpyAsync(d_list.p, set.data(), sizeof(uint32_t) * nscafs, cudaMemcpyHostToDevice, ctx->stream));
 	ABW_CUDA(ctx, cudaMemsetAsync(d_st.p, 0, sizeof(TermStats), ctx->stream));
 	ABW_CUDA(ctx, cudaMemsetAsync(d_un.p, 0, sizeof(uint64_t) * s->W, ctx->stream));
 	if(nscafs)

@@ -659,6 +659,36 @@ def search_features(ctx: capi.Context, fb: "FeatureBuild", length, scgmask, para
     return res, kept[:S.value]
 
 
+def cluster_scg(ctx: capi.Context, scgmask, scaf_lists):
+    """ClusterQuality::scg of every scaffold list in scaf_lists through abw_cluster_scg: [(unique SCG names, average copies per name)].
+    scgmask: uint64 [S][W] SCG masks of the scaffolds.  abw_cluster_scg reads the masks of a search, so every call creates (and destroys) a
+    search of S scaffolds of two equal datapoints each that holds them and is never run: a device sort of 2 S values per call, meant for tests
+    and tools that hold the masks on the host, not for tallies inside a search loop."""
+    L = ctx.lib
+    scgmask = np.ascontiguousarray(scgmask, dtype=np.uint64)
+    if scgmask.ndim == 1:
+        scgmask = scgmask.reshape(-1, 1)
+    S, W = scgmask.shape
+    N = 2 * S
+    T = np.full(S, 2, dtype=np.uint32)
+    values = np.zeros((1, N), dtype=np.float64)
+    length = np.zeros(S, dtype=np.uint64)
+    p = capi.default_params()
+    h = C.c_void_p()
+    ctx.check(L.abw_search_create(ctx.h, capi._p(values), 0, capi.LAYOUT_COLMAJOR, N, N, None, N, 1, None, S, capi._p(T), capi._p(length), capi._p(scgmask), W,
+                                  C.byref(p), capi.SENS_SPEC, C.byref(h)))
+    try:
+        out = []
+        for scafs in scaf_lists:
+            scafs = np.ascontiguousarray(scafs, dtype=np.uint32)
+            u, avg = C.c_uint32(), C.c_double()
+            ctx.check(L.abw_cluster_scg(ctx.h, h, capi._p(scafs), scafs.size, C.byref(u), C.byref(avg)))
+            out.append((u.value, avg.value))
+        return out
+    finally:
+        L.abw_search_destroy(h)
+
+
 def _run_search(ctx, h, N, S, D, p, t0, want_bins, timings, collectives, dim_offset, D_total, scaf_gc, scaf_cvg, buffers, dim_stride=1):
     L = ctx.lib
     t1 = time.perf_counter()

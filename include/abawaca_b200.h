@@ -439,7 +439,9 @@ typedef struct {
 } abw_search_profile;
 int abw_search_get_profile(const abw_search* s, abw_search_profile* out);
 
-/* ClusterQuality::scg (ClusterQuality.cpp:44-48) for an arbitrary scaffold list */
+/* ClusterQuality::scg (ClusterQuality.cpp:44-48) for an arbitrary scaffold list: the number of distinct SCG names on the scaffolds (nunique) and
+ * the average number of copies per distinct name (avg, 0 when there is none).  The list is taken as a set, as the reference's std::set is: a
+ * scaffold listed more than once counts once.  An index >= the number of scaffolds of the search gives ABW_ERR_ARG. */
 int abw_cluster_scg(abw_ctx* ctx, const abw_search* s, const uint32_t* h_scafs, uint32_t nscafs, uint32_t* nunique, double* avg);
 
 #ifdef __cplusplus

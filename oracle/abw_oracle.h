@@ -136,7 +136,7 @@ typedef struct {
 uint32_t abwo_run(const abwo_search_data* d, const abwo_params* p, int strategy, abwo_cluster_rec* recs, uint32_t cap,
                   uint32_t* dp2cluster, uint32_t* scaf2cluster, int nthreads);
 
-/* SCGdb.cpp:6-18,41-55 over a scaffold list */
+/* SCGdb.cpp:6-18,41-55 over a scaffold list; a scaffold listed more than once counts once (the reference walks a std::set) */
 void abwo_cluster_scg(const abwo_search_data* d, const uint32_t* scafs, uint32_t nscafs, uint32_t* nunique, double* avg);
 
 #ifdef __cplusplus

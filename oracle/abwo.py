@@ -177,3 +177,10 @@ class Search:
         s2c = np.zeros(self.S, dtype=np.uint32)
         n = lib().abwo_run(C.byref(self.c), C.byref(p), C.c_int(strategy), recs, C.c_uint32(cap), _ptr(dp2c), _ptr(s2c), C.c_int(nthreads))
         return [recs[i] for i in range(min(n, cap))], dp2c, s2c
+
+    def cluster_scg(self, scafs):
+        """(number of unique SCG names, average copies per unique name) of a scaffold list (abwo_cluster_scg)."""
+        scafs = np.ascontiguousarray(scafs, dtype=np.uint32)
+        u, avg = C.c_uint32(), C.c_double()
+        lib().abwo_cluster_scg(C.byref(self.c), _ptr(scafs), C.c_uint32(scafs.size), C.byref(u), C.byref(avg))
+        return u.value, avg.value

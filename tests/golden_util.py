@@ -143,8 +143,23 @@ def coverage_edge_workload(seed=7, nscaf=160, nsamples=3, depth=40, cover_all_n=
     return seq, offsets, reads
 
 
-def _random_problem(rng, S, D, partial=False, ties=True, scg=True, nclus=3):
-    """Seeded random split-search problem of S scaffolds (T in 2..8 datapoints each, n = T unless partial) in D dimensions around nclus centres."""
+def _pack_names(has):
+    """bool [S][G] (scaffold carries SCG name g) -> uint64 [S][ceil(G/64)] masks, name g in bit g % 64 of word g // 64"""
+    S, G = has.shape
+    W = (G + 63) // 64
+    bits = np.zeros((S, 64 * W), dtype=bool)
+    bits[:, :G] = has
+    return np.packbits(bits, axis=1, bitorder="little").view("<u8").astype(np.uint64).reshape(S, W)
+
+
+def _random_problem(rng, S, D, partial=False, ties=True, scg=True, nclus=3, G=70, carriers=None, contamination=0.0, dense=0, len_hi=400000):
+    """Seeded random split-search problem of S scaffolds (T in 2..8 datapoints each, n = T unless partial) in D dimensions around nclus centres.
+
+    SCG names 0..G-1 (masks of ceil(G/64) words): each name lands, with probability 0.8 per centre, on one scaffold of that centre.
+    carriers: only that many scaffolds (drawn at random) carry names, and each of them carries at least one;
+    contamination: every carrier also carries every name with this probability, whatever its centre;
+    dense: that many carriers carry between 24 and 300 names (at most G) drawn at random.
+    With these three at their defaults the draws are the ones the function always made."""
     T = rng.integers(2, 9, S).astype(np.uint32)
     n = T.copy()
     if partial:
@@ -158,17 +173,31 @@ def _random_problem(rng, S, D, partial=False, ties=True, scg=True, nclus=3):
     if ties:
         vals = np.round(vals, 1)             # heavy ties, negative values and +-0.0
         vals[vals == 0] = np.where(rng.random((vals == 0).sum()) < 0.5, 0.0, -0.0)
-    length = rng.integers(2000, 400000, S).astype(np.uint64)
-    W = 2
+    length = rng.integers(2000, len_hi, S).astype(np.uint64)
+    W = (G + 63) // 64
     mask = np.zeros((S, W), dtype=np.uint64)
     if scg:
-        for g in range(70):
+        is_carrier = np.ones(S, dtype=bool)
+        if carriers is not None:
+            is_carrier[:] = False
+            is_carrier[rng.choice(S, carriers, replace=False)] = True
+        for g in range(G):
             for c in range(nclus):
                 if rng.random() < 0.8:
-                    cand = np.nonzero(grp == c)[0]
+                    cand = np.nonzero((grp == c) & is_carrier)[0]
                     if cand.size:
                         s = cand[rng.integers(0, cand.size)]
                         mask[s, g // 64] |= np.uint64(1) << np.uint64(g % 64)
+        car = np.flatnonzero(is_carrier)
+        extra = np.zeros((car.size, G), dtype=bool)
+        if contamination > 0:
+            extra |= rng.random((car.size, G)) < contamination
+        for i in rng.choice(car.size, dense, replace=False) if dense else ():
+            extra[i, rng.choice(G, int(rng.integers(min(24, G), min(300, G) + 1)), replace=False)] = True
+        if carriers is not None:
+            bare = ~mask[car].any(axis=1) & ~extra.any(axis=1)
+            extra[bare, rng.integers(0, G, int(bare.sum()))] = True
+        mask[car] |= _pack_names(extra)
     return np.ascontiguousarray(vals), dp2scaf, T, length, mask
 
 

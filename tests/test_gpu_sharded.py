@@ -6,7 +6,7 @@ import threading
 import numpy as np
 import pytest
 
-from golden_util import search_problem
+from golden_util import _random_problem, search_problem
 
 pytestmark = pytest.mark.gpu
 
@@ -44,11 +44,20 @@ class ThreadCollectives:
             self.structs.append(type("S", (), {"struct": st})())
 
 
+def _problem(name):
+    """A golden set, or "random_w3": a generated problem whose SCG masks have three words (160 names, contamination across centres, dense scaffolds)."""
+    if name == "random_w3":
+        vals, dp2scaf, T, length, mask = _random_problem(np.random.default_rng(41), 1500, 6, ties=False, nclus=5, G=160, contamination=0.001, dense=6)
+        assert mask.shape[1] == 3 and mask[:, 2].any()
+        return {"values": vals, "dp2scaf": dp2scaf, "T": T, "len": length, "scgmask": mask}
+    return search_problem(name)
+
+
 @pytest.mark.parametrize("name,strategy,world,strided", [("tiny_noisy", 0, 2, False), ("tiny_noisy", 1, 2, False), ("tiny_clean", 0, 3, False),
-                                                         ("tiny_noisy", 0, 3, True), ("tiny_clean", 1, 2, True)])
+                                                         ("tiny_noisy", 0, 3, True), ("tiny_clean", 1, 2, True), ("random_w3", 0, 3, True)])
 def test_sharded_search_equals_single_rank(name, strategy, world, strided):
     from abawaca_b200 import capi, pipeline, distributed
-    prob = search_problem(name)
+    prob = _problem(name)
     vals = prob["values"]
     D = vals.shape[0]
     p = capi.default_params()
@@ -56,6 +65,7 @@ def test_sharded_search_equals_single_rank(name, strategy, world, strided):
     ctx0 = capi.Context(0)
     ref = pipeline.search(ctx0, vals, prob["dp2scaf"], prob["T"], prob["len"], prob["scgmask"], params=p, strategy=strategy)
     ctx0.close()
+    assert len(ref.recs) > 1                            # the search splits: there are child clusters to compare
     ctxs = [capi.Context(0) for _ in range(world)]
     coll = ThreadCollectives(ctxs)
     results, errors = [None] * world, []

@@ -93,3 +93,40 @@ def test_run_ahead_rule_of_the_sharded_search_enqueues_the_same_levels_on_every_
         for last_level in (0, 1, 2, 7, 12, 30):
             counts = {levels_enqueued(last_level, lead, lambda: int(rng.integers(0, 50))) for _ in range(200)}
             assert counts == {last_level + lead}, (lead, last_level, counts)
+
+
+def test_random_problem_defaults_draw_what_they_always_drew():
+    """_random_problem's SCG options (names, carriers, contamination, dense scaffolds) leave the problems of every seed the existing tests use as they
+    were: the same arrays, and the generator left at the same state (digests taken before the options existed)."""
+    import hashlib
+    from golden_util import _random_problem
+
+    def digest(rng, *args, **kw):
+        h = hashlib.sha256()
+        for a in _random_problem(rng, *args, **kw):
+            h.update(np.ascontiguousarray(a).tobytes())
+        h.update(np.int64(rng.integers(0, 2 ** 62)).tobytes())
+        return h.hexdigest()[:16]
+
+    expect = {1: "d2f8f94c78740395", 2: "f83ea99e16e7d2f1", 3: "497d2895c7b93285", 4: "919038c83ef0b061", 5: "c64fa1df96cbde5f", 6: "e018a0caaa61931f",
+              7: "74ea0ebd7b5440fe"}
+    for seed, partial, scg in [(1, False, True), (2, True, True), (3, False, False), (4, True, True), (5, False, True), (6, False, True), (7, True, False)]:
+        rng = np.random.default_rng(seed)                   # test_gpu_parity.py: test_search_matches_oracle_on_random_problems
+        S, D = int(rng.integers(150, 500)), int(rng.integers(3, 12))
+        assert digest(rng, S, D, partial=partial, scg=scg, nclus=int(rng.integers(2, 5))) == expect[seed]
+    rng = np.random.default_rng(11)                         # test_gpu_parity.py: test_small_and_degenerate_searches
+    assert digest(rng, 20, 2) + digest(rng, 300, 3) == "d84b42ec405c059abe5490e3b22594f6"
+    for seed, partial, h in [(21, False, "e0fef066441cbbed"), (22, True, "4945e952166bde9b"), (23, False, "7b97bc26196dd0a7")]:   # test_gpu_lookback_windows.py
+        assert digest(np.random.default_rng(seed), 80000, 3, partial=partial) == h
+    # test_gpu_sort_chunks.py's seeds (there with 30000 scaffolds in 400 dimensions), smaller
+    assert digest(np.random.default_rng(31), 3000, 40, ties=True) == "fe7bc86683dce66f"
+    assert digest(np.random.default_rng(32), 3000, 40, ties=False) == "0740f534a56494d7"
+
+
+def test_oracle_cluster_scg_counts_a_repeated_scaffold_once(oracle):
+    """abwo_cluster_scg takes its scaffold list as a set, like ClusterQuality::scg's std::set: repeats change nothing."""
+    mask = np.array([[0b1011, 0], [0b0001, 1 << 63], [0, 0]], dtype=np.uint64)
+    O = oracle.Search(np.zeros((1, 6)), np.repeat(np.arange(3, dtype=np.uint32), 2), np.full(3, 2, dtype=np.uint32), np.zeros(3, dtype=np.uint64), mask)
+    assert O.cluster_scg([0, 1]) == (4, 5 / 4)
+    assert O.cluster_scg([1, 0, 1, 1, 2, 0]) == (4, 5 / 4)
+    assert O.cluster_scg([]) == (0, 0.0) and O.cluster_scg([2, 2]) == (0, 0.0)
