@@ -11,18 +11,11 @@
 // Data flow: newline positions are counted per 4 KB tile and scanned, which gives every line its index; a second pass writes the line starts;
 // the first byte of a line decides whether it is a record, and a scan over those flags gives the record its slot; one thread then parses one line.
 #include "common.cuh"
+#include "reads.cuh"
 #include <algorithm>
 #include <cstring>
 #include <cstdlib>
 #include <vector>
-
-struct abw_names {
-	uint32_t nscaf = 0, nslots = 0;
-	DevBuf<unsigned long long> slot_hash;     // open addressing, 0 = empty (hashes are forced non-zero)
-	DevBuf<uint32_t> slot_index;
-	DevBuf<char> blob;                        // concatenated names
-	DevBuf<uint64_t> off;                     // [nscaf+1]
-};
 
 struct abw_fasta {
 	uint64_t nbytes = 0, nlines = 0, nrec = 0;
@@ -38,16 +31,6 @@ namespace {
 constexpr int LN_THREADS = 256;
 constexpr int LN_BYTES_PER_THREAD = 16;
 constexpr int LN_TILE = LN_THREADS * LN_BYTES_PER_THREAD;      // 4 KB of text per block
-
-__host__ __device__ __forceinline__ unsigned long long fnv1a(const char* s, uint64_t n)
-{
-	unsigned long long h = 1469598103934665603ull;
-	for(uint64_t i = 0; i < n; i++) {
-		h ^= (unsigned char)s[i];
-		h *= 1099511628211ull;
-	}
-	return h? h : 1ull;
-}
 
 __global__ void __launch_bounds__(LN_THREADS) k_sam_count_newlines(const char* __restrict__ text, uint64_t nbytes, uint32_t* __restrict__ tile_counts)
 {
@@ -174,28 +157,8 @@ __global__ void __launch_bounds__(128) k_sam_parse(const char* __restrict__ text
 			const char* fe = q;
 			if(field == 1)
 				flag = (uint32_t)dev_atoi(fs, fe);
-			else if(field == 2) {
-				const uint64_t n = (uint64_t)(fe - fs);
-				const unsigned long long h = fnv1a(fs, n);
-				uint32_t s = (uint32_t)(h & (nslots - 1));
-				for(uint32_t probe = 0; probe < nslots; probe++) {
-					const unsigned long long sh = slot_hash[s];
-					if(sh == 0)
-						break;
-					if(sh == h) {
-						const uint32_t idx = slot_index[s];
-						const uint64_t a = name_off[idx], b = name_off[idx + 1];
-						bool same = (b - a) == n;
-						for(uint64_t i = 0; same && i < n; i++)
-							same = name_blob[a + i] == fs[i];
-						if(same) {
-							scaf = idx;
-							break;
-						}
-					}
-					s = (s + 1) & (nslots - 1);
-				}
-			}
+			else if(field == 2)
+				scaf = abw_name_probe(fs, (uint64_t)(fe - fs), slot_hash, slot_index, nslots, name_blob, name_off);
 			else if(field == 3)
 				pos0 = (uint32_t)(dev_atoi(fs, fe) - 1);    // stored 0-based, ReadMapping.cpp:41
 			else if(field == 5) {
@@ -217,32 +180,8 @@ __global__ void __launch_bounds__(128) k_sam_parse(const char* __restrict__ text
 						const char* me = m;
 						while(me < fe && *me != ' ')
 							me++;
-						// MD:Z:[0-9]+(([A-Z]|\^[^0-9]+)[0-9]+)*  as determine_snps walks it (:94-125)
-						while(m < me && *m >= '0' && *m <= '9')
-							m++;
-						while(m < me) {
-							if(*m == '^') {
-								m++;
-								while(m < me && !(*m >= '0' && *m <= '9')) {
-									nsnps++;
-									m++;
-								}
-							}
-							else if(*m >= 'A' && *m <= 'Z') {
-								nsnps++;
-								m++;
-							}
-							else {
-								bad |= SAM_ERR_MDZ;
-								break;
-							}
-							if(m >= me || !(*m >= '0' && *m <= '9')) {
-								bad |= SAM_ERR_MDZ;
-								break;
-							}
-							while(m < me && *m >= '0' && *m <= '9')
-								m++;
-						}
+						if(!abw_md_snps(m, me, &nsnps))
+							bad |= SAM_ERR_MDZ;
 						break;
 					}
 				}
@@ -526,7 +465,7 @@ int abw_names_create(abw_ctx* ctx, const char* names_blob, const uint64_t* h_nam
 		for(uint32_t i = 0; i < nscaf; i++) {
 			if(h_name_off[i + 1] < h_name_off[i])
 				return abw_fail(ctx, ABW_ERR_ARG, "abw_names_create: offsets must be non-decreasing");
-			const unsigned long long h = fnv1a(names_blob + h_name_off[i], h_name_off[i + 1] - h_name_off[i]);
+			const unsigned long long h = abw_fnv1a(names_blob + h_name_off[i], h_name_off[i + 1] - h_name_off[i]);
 			uint32_t s = (uint32_t)(h & (nslots - 1));
 			while(sh[s] != 0)
 				s = (s + 1) & (nslots - 1);

@@ -5,7 +5,8 @@
 //   Scaf::Scaf                      -> abw_segment
 //   Scaf_segment::Scaf_segment      -> abw_kmer_features
 //   Scaf::add_mapped_read           -> abw_coverage (one call per SAM file, reads in file order)
-//   SAMReader / ReadMapping(line)   -> abw_parse_sam (SAM text goes to the device in 64 MB chunks cut at line boundaries)
+//   SAMReader / ReadMapping(line)   -> abw_parse_sam (SAM text goes to the device in 64 MB chunks cut at line boundaries), or for a BAM file
+//                                      abw_bam_feed / abw_bam_finish (the file goes to the device in 64 MB reads, inflated and parsed there)
 //   the "%.3lf" rows of abawaca.lrn   -> abw_format_lrn (text made on the device in 64 MB pieces, written with fwrite)
 // The other text writers stay on the host.  Not ported (out of the hot path, SURVEY.md section 2):
 // paired-end link counting (abawaca.links is written empty: `abawaca` only checks that it exists) and the calls to
@@ -15,6 +16,7 @@
 #include <chrono>
 #include <ctime>
 #include <iostream>
+#include <memory>
 
 using namespace abwh;
 
@@ -196,6 +198,31 @@ int main(int argc, const char* argv[])
 			FILE* fp = fopen(sam_files[j].c_str(), "rb");
 			if(!fp)
 				throw std::runtime_error("Failed to open SAM file " + sam_files[j]);
+			if(is_bgzf(fp)) {
+				// BAM: the file in 64 MB reads; blocks, header and records may be cut anywhere, the reader carries what is unfinished
+				std::unique_ptr<FILE, int (*)(FILE*)> file(fp, fclose);
+				abw_bam* bam_raw = nullptr;
+				ABWH_CHECK(ctx, abw_bam_create(ctx, names, &bam_raw));
+				std::unique_ptr<abw_bam, void (*)(abw_bam*)> bam(bam_raw, abw_bam_destroy);
+				size_t n;
+				while((n = fread(buf.data(), 1, CHUNK, fp)) > 0)
+					if(abw_bam_feed(ctx, bam.get(), buf.data(), n) != ABW_OK)
+						throw std::runtime_error(std::string("abw_bam_feed failed on ") + sam_files[j] + ": " + abw_last_error(ctx));
+				file.reset();
+				const abw_read* d_reads = nullptr;
+				uint64_t nreads = 0;
+				if(abw_bam_finish(ctx, bam.get(), &d_reads, &nreads) != ABW_OK)
+					throw std::runtime_error(std::string("abw_bam_finish failed on ") + sam_files[j] + ": " + abw_last_error(ctx));
+				ABWH_CHECK(ctx, abw_coverage(ctx, sg, d_reads, nreads, 1, max_snps, ABW_FEAT_TRUNC3, d_rows, ld, (uint32_t)(179 + j), is_this_sample? d_nbps : nullptr));
+				ABWH_CHECK(ctx, abw_ctx_synchronize(ctx));      // the records are the reader's: coverage has read them before it goes
+				bam.reset();
+				milestone("BAM " + std::to_string(j));
+				if(is_this_sample) {
+					FILE* fl = fopen(links_file.c_str(), "w");
+					if(fl) fclose(fl);
+				}
+				continue;
+			}
 			// a record line has at least 11 fields, i.e. at least 10 tabs and a newline: the file size bounds the number of records
 			fseek(fp, 0, SEEK_END);
 			const uint64_t nlines = (uint64_t)ftell(fp) / 11 + 2;

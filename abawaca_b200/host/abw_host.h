@@ -114,6 +114,15 @@ inline std::vector<FastaRecord> read_twobit(abw_ctx* ctx, const std::string& pat
 	return out;
 }
 
+// a BAM file starts with a BGZF block header (gzip magic 1f 8b); no SAM file starts with byte 0x1F.  Leaves the file at its start.
+inline bool is_bgzf(FILE* fp)
+{
+	unsigned char b[2] = {0, 0};
+	const size_t n = fread(b, 1, 2, fp);
+	rewind(fp);
+	return n == 2 && b[0] == 0x1F && b[1] == 0x8B;
+}
+
 inline bool directory_exists(const std::string& d)
 {
 	struct stat st;

@@ -55,6 +55,41 @@ class SamParser:
             self.h = None
 
 
+class BamReader:
+    """BAM file -> abw_read records on the device (abw_bam_*), the counterpart of SamParser.  feed() takes the file's bytes in pieces split
+    anywhere; finish() returns (device pointer, number of records) of the array the reader owns until close()."""
+
+    def __init__(self, ctx, names):
+        self.ctx = ctx
+        self.names = SamParser(ctx, names)
+        h = C.c_void_p()
+        ctx.check(ctx.lib.abw_bam_create(ctx.h, self.names.h, C.byref(h)))
+        self.h = h
+
+    def feed(self, data):
+        arr = np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else np.ascontiguousarray(data, dtype=np.uint8)
+        self.ctx.check(self.ctx.lib.abw_bam_feed(self.ctx.h, self.h, capi._p(arr) if arr.size else None, arr.size))
+
+    def finish(self):
+        d, n = C.c_void_p(), C.c_uint64()
+        self.ctx.check(self.ctx.lib.abw_bam_finish(self.ctx.h, self.h, C.byref(d), C.byref(n)))
+        return d.value, int(n.value)
+
+    def to_host(self):
+        """finish() and fetch the records"""
+        d, n = self.finish()
+        out = np.zeros(n, dtype=capi.READ_DTYPE)
+        if n:
+            self.ctx.to_host(out, d)
+        return out
+
+    def close(self):
+        if self.h:
+            self.ctx.lib.abw_bam_destroy(self.h)
+            self.h = None
+        self.names.close()
+
+
 def parse_lrn_rows(ctx, text, D):
     """data lines of a .lrn file (bytes, after the four header lines) -> (keys uint64 [n], device pointer of the row-major [n][D] matrix, n).
     The caller frees the matrix with ctx.free()."""

@@ -17,6 +17,9 @@ from __future__ import annotations
 
 import dataclasses
 import os
+import struct
+import zlib
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
@@ -228,3 +231,204 @@ def write_reference_inputs(mg: Metagenome, directory: str):
         for s in mg.scg_names:
             f.write(s + "\n")
     return dict(fasta=fa, sams=sams, gene2scg=g2s, scg_list=lst)
+
+
+# ---- BAM ------------------------------------------------------------------------------------------------------------------------
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+_BAM_FIXED = np.dtype([("block_size", "<i4"), ("refID", "<i4"), ("pos", "<i4"), ("l_read_name", "u1"), ("mapq", "u1"), ("bin", "<u2"),
+                       ("n_cigar_op", "<u2"), ("flag", "<u2"), ("l_seq", "<i4"), ("next_refID", "<i4"), ("next_pos", "<i4"), ("tlen", "<i4")])
+_NT16 = np.full(256, 15, dtype=np.uint8)
+for _i, _c in enumerate("=ACMGRSVTWYHKDBN"):
+    _NT16[ord(_c)] = _i
+    _NT16[ord(_c.lower())] = _i
+
+
+def bam_header(names, lengths, text="@HD\tVN:1.6\tSO:unsorted\n") -> bytes:
+    """magic, SAM header text and the reference list"""
+    out = [b"BAM\1", struct.pack("<i", len(text)), text.encode(), struct.pack("<i", len(names))]
+    for n, ln in zip(names, lengths):
+        b = n.encode() + b"\0"
+        out += [struct.pack("<i", len(b)), b, struct.pack("<i", int(ln))]
+    return b"".join(out)
+
+
+def bam_record(refID, pos, name, flag, cigar=(), seq="", qual=None, aux=b"", mapq=42, next_refID=-1, next_pos=-1, tlen=0) -> bytes:
+    """one BAM record; cigar: (op code, length) pairs, seq: the bases as text, aux: the encoded aux fields"""
+    nb = name.encode() + b"\0"
+    codes = _NT16[np.frombuffer(seq.encode(), dtype=np.uint8)] if seq else np.zeros(0, dtype=np.uint8)
+    if codes.size % 2:
+        codes = np.append(codes, 0)
+    packed = ((codes[0::2] << 4) | codes[1::2]).astype(np.uint8).tobytes()
+    q = bytes([0xFF] * len(seq)) if qual is None else bytes(qual)
+    body = struct.pack("<iiBBHHHiiii", refID, pos, len(nb), mapq, 4680, len(cigar), flag, len(seq), next_refID, next_pos, tlen) + nb + \
+        b"".join(struct.pack("<I", (ln << 4) | op) for op, ln in cigar) + packed + q + aux
+    return struct.pack("<i", len(body)) + body
+
+
+def _md_text(ln, nsnps):
+    if nsnps == 0:
+        return f"{ln}"
+    return "0" + "".join("C0" for _ in range(nsnps - 1)) + f"C{ln - nsnps}"    # as write_reference_inputs writes it
+
+
+def sample_bam_records(mg: Metagenome, j, seed=0, chunk=1 << 17):
+    """The records of sample j as BAM, in chunks: (uint8 array of whole records, record sizes).  The fields are those of the SAM lines
+    write_reference_inputs writes (FLAG, RNAME, POS, CIGAR {len}M, the MD:Z field, no fields for unmapped reads), with the scaffold's bases as
+    SEQ and random qualities; the read names are zero-padded."""
+    rec = mg.reads[j]
+    rng = np.random.default_rng([seed, 5813, j])
+    nscaf = mg.nscaf
+    slen = np.diff(mg.offsets.astype(np.int64))
+    for c0 in range(0, rec.size, chunk):
+        r = rec[c0:c0 + chunk]
+        n = r.size
+        flag = (r["flag_nsnps"] & 0xFFFF).astype(np.uint32)
+        nsnps = (r["flag_nsnps"] >> 16).astype(np.uint32)
+        ln = r["len"].astype(np.int64)
+        unm = (flag & 4) != 0
+        keys = np.stack([unm.astype(np.int64), nsnps.astype(np.int64), ln], axis=1)
+        groups, inv = np.unique(keys, axis=0, return_inverse=True)
+        inv = inv.reshape(-1)
+        names_w = 9
+        prefix = f"r{j}_".encode()
+        lrn = len(prefix) + names_w + 3
+        size = np.zeros(n, dtype=np.int64)
+        parts = []
+        for g, (u, ns, L) in enumerate(groups.tolist()):
+            sel = np.flatnonzero(inv == g)
+            aux = b"" if u else b"MDZ" + _md_text(L, ns).encode() + b"\0"
+            ncig = 0 if u else 1
+            reclen = 36 + lrn + 4 * ncig + (L + 1) // 2 + L + len(aux)
+            size[sel] = reclen
+            parts.append((sel, reclen, u, L, aux, ncig))
+        off = np.zeros(n + 1, dtype=np.int64)
+        off[1:] = np.cumsum(size)
+        buf = np.zeros(int(off[-1]), dtype=np.uint8)
+        for sel, reclen, u, L, aux, ncig in parts:
+            k = sel.size
+            rows = np.zeros((k, reclen), dtype=np.uint8)
+            fx = np.zeros(k, dtype=_BAM_FIXED)
+            fx["block_size"] = reclen - 4
+            fx["refID"] = -1 if u else r["scaf"][sel].astype(np.int64)
+            fx["pos"] = -1 if u else r["pos0"][sel].astype(np.int64)
+            fx["l_read_name"] = lrn
+            fx["mapq"] = 42
+            fx["bin"] = 4680
+            fx["n_cigar_op"] = ncig
+            fx["flag"] = flag[sel]
+            fx["l_seq"] = L
+            fx["next_refID"] = -1
+            fx["next_pos"] = -1
+            rows[:, :36] = fx.view(np.uint8).reshape(k, 36)
+            o = 36
+            rows[:, o:o + len(prefix)] = np.frombuffer(prefix, dtype=np.uint8)
+            num = (c0 + sel).astype(np.int64)
+            for d in range(names_w):
+                rows[:, o + len(prefix) + names_w - 1 - d] = 48 + (num // 10 ** d) % 10
+            rows[:, o + len(prefix) + names_w:o + lrn] = np.frombuffer(b"/1\0", dtype=np.uint8)
+            o += lrn
+            if ncig:
+                rows[:, o:o + 4] = np.frombuffer(struct.pack("<I", L << 4), dtype=np.uint8)
+                o += 4
+            sc = np.minimum(r["scaf"][sel].astype(np.int64), nscaf - 1)
+            p = np.minimum(r["pos0"][sel].astype(np.int64)[:, None] + np.arange(L), slen[sc][:, None] - 1)
+            codes = _NT16[mg.seq[mg.offsets[sc].astype(np.int64)[:, None] + np.maximum(p, 0)]]
+            if L % 2:
+                codes = np.concatenate([codes, np.zeros((k, 1), dtype=np.uint8)], axis=1)
+            rows[:, o:o + (L + 1) // 2] = (codes[:, 0::2] << 4) | codes[:, 1::2]
+            o += (L + 1) // 2
+            rows[:, o:o + L] = rng.integers(0, 41, (k, L), dtype=np.uint8)
+            o += L
+            rows[:, o:] = np.frombuffer(aux, dtype=np.uint8)
+            buf[(off[sel][:, None] + np.arange(reclen)).reshape(-1)] = rows.reshape(-1)
+        yield buf, size
+
+
+def _bgzf_block(payload, level, strategy) -> bytes:
+    c = zlib.compressobj(level, zlib.DEFLATED, -15, 9, strategy)
+    cdata = c.compress(payload) + c.flush()
+    return struct.pack("<BBBBIBBHBBHH", 31, 139, 8, 4, 0, 0, 255, 6, ord("B"), ord("C"), 2, len(cdata) + 25) + cdata + \
+        struct.pack("<II", zlib.crc32(payload), len(payload))
+
+
+class BgzfWriter:
+    """BGZF blocks of a byte stream.  aligned=True cuts as htslib does: a block holds at most 0xff00 bytes and a new block starts before a record
+    that would not fit (records longer than that are split); aligned=False cuts wherever the running byte count says, into pieces of `cut` bytes or,
+    without it, of random sizes in 1 .. 0xff00 (records and the header then cross blocks, as htsjdk writes them)."""
+
+    def __init__(self, f, aligned=True, level=6, strategy=zlib.Z_DEFAULT_STRATEGY, cut=None, seed=0, threads=8):
+        self.f, self.aligned, self.level, self.strategy, self.cut = f, aligned, level, strategy, cut
+        self.rng = np.random.default_rng([seed, 4099])
+        self.pool = ThreadPoolExecutor(threads)
+        self.pend = b""
+        self.k = self._piece()
+
+    def _emit(self, payloads):
+        for blk in self.pool.map(lambda p: _bgzf_block(p, self.level, self.strategy), payloads):
+            self.f.write(blk)
+
+    def _piece(self):
+        return self.cut if self.cut else int(self.rng.integers(1, 0xff00 + 1))
+
+    def write(self, data, sizes=None):
+        """data: bytes or uint8 array; sizes: the record sizes it consists of (aligned mode), None for one unit (e.g. the header)"""
+        data = bytes(data) if not isinstance(data, bytes) else data
+        if not self.aligned:
+            buf = self.pend + data
+            pieces, o = [], 0
+            while o + self.k <= len(buf):
+                pieces.append(buf[o:o + self.k])
+                o += self.k
+                self.k = self._piece()
+            self.pend = buf[o:]
+            self._emit(pieces)
+            return
+        ends = np.cumsum(np.asarray([len(data)] if sizes is None else sizes, dtype=np.int64))
+        starts = ends - np.asarray([len(data)] if sizes is None else sizes, dtype=np.int64)
+        pieces, cur, i = [], self.pend, 0
+        while i < ends.size:
+            room = 0xff00 - len(cur)
+            # records i .. j-1 fit into the open block
+            j = int(np.searchsorted(ends, starts[i] + room, side="right"))
+            if j > i:
+                cur += data[starts[i]:ends[j - 1]]
+                i = j
+                continue
+            if cur:
+                pieces.append(cur)
+                cur = b""
+                continue
+            rec = data[starts[i]:ends[i]]                      # longer than a block: split
+            for o in range(0, len(rec), 0xff00):
+                pieces.append(rec[o:o + 0xff00])
+            cur = pieces.pop()
+            i += 1
+        self.pend = cur
+        self._emit(pieces)
+
+    def flush(self):
+        """end the open block (htslib flushes after the header)"""
+        if self.aligned and self.pend:
+            self._emit([self.pend])
+            self.pend = b""
+
+    def close(self, eof=True):
+        if self.pend:
+            rest = self.pend
+            self.pend = b""
+            self._emit([rest[o:o + 0xff00] for o in range(0, len(rest), 0xff00)])
+        if eof:
+            self.f.write(BGZF_EOF)
+        self.pool.shutdown()
+
+
+def write_bam(path, mg: Metagenome, j, aligned=True, level=6, strategy=zlib.Z_DEFAULT_STRATEGY, cut=None, seed=0, threads=8):
+    """Sample j as a BAM file (the reads of write_reference_inputs' SAM file), in htslib's block layout or cut at arbitrary sizes."""
+    with open(path, "wb") as f:
+        w = BgzfWriter(f, aligned=aligned, level=level, strategy=strategy, cut=cut, seed=seed, threads=threads)
+        w.write(bam_header(mg.names, np.diff(mg.offsets.astype(np.int64))))
+        w.flush()
+        for buf, size in sample_bam_records(mg, j, seed=seed):
+            w.write(buf, size)
+        w.close()
+    return path

@@ -189,6 +189,26 @@ void abw_names_destroy(abw_names* n);
  * lower-case 'n' in SEQ (ABW_ERR_ILLEGAL_DNA), fewer than 11 fields or a malformed MD:Z description (ABW_ERR_ARG). */
 int abw_parse_sam(abw_ctx* ctx, const abw_names* names, const char* text, uint64_t nbytes, int text_on_device, abw_read* d_reads, uint64_t cap, uint64_t* nreads);
 
+/* ---- BAM files -> read records on the device: the counterpart of abw_parse_sam --------------------------------------------------
+ * abw_bam_feed takes the next bytes of a BAM file (host memory) split anywhere: inside a BGZF block header, a block, the BAM header or a record.
+ * The BGZF blocks are inflated and their CRC-32 checked on the device, in batches of at most 64 MB of decoded bytes whatever the compression
+ * ratio; record boundaries are found on the device, so records may cross blocks (htsjdk/Picard files) or not (htslib).  The reader carries at
+ * most one compressed block and the decoded bytes after the last complete record into the next feed.  abw_bam_finish hands out all records of the
+ * file in file order as one device array owned by the reader (valid until abw_bam_destroy), ready for abw_coverage(..., reads_on_device = 1, ...)
+ * or an abw_sample of format ABW_READS_FULL; ABW_ERR_ARG if the stream ended inside a block, the header or a record.
+ * Record i is what abw_parse_sam makes of the line `samtools view` prints for it: FLAG; scaf = the index in `names` of the header's reference
+ * name (refID -1: of the name "*"); pos0 = (uint32_t)pos (-1 gives 0xFFFFFFFF); len = l_seq, or 1 when l_seq is 0 (SEQ printed as "*"); the SNP
+ * count of the first aux field whose printed text holds "MD:Z:" (a Z field tagged MD or a Z value containing it; description up to the first
+ * space), plus the CIGAR's I operations (the CG:B:I tag's under htslib's long-CIGAR convention), capped at 0xFFFF; zero without such a field.
+ * Malformed input gives ABW_ERR_ARG (and the reader refuses further calls): a block header that is not the 18-byte BGZF header, ISIZE > 65536,
+ * any DEFLATE error zlib's inflate reports, output short of or past ISIZE, a CRC-32 mismatch, a bad magic or header length, a record whose
+ * block_size disagrees with its fixed fields or whose aux fields do not end at its end, a malformed MD description (abw_parse_sam's message). */
+typedef struct abw_bam abw_bam;
+int  abw_bam_create(abw_ctx* ctx, const abw_names* names, abw_bam** out);
+int  abw_bam_feed(abw_ctx* ctx, abw_bam* b, const void* h_data, uint64_t nbytes);
+int  abw_bam_finish(abw_ctx* ctx, abw_bam* b, const abw_read** d_reads, uint64_t* nreads);
+void abw_bam_destroy(abw_bam* b);
+
 /* ---- FASTA text -> packed assembly on the device -----------------------------------------------------------------------
  * Replaces SeqIORead_fasta<DNASequence>::next_seq (SeqIORead_fasta.h:51-103, with SeqIORead::getline(true), SeqIORead.h:85-121) for a whole
  * file: lines are trimmed of white space on both ends, blank lines skipped, a line starting with '>' opens a record whose id is the text up
