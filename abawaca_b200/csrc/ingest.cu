@@ -1,15 +1,18 @@
-// SAM text -> read records on the device (SURVEY.md section 8f, row 1: host text parsing is > 80 % of abawaca-build).
+// Text parsers on the device (SURVEY.md section 8f: host text parsing is > 80 % of abawaca-build):
+//   SAM    (abw_parse_sam)    -> the abw_read record stream abw_coverage consumes, in file order
+//   FASTA  (abw_fasta_scan)   -> records with their ids and trimmed sequence lines, packed by abw_fasta_pack
+//   .lrn   (abw_parse_lrn)    -> keys and a row-major matrix of doubles
 //
-// Replaces, for one chunk of SAM text,
+// The three share one line index (line_index): newline positions are counted per 4 KB tile and scanned, which gives every line its index, and a
+// second pass writes the line starts.  SAM and .lrn also share one line selection (select_lines): the last byte and the first byte of a line decide
+// whether it is a record, and a scan over those flags gives the record its slot.  One thread then parses one line.
+//
+// For SAM this replaces, for one chunk of text,
 //   SAMReader::next_mapping            ReadMappingReader.cpp:80-116  (lines; '@' header lines and empty lines are skipped)
 //   ReadMapping::ReadMapping(line)     ReadMapping.cpp:23-72         (tab-separated fields: FLAG, RNAME, POS-1, CIGAR, SEQ, the field holding "MD:Z:")
 //   ReadMapping::determine_snps        ReadMapping.cpp:78-185        (only num_snps() reaches the hot path: one per mismatch letter of MD:Z, one per
 //                                                                     deleted reference base after '^', one per insertion operation of the CIGAR string)
 //   scafs.find(ref_name)               abawaca-build.cpp:549         (reference name -> scaffold index; unknown names give index 0xFFFFFFFF)
-// The output is the abw_read record stream abw_coverage consumes, in file order.
-//
-// Data flow: newline positions are counted per 4 KB tile and scanned, which gives every line its index; a second pass writes the line starts;
-// the first byte of a line decides whether it is a record, and a scan over those flags gives the record its slot; one thread then parses one line.
 #include "common.cuh"
 #include "reads.cuh"
 #include <algorithm>
@@ -17,22 +20,13 @@
 #include <cstdlib>
 #include <vector>
 
-struct abw_fasta {
-	uint64_t nbytes = 0, nlines = 0, nrec = 0;
-	DevBuf<char> text;                        // the text, when it was given on the host
-	const char* d_text = nullptr;
-	DevBuf<uint64_t> line_a, hdr_before, chars_before, rec_id_off, rec_chars0;
-	DevBuf<uint32_t> line_len, rec_id_len;
-	std::vector<uint64_t> h_seq_len;
-};
-
 namespace {
 
 constexpr int LN_THREADS = 256;
 constexpr int LN_BYTES_PER_THREAD = 16;
 constexpr int LN_TILE = LN_THREADS * LN_BYTES_PER_THREAD;      // 4 KB of text per block
 
-__global__ void __launch_bounds__(LN_THREADS) k_sam_count_newlines(const char* __restrict__ text, uint64_t nbytes, uint32_t* __restrict__ tile_counts)
+__global__ void __launch_bounds__(LN_THREADS) k_line_count(const char* __restrict__ text, uint64_t nbytes, uint32_t* __restrict__ tile_counts)
 {
 	__shared__ uint32_t sm[LN_THREADS / 32];
 	const uint64_t i0 = (uint64_t)blockIdx.x * LN_TILE + (uint64_t)threadIdx.x * LN_BYTES_PER_THREAD;
@@ -60,7 +54,7 @@ __global__ void __launch_bounds__(LN_THREADS) k_sam_count_newlines(const char* _
 }
 
 // line l (l >= 1) starts after the l-th newline; line 0 starts at 0.  A final newline opens an empty last line, which is not a record.
-__global__ void __launch_bounds__(LN_THREADS) k_sam_line_starts(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ tile_offs, uint64_t* __restrict__ line_start)
+__global__ void __launch_bounds__(LN_THREADS) k_line_starts(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ tile_offs, uint64_t* __restrict__ line_start)
 {
 	__shared__ uint32_t sm[LN_THREADS / 32];
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -94,22 +88,81 @@ __global__ void __launch_bounds__(LN_THREADS) k_sam_line_starts(const char* __re
 	}
 }
 
-// 1 for a line that becomes a record: not empty after chomp (ReadMappingReader.cpp:113) and not a header line (:108)
-__global__ void k_sam_is_record(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines, uint32_t* __restrict__ is_record)
+// The line index of a text on the device: line l is [start[l], start[l + 1] - 1), the last line ends at nbytes.
+struct LineIndex {
+	DevBuf<char> staged;                      // the text, when it was given on the host
+	const char* text = nullptr;
+	uint64_t nbytes = 0, nlines = 0;
+	DevBuf<uint64_t> start;
+};
+
+// Stages host text (text_on_device == 0) and indexes its lines, with one wait on the context stream for the number of newlines.  nbytes > 0.
+int line_index(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_device, LineIndex* li)
+{
+	li->nbytes = nbytes;
+	li->text = text;
+	if(!text_on_device) {
+		ABW_CUDA(ctx, li->staged.alloc(nbytes + 16));
+		ABW_CUDA(ctx, cudaMemcpyAsync(li->staged.p, text, nbytes, cudaMemcpyHostToDevice, ctx->stream));
+		li->text = li->staged.p;
+	}
+	const unsigned int ntiles = abw_div_up(nbytes, LN_TILE);
+	DevBuf<uint32_t> tile_counts;
+	DevBuf<uint64_t> tile_offs, total;
+	ABW_CUDA(ctx, tile_counts.alloc(ntiles));
+	ABW_CUDA(ctx, tile_offs.alloc(ntiles));
+	ABW_CUDA(ctx, total.alloc(1));
+	ABW_LAUNCH(ctx, k_line_count, ntiles, LN_THREADS, 0, li->text, nbytes, tile_counts.p);
+	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, tile_counts.p, tile_offs.p, ntiles, total.p));
+	uint64_t nnl = 0;
+	ABW_CUDA(ctx, abw_fetch(ctx, &nnl, total.p, sizeof(uint64_t)));
+	ABW_CUDA(ctx, abw_sync(ctx));
+	li->nlines = nnl + 1;
+	ABW_CUDA(ctx, li->start.alloc(li->nlines));
+	ABW_LAUNCH(ctx, k_line_starts, ntiles, LN_THREADS, 0, li->text, nbytes, tile_offs.p, li->start.p);
+	return ABW_OK;
+}
+
+// [a, b) of line l, without its newline
+struct LineExtent { uint64_t a, b; };
+__device__ __forceinline__ LineExtent line_extent(const uint64_t* __restrict__ line_start, uint64_t nlines, uint64_t nbytes, uint64_t l)
+{
+	return {line_start[l], (l + 1 < nlines)? line_start[l + 1] - 1 : nbytes};
+}
+
+__device__ __forceinline__ bool dev_isspace(char c) { return c == ' ' || (c >= '\t' && c <= '\r'); }
+
+// 1 for a line that is not empty after trimming its end and does not start with `skip`.  The end is trimmed of all white space (trim_space) or
+// only of '\r' and '\n':
+//   SAM   ('@', false): chomp (ReadMappingReader.cpp:113) and header lines (:108).  fgets-based reading stops a line at '\n'; a line that is just
+//         "\n" or "\r\n" has next_line[0] == '\n' (not 0 and not '@'), so the reference would try to parse it and fail on fs[1]; real SAM files
+//         have no such lines and abawaca_b200's host parser skips them, as does this one.  A line of blanks is a record (and too short).
+//   .lrn  ('%', true): empty and comment lines (ClusterData.cpp:110-168); a line of blanks is empty.
+__global__ void k_line_select(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines, char skip, bool trim_space,
+                              uint32_t* __restrict__ keep)
 {
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines)
 		return;
-	const uint64_t a = line_start[l];
-	uint64_t b = (l + 1 < nlines)? line_start[l + 1] - 1 : nbytes;   // exclusive end, without the newline
-	// fgets-based reading stops a line at '\n'; a line that is just "\n" or "\r\n" has next_line[0] == '\n' (not 0 and not '@'), so the reference
-	// would try to parse it and fail on fs[1]; real SAM files have no such lines and abawaca_b200's host parser skips them, as does this one
-	while(b > a && (text[b - 1] == '\r' || text[b - 1] == '\n'))
+	auto [a, b] = line_extent(line_start, nlines, nbytes, l);
+	while(b > a && (trim_space? dev_isspace(text[b - 1]) : (text[b - 1] == '\r' || text[b - 1] == '\n')))
 		b--;
-	is_record[l] = (b > a && text[a] != '@')? 1u : 0u;
+	keep[l] = (b > a && text[a] != skip)? 1u : 0u;
 }
 
-__device__ __forceinline__ bool dev_isspace(char c) { return c == ' ' || (c >= '\t' && c <= '\r'); }
+// Flags the lines k_line_select keeps and numbers them (slot[l] = kept lines before l); *count is the number kept, after one wait.
+int select_lines(abw_ctx* ctx, const LineIndex& li, char skip, bool trim_space, DevBuf<uint32_t>& keep, DevBuf<uint64_t>& slot, uint64_t* count)
+{
+	DevBuf<uint64_t> total;
+	ABW_CUDA(ctx, keep.alloc(li.nlines));
+	ABW_CUDA(ctx, slot.alloc(li.nlines));
+	ABW_CUDA(ctx, total.alloc(1));
+	ABW_LAUNCH(ctx, k_line_select, abw_div_up(li.nlines, 256), 256, 0, li.text, li.nbytes, li.start.p, li.nlines, skip, trim_space, keep.p);
+	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, keep.p, slot.p, li.nlines, total.p));
+	ABW_CUDA(ctx, abw_fetch(ctx, count, total.p, sizeof(uint64_t)));
+	ABW_CUDA(ctx, abw_sync(ctx));
+	return ABW_OK;
+}
 
 // atoi on a field [p, e): optional white space, optional sign, digits (ReadMapping.cpp:39,41 call atoi on the field text)
 __device__ __forceinline__ int dev_atoi(const char* __restrict__ p, const char* __restrict__ e)
@@ -142,8 +195,9 @@ __global__ void __launch_bounds__(128) k_sam_parse(const char* __restrict__ text
 	const uint64_t slot = rec_slot[l];
 	if(slot >= cap)
 		return;
-	const char* p = text + line_start[l];
-	const char* e = text + ((l + 1 < nlines)? line_start[l + 1] - 1 : nbytes);
+	const auto [a, b] = line_extent(line_start, nlines, nbytes, l);
+	const char* p = text + a;
+	const char* e = text + b;
 	while(e > p && (e[-1] == '\r' || e[-1] == '\n'))       // chomp, ReadMappingReader.cpp:113
 		e--;
 	// walk the tab-separated fields (split('\t', ...), ReadMapping.cpp:36)
@@ -226,7 +280,7 @@ __global__ void k_fa_classify(const char* __restrict__ text, uint64_t nbytes, co
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines)
 		return;
-	uint64_t a = line_start[l], b = (l + 1 < nlines)? line_start[l + 1] : nbytes;
+	auto [a, b] = line_extent(line_start, nlines, nbytes, l);
 	while(a < b && dev_isspace(text[a]))
 		a++;
 	while(b > a && dev_isspace(text[b - 1]))
@@ -373,19 +427,6 @@ __device__ __forceinline__ double dev_atof(const char* __restrict__ p, const cha
 	return neg? -r : r;
 }
 
-// which lines are data lines: not empty after trimming trailing white space, not starting with '%'
-__global__ void k_lrn_is_row(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines, uint32_t* __restrict__ is_row)
-{
-	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if(l >= nlines)
-		return;
-	const uint64_t a = line_start[l];
-	uint64_t b = (l + 1 < nlines)? line_start[l + 1] : nbytes;
-	while(b > a && dev_isspace(text[b - 1]))
-		b--;
-	is_row[l] = (b > a && text[a] != '%')? 1u : 0u;
-}
-
 struct LrnFallback { uint64_t row; uint32_t col; uint32_t len; uint64_t off; };
 
 __global__ void __launch_bounds__(128) k_lrn_parse(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines,
@@ -399,8 +440,9 @@ __global__ void __launch_bounds__(128) k_lrn_parse(const char* __restrict__ text
 	const uint64_t row = row_slot[l];
 	if(row >= cap)
 		return;
-	const char* p = text + line_start[l];
-	const char* e = text + ((l + 1 < nlines)? line_start[l + 1] : nbytes);
+	const auto [a, b] = line_extent(line_start, nlines, nbytes, l);
+	const char* p = text + a;
+	const char* e = text + b;
 	while(e > p && dev_isspace(e[-1]))
 		e--;
 	uint32_t field = 0;
@@ -445,6 +487,14 @@ __global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ 
 }
 
 }  // namespace
+
+struct abw_fasta {
+	LineIndex lines;                          // the text; its line starts are released once the lines are classified
+	uint64_t nrec = 0;
+	DevBuf<uint64_t> line_a, hdr_before, chars_before, rec_id_off, rec_chars0;
+	DevBuf<uint32_t> line_len, rec_id_len;
+	std::vector<uint64_t> h_seq_len;
+};
 
 extern "C" {
 
@@ -503,43 +553,21 @@ int abw_parse_sam(abw_ctx* ctx, const abw_names* names, const char* text, uint64
 	*nreads = 0;
 	if(nbytes == 0)
 		return ABW_OK;
-	DevBuf<char> d_text;
-	const char* src = text;
-	if(!text_on_device) {
-		ABW_CUDA(ctx, d_text.alloc(nbytes + 16));
-		ABW_CUDA(ctx, cudaMemcpyAsync(d_text.p, text, nbytes, cudaMemcpyHostToDevice, ctx->stream));
-		src = d_text.p;
-	}
-	const unsigned int ntiles = abw_div_up(nbytes, LN_TILE);
-	DevBuf<uint32_t> tile_counts, is_record;
-	DevBuf<uint64_t> tile_offs, total, line_start, rec_slot;
 	DevBuf<int> d_err;
-	ABW_CUDA(ctx, tile_counts.alloc(ntiles));
-	ABW_CUDA(ctx, tile_offs.alloc(ntiles));
-	ABW_CUDA(ctx, total.alloc(2));
 	ABW_CUDA(ctx, d_err.alloc(1));
 	ABW_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(int), ctx->stream));
-	ABW_LAUNCH(ctx, k_sam_count_newlines, ntiles, LN_THREADS, 0, src, nbytes, tile_counts.p);
-	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, tile_counts.p, tile_offs.p, ntiles, total.p));
-	uint64_t nnl = 0;
-	ABW_CUDA(ctx, abw_fetch(ctx, &nnl, total.p, sizeof(uint64_t)));
-	ABW_CUDA(ctx, abw_sync(ctx));
-	const uint64_t nlines = nnl + 1;
-	ABW_CUDA(ctx, line_start.alloc(nlines));
-	ABW_CUDA(ctx, is_record.alloc(nlines));
-	ABW_CUDA(ctx, rec_slot.alloc(nlines));
-	ABW_LAUNCH(ctx, k_sam_line_starts, ntiles, LN_THREADS, 0, src, nbytes, tile_offs.p, line_start.p);
-	ABW_LAUNCH(ctx, k_sam_is_record, abw_div_up(nlines, 256), 256, 0, src, nbytes, line_start.p, nlines, is_record.p);
-	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, is_record.p, rec_slot.p, nlines, total.p + 1));
+	LineIndex li;
+	ABW_CHECK(line_index(ctx, text, nbytes, text_on_device, &li));
+	DevBuf<uint32_t> is_record;
+	DevBuf<uint64_t> rec_slot;
 	uint64_t nrec = 0;
-	ABW_CUDA(ctx, abw_fetch(ctx, &nrec, total.p + 1, sizeof(uint64_t)));
-	ABW_CUDA(ctx, abw_sync(ctx));
+	ABW_CHECK(select_lines(ctx, li, '@', false, is_record, rec_slot, &nrec));
 	*nreads = nrec;
 	if(nrec > cap)
 		return abw_fail(ctx, ABW_ERR_ARG, "abw_parse_sam: the record buffer is too small for this chunk (nreads holds the number needed)");
 	if(nrec) {
-		ABW_LAUNCH(ctx, k_sam_parse, abw_div_up(nlines, 128), 128, 0, src, nbytes, line_start.p, nlines, is_record.p, rec_slot.p, names->slot_hash.p, names->slot_index.p,
-		           names->nslots, names->blob.p, names->off.p, d_reads, cap, d_err.p);
+		ABW_LAUNCH(ctx, k_sam_parse, abw_div_up(li.nlines, 128), 128, 0, li.text, nbytes, li.start.p, li.nlines, is_record.p, rec_slot.p, names->slot_hash.p,
+		           names->slot_index.p, names->nslots, names->blob.p, names->off.p, d_reads, cap, d_err.p);
 	}
 	int h_err = 0;
 	ABW_CUDA(ctx, abw_fetch(ctx, &h_err, d_err.p, sizeof(int)));
@@ -560,46 +588,30 @@ int abw_fasta_scan(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_
 	ABW_ENTER(ctx);
 	abw_fasta* f = new abw_fasta();
 	int rc = [&]() -> int {
-		f->nbytes = nbytes;
 		if(nbytes == 0)
 			return ABW_OK;
-		if(!text_on_device) {
-			ABW_CUDA(ctx, f->text.alloc(nbytes + 16));
-			ABW_CUDA(ctx, cudaMemcpyAsync(f->text.p, text, nbytes, cudaMemcpyHostToDevice, ctx->stream));
-			f->d_text = f->text.p;
-		}
-		else
-			f->d_text = text;
-		const unsigned int ntiles = abw_div_up(nbytes, LN_TILE);
-		DevBuf<uint32_t> tile_counts, is_header, id_len;
-		DevBuf<uint64_t> tile_offs, total, line_start;
+		DevBuf<uint32_t> is_header, id_len;
+		DevBuf<uint64_t> total;
 		DevBuf<int> d_err;
-		ABW_CUDA(ctx, tile_counts.alloc(ntiles));
-		ABW_CUDA(ctx, tile_offs.alloc(ntiles));
-		ABW_CUDA(ctx, total.alloc(3));
+		ABW_CUDA(ctx, total.alloc(2));
 		ABW_CUDA(ctx, d_err.alloc(1));
 		ABW_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(int), ctx->stream));
-		ABW_LAUNCH(ctx, k_sam_count_newlines, ntiles, LN_THREADS, 0, f->d_text, nbytes, tile_counts.p);
-		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, tile_counts.p, tile_offs.p, ntiles, total.p));
-		uint64_t nnl = 0;
-		ABW_CUDA(ctx, abw_fetch(ctx, &nnl, total.p, sizeof(uint64_t)));
-		ABW_CUDA(ctx, abw_sync(ctx));
-		const uint64_t nlines = nnl + 1;
-		f->nlines = nlines;
-		ABW_CUDA(ctx, line_start.alloc(nlines));
+		LineIndex& li = f->lines;
+		ABW_CHECK(line_index(ctx, text, nbytes, text_on_device, &li));
+		const uint64_t nlines = li.nlines;
 		ABW_CUDA(ctx, f->line_a.alloc(nlines));
 		ABW_CUDA(ctx, f->line_len.alloc(nlines));
 		ABW_CUDA(ctx, is_header.alloc(nlines));
 		ABW_CUDA(ctx, id_len.alloc(nlines));
 		ABW_CUDA(ctx, f->hdr_before.alloc(nlines));
 		ABW_CUDA(ctx, f->chars_before.alloc(nlines));
-		ABW_LAUNCH(ctx, k_sam_line_starts, ntiles, LN_THREADS, 0, f->d_text, nbytes, tile_offs.p, line_start.p);
-		ABW_LAUNCH(ctx, k_fa_classify, abw_div_up(nlines, 256), 256, 0, f->d_text, nbytes, line_start.p, nlines, f->line_a.p, f->line_len.p, is_header.p, id_len.p, d_err.p);
+		ABW_LAUNCH(ctx, k_fa_classify, abw_div_up(nlines, 256), 256, 0, li.text, nbytes, li.start.p, nlines, f->line_a.p, f->line_len.p, is_header.p, id_len.p, d_err.p);
+		li.start.release();
 		// hdr_before[l] = header lines strictly before l; a header line itself gets its own record index, a sequence line index + 1 of its record
-		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, is_header.p, f->hdr_before.p, nlines, total.p + 1));
-		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, f->line_len.p, f->chars_before.p, nlines, total.p + 2));
+		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, is_header.p, f->hdr_before.p, nlines, total.p));
+		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, f->line_len.p, f->chars_before.p, nlines, total.p + 1));
 		uint64_t tot[2] = {0, 0};
-		ABW_CUDA(ctx, abw_fetch(ctx, tot, total.p + 1, 2 * sizeof(uint64_t)));
+		ABW_CUDA(ctx, abw_fetch(ctx, tot, total.p, 2 * sizeof(uint64_t)));
 		ABW_CUDA(ctx, abw_sync(ctx));
 		const uint64_t nrec = tot[0], nchars = tot[1];
 		f->nrec = nrec;
@@ -670,8 +682,9 @@ int abw_fasta_pack(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_order, ui
 	ABW_CUDA(ctx, d_dst.alloc(f->nrec));
 	if(f->nrec) {
 		ABW_CUDA(ctx, cudaMemcpyAsync(d_dst.p, rec_dst.data(), sizeof(uint64_t) * f->nrec, cudaMemcpyHostToDevice, ctx->stream));
-		const unsigned int blocks = (unsigned int)std::min<uint64_t>(abw_div_up(f->nlines * 32, 256), (uint64_t)ctx->sm_count * 16);
-		ABW_LAUNCH(ctx, k_fa_copy, blocks, 256, 0, f->d_text, f->line_a.p, f->line_len.p, f->hdr_before.p, f->chars_before.p, f->nlines, f->rec_chars0.p, d_dst.p, ascii.p);
+		const unsigned int blocks = (unsigned int)std::min<uint64_t>(abw_div_up(f->lines.nlines * 32, 256), (uint64_t)ctx->sm_count * 16);
+		ABW_LAUNCH(ctx, k_fa_copy, blocks, 256, 0, f->lines.text, f->line_a.p, f->line_len.p, f->hdr_before.p, f->chars_before.p, f->lines.nlines, f->rec_chars0.p, d_dst.p,
+		           ascii.p);
 	}
 	ABW_CUDA(ctx, abw_sync(ctx));      // rec_dst is a local
 	return abw_pack_sequences(ctx, ascii.p, 1, offsets.data(), nout, out);
@@ -685,49 +698,28 @@ int abw_parse_lrn(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_d
 	*nrows = 0;
 	if(nbytes == 0)
 		return ABW_OK;
-	DevBuf<char> d_text;
-	const char* src = text;
-	if(!text_on_device) {
-		ABW_CUDA(ctx, d_text.alloc(nbytes + 16));
-		ABW_CUDA(ctx, cudaMemcpyAsync(d_text.p, text, nbytes, cudaMemcpyHostToDevice, ctx->stream));
-		src = d_text.p;
-	}
-	const unsigned int ntiles = abw_div_up(nbytes, LN_TILE);
-	DevBuf<uint32_t> tile_counts, is_row, fb_count;
-	DevBuf<uint64_t> tile_offs, total, line_start, row_slot;
+	DevBuf<uint32_t> fb_count;
 	DevBuf<LrnFallback> fb;
 	DevBuf<int> d_err;
 	const uint32_t fb_cap = 1u << 20;
-	ABW_CUDA(ctx, tile_counts.alloc(ntiles));
-	ABW_CUDA(ctx, tile_offs.alloc(ntiles));
-	ABW_CUDA(ctx, total.alloc(2));
 	ABW_CUDA(ctx, d_err.alloc(1));
 	ABW_CUDA(ctx, fb_count.alloc(1));
 	ABW_CUDA(ctx, fb.alloc(fb_cap));
 	ABW_CUDA(ctx, cudaMemsetAsync(d_err.p, 0, sizeof(int), ctx->stream));
 	ABW_CUDA(ctx, cudaMemsetAsync(fb_count.p, 0, sizeof(uint32_t), ctx->stream));
-	ABW_LAUNCH(ctx, k_sam_count_newlines, ntiles, LN_THREADS, 0, src, nbytes, tile_counts.p);
-	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, tile_counts.p, tile_offs.p, ntiles, total.p));
-	uint64_t nnl = 0;
-	ABW_CUDA(ctx, abw_fetch(ctx, &nnl, total.p, sizeof(uint64_t)));
-	ABW_CUDA(ctx, abw_sync(ctx));
-	const uint64_t nlines = nnl + 1;
-	ABW_CUDA(ctx, line_start.alloc(nlines));
-	ABW_CUDA(ctx, is_row.alloc(nlines));
-	ABW_CUDA(ctx, row_slot.alloc(nlines));
-	ABW_LAUNCH(ctx, k_sam_line_starts, ntiles, LN_THREADS, 0, src, nbytes, tile_offs.p, line_start.p);
-	ABW_LAUNCH(ctx, k_lrn_is_row, abw_div_up(nlines, 256), 256, 0, src, nbytes, line_start.p, nlines, is_row.p);
-	ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, is_row.p, row_slot.p, nlines, total.p + 1));
+	LineIndex li;
+	ABW_CHECK(line_index(ctx, text, nbytes, text_on_device, &li));
+	DevBuf<uint32_t> is_row;
+	DevBuf<uint64_t> row_slot;
 	uint64_t nr = 0;
-	ABW_CUDA(ctx, abw_fetch(ctx, &nr, total.p + 1, sizeof(uint64_t)));
-	ABW_CUDA(ctx, abw_sync(ctx));
+	ABW_CHECK(select_lines(ctx, li, '%', true, is_row, row_slot, &nr));
 	*nrows = nr;
 	if(nr > cap_rows)
 		return abw_fail(ctx, ABW_ERR_ARG, "abw_parse_lrn: more data lines than the caller made room for (nrows holds the number found)");
 	if(nr == 0)
 		return ABW_OK;
-	ABW_LAUNCH(ctx, k_lrn_parse, abw_div_up(nlines, 128), 128, 0, src, nbytes, line_start.p, nlines, is_row.p, row_slot.p, D, cap_rows, d_keys, d_values, fb.p, fb_cap,
-	           fb_count.p, d_err.p);
+	ABW_LAUNCH(ctx, k_lrn_parse, abw_div_up(li.nlines, 128), 128, 0, li.text, nbytes, li.start.p, li.nlines, is_row.p, row_slot.p, D, cap_rows, d_keys, d_values, fb.p,
+	           fb_cap, fb_count.p, d_err.p);
 	int h_err = 0;
 	uint32_t h_fb = 0;
 	ABW_CUDA(ctx, abw_fetch(ctx, &h_err, d_err.p, sizeof(int)));
@@ -746,7 +738,7 @@ int abw_parse_lrn(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_d
 		for(const LrnFallback& f : h) {
 			tmp.assign((size_t)f.len + 1, 0);
 			if(text_on_device)
-				ABW_CUDA(ctx, cudaMemcpy(tmp.data(), src + f.off, f.len, cudaMemcpyDeviceToHost));
+				ABW_CUDA(ctx, cudaMemcpy(tmp.data(), li.text + f.off, f.len, cudaMemcpyDeviceToHost));
 			else
 				memcpy(tmp.data(), text + f.off, f.len);
 			const double v = atof(tmp.data());

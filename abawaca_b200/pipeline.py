@@ -15,6 +15,26 @@ import numpy as np
 from . import capi
 
 
+def _host_bytes(data):
+    """bytes, bytearray, memoryview or array -> (contiguous uint8 array, its pointer for the C ABI or None when it is empty)"""
+    arr = np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else np.ascontiguousarray(data, dtype=np.uint8)
+    return arr, capi._p(arr) if arr.size else None
+
+
+def _first_of_each_name(ctx, data, h, n, get):
+    """(names, record indices, lengths) of the scaffolds among the n records of `data`: the first of every name, in byte-wise name order (abawaca-build.cpp:482-490)"""
+    name_off = np.zeros(n, dtype=np.uint64)
+    name_len = np.zeros(n, dtype=np.uint32)
+    seq_len = np.zeros(n, dtype=np.uint64)
+    ctx.check(get(ctx.h, h, capi._p(name_off), capi._p(name_len), capi._p(seq_len)))
+    first = {}
+    for i in range(n):
+        first.setdefault(bytes(data[int(name_off[i]):int(name_off[i]) + int(name_len[i])]), i)
+    names = sorted(first)
+    order = np.array([first[k] for k in names], dtype=np.uint32)
+    return [k.decode() for k in names], order, seq_len[order]
+
+
 class SamParser:
     """SAM text -> abw_read records on the device (abw_names_create / abw_parse_sam)."""
 
@@ -30,14 +50,14 @@ class SamParser:
 
     def parse(self, text, d_reads, cap):
         """text: bytes or uint8 array (host), ending at a line boundary.  Returns the number of records written to d_reads."""
-        arr = np.frombuffer(text, dtype=np.uint8) if isinstance(text, (bytes, bytearray)) else np.ascontiguousarray(text, dtype=np.uint8)
+        arr, p = _host_bytes(text)
         n = C.c_uint64()
-        self.ctx.check(self.ctx.lib.abw_parse_sam(self.ctx.h, self.h, capi._p(arr) if arr.size else None, arr.size, 0, C.c_void_p(d_reads), cap, C.byref(n)))
+        self.ctx.check(self.ctx.lib.abw_parse_sam(self.ctx.h, self.h, p, arr.size, 0, C.c_void_p(d_reads), cap, C.byref(n)))
         return int(n.value)
 
     def parse_to_host(self, text):
         """convenience for tests: parse one chunk and fetch the records"""
-        arr = np.frombuffer(text, dtype=np.uint8) if isinstance(text, (bytes, bytearray)) else np.ascontiguousarray(text, dtype=np.uint8)
+        arr, _ = _host_bytes(text)
         cap = int(np.count_nonzero(arr == 10)) + 1
         d = self.ctx.alloc(max(cap, 1) * 16)
         try:
@@ -67,8 +87,8 @@ class BamReader:
         self.h = h
 
     def feed(self, data):
-        arr = np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else np.ascontiguousarray(data, dtype=np.uint8)
-        self.ctx.check(self.ctx.lib.abw_bam_feed(self.ctx.h, self.h, capi._p(arr) if arr.size else None, arr.size))
+        arr, p = _host_bytes(data)
+        self.ctx.check(self.ctx.lib.abw_bam_feed(self.ctx.h, self.h, p, arr.size))
 
     def finish(self):
         d, n = C.c_void_p(), C.c_uint64()
@@ -93,13 +113,13 @@ class BamReader:
 def parse_lrn_rows(ctx, text, D):
     """data lines of a .lrn file (bytes, after the four header lines) -> (keys uint64 [n], device pointer of the row-major [n][D] matrix, n).
     The caller frees the matrix with ctx.free()."""
-    arr = np.frombuffer(text, dtype=np.uint8)
+    arr, p = _host_bytes(text)
     cap = int(np.count_nonzero(arr == 10)) + 1
     d_keys = ctx.alloc(cap * 8)
     d_vals = ctx.alloc(max(cap * D, 1) * 8)
     n = C.c_uint64()
     try:
-        ctx.check(ctx.lib.abw_parse_lrn(ctx.h, capi._p(arr) if arr.size else None, arr.size, 0, D, C.c_void_p(d_keys), C.c_void_p(d_vals), cap, C.byref(n)))
+        ctx.check(ctx.lib.abw_parse_lrn(ctx.h, p, arr.size, 0, D, C.c_void_p(d_keys), C.c_void_p(d_vals), cap, C.byref(n)))
     except Exception:
         ctx.free(d_keys); ctx.free(d_vals)
         raise
@@ -137,58 +157,37 @@ def format_lrn_rows(ctx, d_values, ld, ncols, rows=None, nlines=None, fmt=capi.T
 
 
 def fasta_to_seqset(ctx, text):
-    """FASTA text (bytes) -> (seqset handle, names in scaffold order, lengths): records indexed on the device (abw_fasta_scan), the first record of
-    every name kept, scaffolds in byte-wise name order (abawaca-build.cpp:482-490), sequences packed by abw_fasta_pack."""
+    """FASTA text (bytes) -> (seqset handle, names in scaffold order, lengths): records indexed on the device (abw_fasta_scan), packed by abw_fasta_pack"""
     L = ctx.lib
-    arr = np.frombuffer(text, dtype=np.uint8)
+    arr, p = _host_bytes(text)
     f = C.c_void_p()
-    ctx.check(L.abw_fasta_scan(ctx.h, capi._p(arr) if arr.size else None, arr.size, 0, C.byref(f)))
+    ctx.check(L.abw_fasta_scan(ctx.h, p, arr.size, 0, C.byref(f)))
     try:
-        n = int(L.abw_fasta_count(f))
-        id_off = np.zeros(n, dtype=np.uint64)
-        id_len = np.zeros(n, dtype=np.uint32)
-        seq_len = np.zeros(n, dtype=np.uint64)
-        ctx.check(L.abw_fasta_get(ctx.h, f, capi._p(id_off), capi._p(id_len), capi._p(seq_len)))
-        first = {}
-        for i in range(n):
-            name = bytes(text[int(id_off[i]):int(id_off[i]) + int(id_len[i])])
-            first.setdefault(name, i)
-        names = sorted(first)
-        order = np.array([first[k] for k in names], dtype=np.uint32)
+        names, order, lengths = _first_of_each_name(ctx, text, f, int(L.abw_fasta_count(f)), L.abw_fasta_get)
         ss = C.c_void_p()
         ctx.check(L.abw_fasta_pack(ctx.h, f, capi._p(order), order.size, C.byref(ss)))
-        return ss, [k.decode() for k in names], seq_len[order]
+        return ss, names, lengths
     finally:
         L.abw_fasta_destroy(f)
 
 
 def twobit_to_seqset(ctx, data):
     """UCSC .2bit file image (bytes) -> (seqset handle, names in scaffold order, lengths), the counterpart of fasta_to_seqset: header and records
-    parsed by abw_twobit_scan, the first record of every name kept, scaffolds in byte-wise name order, the file copied to the device once as it is
-    and decoded there (abw_twobit_pack)."""
+    parsed by abw_twobit_scan, the file copied to the device once as it is and decoded there (abw_twobit_pack)."""
     L = ctx.lib
-    arr = np.frombuffer(data, dtype=np.uint8)
+    arr, p = _host_bytes(data)
     t = C.c_void_p()
-    ctx.check(L.abw_twobit_scan(ctx.h, capi._p(arr) if arr.size else None, arr.size, C.byref(t)))
+    ctx.check(L.abw_twobit_scan(ctx.h, p, arr.size, C.byref(t)))
     d_file = None
     try:
-        n = int(L.abw_twobit_count(t))
-        name_off = np.zeros(n, dtype=np.uint64)
-        name_len = np.zeros(n, dtype=np.uint32)
-        seq_len = np.zeros(n, dtype=np.uint64)
-        ctx.check(L.abw_twobit_get(ctx.h, t, capi._p(name_off), capi._p(name_len), capi._p(seq_len)))
-        first = {}
-        for i in range(n):
-            first.setdefault(bytes(data[int(name_off[i]):int(name_off[i]) + int(name_len[i])]), i)
-        names = sorted(first)
-        order = np.array([first[k] for k in names], dtype=np.uint32)
+        names, order, lengths = _first_of_each_name(ctx, data, t, int(L.abw_twobit_count(t)), L.abw_twobit_get)
         d_file = ctx.alloc(max(arr.size, 1))
         if arr.size:
             ctx.to_device(d_file, arr)
         ss = C.c_void_p()
         ctx.check(L.abw_twobit_pack(ctx.h, t, C.c_void_p(d_file), 0, capi._p(order), order.size, C.byref(ss)))
         ctx.synchronize()
-        return ss, [k.decode() for k in names], seq_len[order]
+        return ss, names, lengths
     finally:
         if d_file is not None:
             ctx.free(d_file)

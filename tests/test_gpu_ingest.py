@@ -119,6 +119,9 @@ def test_errors_like_the_reference(ctx):
             sp.parse_to_host(b"r\t0\ts1\t1\t42\t4M\t*\t0\t0\tACGT\n")
         with pytest.raises(capi.AbwError, match="MD:Z"):
             sp.parse_to_host(b"r\t0\ts1\t1\t42\t4M\t*\t0\t0\tACGT\tIIII\tMD:Z:2a1\n")
+        for blank in (b" ", b"  \t ", b" \r"):          # chomp strips only '\r' and '\n': a line of blanks is a record, as the reference reads it
+            with pytest.raises(capi.AbwError, match="fewer than 11"):
+                sp.parse_to_host(b"r\t0\ts1\t1\t42\t4M\t*\t0\t0\tACGT\tIIII\n" + blank + b"\n")
     finally:
         sp.close()
 
@@ -300,6 +303,14 @@ def test_lrn_values_equal_atof(ctx):
     libc.atof.restype = ctypes.c_double
     exp = np.array([[libc.atof(v.encode()) for v in row] for row in rows])
     assert np.array_equal(got.view(np.uint64), exp.view(np.uint64)), [(v, g, e) for v, g, e in zip(sum(rows, []), got.ravel(), exp.ravel()) if np.float64(g).view(np.uint64) != np.float64(e).view(np.uint64)][:10]
+    # a data line ends at its last non-blank character: CRLF, trailing blanks and tabs, lines of blanks (skipped), no final newline
+    body = ["%d\t%s" % (10 * r + 3, "\t".join(row)) for r, row in enumerate(rows)]
+    for text in ("\r\n".join(body) + "\r\n", " \t\n".join(body) + "\t ", "\n \t  \n".join(body) + "\n \n", "\n".join(body)):
+        keys2, d_vals2, n2 = pipeline.parse_lrn_rows(ctx, text.encode(), D)
+        got2 = np.zeros((n2, D), dtype=np.float64)
+        ctx.to_host(got2, d_vals2)
+        ctx.free(d_vals2)
+        assert n2 == len(rows) and keys2.tolist() == keys.tolist() and np.array_equal(got2.view(np.uint64), got.view(np.uint64))
     with pytest.raises(capi.AbwError, match="number of tab-separated fields"):
         pipeline.parse_lrn_rows(ctx, b"1\t0.5\t0.25\n2\t0.5\n", 2)
 
@@ -324,3 +335,155 @@ def test_lrn_text_of_the_golden_sets(ctx, name):
         res = pipeline.search(ctx, d_vals, prob["dp2scaf"], prob["T"], prob["len"], prob["scgmask"], layout=capi.LAYOUT_ROWMAJOR, values_on_device=True, nrows=n, D=D, ld=D)
         assert res.scaf2cluster.tolist() == ref.scaf2cluster.tolist() and [(r.id, r.split, r.best.dim, r.best.value) for r in res.recs] == [(r.id, r.split, r.best.dim, r.best.value) for r in ref.recs]
     ctx.free(d_vals)
+
+
+# ---------------------------------------------------------------------------------------------------
+# Text already on the device (text_on_device = 1), at aligned and unaligned addresses, with newlines on the 4 KB tiles of the line index
+# ---------------------------------------------------------------------------------------------------
+TILE = 4096
+
+
+def tile_edge_texts(make, minlen):
+    """texts of lines make(i, length) with newlines at the last byte of a tile, at the first byte of the next (alone, and after an empty line),
+    and texts of exactly one tile with and without a final newline; every other line is at least minlen bytes long"""
+    out = []
+    for marks, end in (([TILE - 1], 3 * TILE + 77), ([TILE], 2 * TILE + 1000), ([2 * TILE - 1, 2 * TILE], 3 * TILE), ([TILE - 1], TILE), ([], TILE)):
+        cuts = sorted(marks + [p for p in range(120, end, 120) if all(abs(p - m) > minlen for m in marks + [end])])
+        lines, prev = [], -1
+        for i, c in enumerate(cuts):
+            lines.append(make(i, c - prev - 1) + "\n")
+            prev = c
+        lines.append(make(len(cuts), end - prev - 1))
+        text = "".join(lines).encode()
+        assert len(text) == end and all(text[m] == 10 for m in marks)
+        out.append(text)
+    return out
+
+
+def _pad(head, n, tail="", fill="x"):
+    assert n == 0 or len(head) + len(tail) <= n
+    return head + fill * (n - len(head) - len(tail)) + tail if n else ""
+
+
+def sam_line(i, n):
+    if i % 11 == 3:
+        return _pad("@CO\t", n)
+    return _pad("r%d\t%d\ts%d\t%d\t42\t4M\t*\t0\t0\tACGT\tIIII\tMD:Z:%dA%d\tXP:Z:" % (i, 16 * (i % 2), i % 3, i + 1, i % 3, 3 - i % 3), n)
+
+
+def fasta_line(i, n):
+    if i % 6 == 0:
+        return _pad(">c%d " % i, n)
+    return ("ACGTTGCANC" * (n // 10 + 2))[i % 10:i % 10 + n]
+
+
+def lrn_line(i, n):
+    if i % 13 == 5:
+        return _pad("%", n)
+    v = "1e30" if i % 7 == 3 else "%d.25" % i              # 1e30 is converted by the host, which reads it from the device text
+    return _pad("%d\t" % (i + 1), n, v + "\t0.5", fill="0")
+
+
+def _device_text(ctx, text, off):
+    """device buffer holding text at byte offset off -> (buffer, text pointer)"""
+    buf = np.zeros(len(text) + 32, dtype=np.uint8)
+    buf[off:off + len(text)] = np.frombuffer(text, dtype=np.uint8)
+    d = ctx.alloc(buf.size)
+    ctx.to_device(d, buf)
+    return d, d + off
+
+
+def _sam_records(ctx, sp, text, ptr):
+    import ctypes as C
+    from abawaca_b200 import capi
+    cap = text.count(b"\n") + 1
+    d = ctx.alloc(cap * 16)
+    n = C.c_uint64()
+    try:
+        ctx.check(ctx.lib.abw_parse_sam(ctx.h, sp.h, C.c_void_p(ptr), len(text), 1, C.c_void_p(d), cap, C.byref(n)))
+        out = np.zeros(n.value, dtype=capi.READ_DTYPE)
+        ctx.to_host(out, d)
+        return out
+    finally:
+        ctx.free(d)
+
+
+def _fasta_records(ctx, text, ptr):
+    """ids, lengths, N and GC counts and 50-base k-mer rows of all records, through abw_fasta_scan of the host text (ptr None) or of device text"""
+    import ctypes as C
+    from abawaca_b200 import capi, pipeline
+    L = ctx.lib
+    arr = np.frombuffer(text, dtype=np.uint8)
+    f = C.c_void_p()
+    ctx.check(L.abw_fasta_scan(ctx.h, capi._p(arr) if ptr is None else C.c_void_p(ptr), len(text), 0 if ptr is None else 1, C.byref(f)))
+    try:
+        n = int(L.abw_fasta_count(f))
+        id_off, id_len, seq_len = np.zeros(n, dtype=np.uint64), np.zeros(n, dtype=np.uint32), np.zeros(n, dtype=np.uint64)
+        ctx.check(L.abw_fasta_get(ctx.h, f, capi._p(id_off), capi._p(id_len), capi._p(seq_len)))
+        order = np.arange(n, dtype=np.uint32)
+        ss = C.c_void_p()
+        ctx.check(L.abw_fasta_pack(ctx.h, f, capi._p(order), n, C.byref(ss)))
+    finally:
+        L.abw_fasta_destroy(f)
+    offsets = np.zeros(n + 1, dtype=np.uint64)
+    offsets[1:] = np.cumsum(seq_len)
+    p = capi.default_params()
+    p.window_size = 50
+    fb = pipeline.build_features(ctx, None, offsets, [], seqset=ss, params=p)
+    nN, nGC = np.zeros(n, dtype=np.uint64), np.zeros(n, dtype=np.uint64)
+    ctx.check(L.abw_seqset_stats(ctx.h, fb.seqset, capi._p(nN), capi._p(nGC)))
+    out = [id_off.tolist(), id_len.tolist(), seq_len.tolist(), nN.tolist(), nGC.tolist(), fb.rows_host().tobytes()]
+    fb.close()
+    return out
+
+
+def _lrn_rows(ctx, text, ptr, D):
+    import ctypes as C
+    cap = text.count(b"\n") + 1
+    d_keys, d_vals = ctx.alloc(cap * 8), ctx.alloc(cap * D * 8)
+    n = C.c_uint64()
+    try:
+        ctx.check(ctx.lib.abw_parse_lrn(ctx.h, C.c_void_p(ptr), len(text), 1, D, C.c_void_p(d_keys), C.c_void_p(d_vals), cap, C.byref(n)))
+        keys, vals = np.zeros(n.value, dtype=np.uint64), np.zeros((n.value, D), dtype=np.float64)
+        ctx.to_host(keys, d_keys)
+        ctx.to_host(vals, d_vals)
+        return keys, vals
+    finally:
+        ctx.free(d_keys); ctx.free(d_vals)
+
+
+@pytest.mark.parametrize("fmt", ["sam", "fasta", "lrn"])
+def test_text_on_the_device(ctx, fmt):
+    """each parser returns for text on the device, at byte offsets 0, 1 and 15 of a buffer, exactly what it returns for the same text on the host;
+    the texts put newlines on the last byte of a 4 KB tile and the first byte of the next, and are one tile long"""
+    from abawaca_b200 import pipeline
+    names = ["s0", "s1", "s2"]
+    sp = pipeline.SamParser(ctx, names)
+    try:
+        for text in tile_edge_texts({"sam": sam_line, "fasta": fasta_line, "lrn": lrn_line}[fmt], 64):
+            if fmt == "sam":
+                want = sp.parse_to_host(text)
+                assert [tuple(int(x) for x in r) for r in want.tolist()] == ref_parse_sam(text.decode(), {n: i for i, n in enumerate(names)})
+            elif fmt == "fasta":
+                want = _fasta_records(ctx, text, None)
+                assert [bytes(text[a:a + l]).decode() for a, l in zip(want[0], want[1])] == [r[0] for r in ref_read_fasta(text.decode())]
+            else:
+                keys, d_vals, n = pipeline.parse_lrn_rows(ctx, text, 2)
+                vals = np.zeros((n, 2), dtype=np.float64)
+                ctx.to_host(vals, d_vals)
+                ctx.free(d_vals)
+                assert n > 10 and 1e30 in vals[:, 0]
+            for off in (0, 1, 15):
+                d, ptr = _device_text(ctx, text, off)
+                try:
+                    if fmt == "sam":
+                        assert _sam_records(ctx, sp, text, ptr).tobytes() == want.tobytes()
+                    elif fmt == "fasta":
+                        assert _fasta_records(ctx, text, ptr) == want
+                    else:
+                        k2, v2 = _lrn_rows(ctx, text, ptr, 2)
+                        assert np.array_equal(k2, keys) and np.array_equal(v2.view(np.uint64), vals.view(np.uint64))
+                finally:
+                    ctx.free(d)
+    finally:
+        sp.close()
