@@ -12,7 +12,6 @@
 #include <fstream>
 #include <iostream>
 #include <set>
-#include <chrono>
 
 using namespace abwh;
 
@@ -132,8 +131,9 @@ struct Model {
 	std::vector<uint32_t> dp2scaf;              // 0-based scaffold of 0-based dp
 	std::vector<unsigned long> dp_name;
 	std::vector<std::string> dim_names;
-	std::vector<double> values;                 // column major [D][N]
-	double* d_rows = nullptr;                   // the same on the device, row major [N][D] (row = 0-based dp id): what the cluster dumps print
+	std::vector<double> rows;                   // the .lrn rows in file order, row major [rows][D]
+	std::vector<uint64_t> row_of_dp;            // row of rows of 0-based dp
+	double* d_rows = nullptr;                   // on the device in dp order, row major [N][D]: what the search reads and the cluster dumps print
 	std::vector<uint64_t> scgmask;              // [S][W]
 	uint32_t W = 1;
 	int total_num_scgs = 0;
@@ -264,7 +264,6 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 			if(M.dim_names.size() != ndims) { std::cerr << "Fatal error: number of dimensions found in line 4 (" << M.dim_names.size() << ") is different than expected (" << ndims << ")" << std::endl; exit(-1); }
 		}
 		const size_t N = M.N(), D = ndims;
-		M.values.assign(D * N, 0.0);
 		std::vector<char> seen(N, 0);
 		// the datapoint lines are parsed on the device (abw_parse_lrn): keys and a row-major matrix come back
 		std::string body;
@@ -290,29 +289,27 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 		if(entry > ndps) { std::cerr << "Fatal error: number of datapoint lines found is higher than expected (" << ndps << "), file " << P.lrn_file << std::endl; exit(-1); }
 		if(entry != ndps) { std::cerr << "Fatal error: number of datapoint lines found (" << entry << ") is different than expected (" << ndps << "), file " << P.lrn_file << std::endl; exit(-1); }
 		std::vector<uint64_t> keys(entry);
-		std::vector<double> rows_rm(entry * D);
+		M.rows.resize(entry * D);
 		if(entry) {
 			ABWH_CHECK(ctx, abw_copy_to_host(ctx, keys.data(), d_keys, entry * sizeof(uint64_t)));
-			ABWH_CHECK(ctx, abw_copy_to_host(ctx, rows_rm.data(), d_vals, entry * D * sizeof(double)));
+			ABWH_CHECK(ctx, abw_copy_to_host(ctx, M.rows.data(), d_vals, entry * D * sizeof(double)));
 		}
 		ABWH_CHECK(ctx, abw_device_free(ctx, d_keys));
-		std::vector<uint64_t> row_of_dp(N);
+		M.row_of_dp.assign(N, 0);
 		for(uint64_t r = 0; r < entry; r++) {
 			auto it = dp_name2id.find((unsigned long)keys[r]);
 			if(it != dp_name2id.end()) {
 				const size_t dp = it->second - 1;
 				seen[dp] = 1;
-				row_of_dp[dp] = r;
-				for(size_t d = 0; d < D; d++)
-					M.values[d * N + dp] = rows_rm[r * D + d];
+				M.row_of_dp[dp] = r;
 			}
 		}
 		for(size_t i = 0; i < N; i++)
 			if(!seen[i])
 				throw std::invalid_argument("datapoint " + std::to_string(M.dp_name[i]) + " of " + P.names_file + " has no row in " + P.lrn_file);
-		// the rows of the file put into dp order where they already are, for the cluster dumps
+		// the rows of the file put into dp order where they already are, for the search and the cluster dumps
 		ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<size_t>(N * D, 1) * sizeof(double), (void**)&M.d_rows));
-		ABWH_CHECK(ctx, abw_gather_rows(ctx, d_vals, D, row_of_dp.data(), 0, N, (uint32_t)D, M.d_rows, D));
+		ABWH_CHECK(ctx, abw_gather_rows(ctx, d_vals, D, M.row_of_dp.data(), 0, N, (uint32_t)D, M.d_rows, D));
 		ABWH_CHECK(ctx, abw_device_free(ctx, d_vals));
 	}
 	// SCG database (SCGdb.cpp:58-120): number of names in scg.list; gene -> SCG, gene = <scaffold>_<non-zero integer>
@@ -360,18 +357,6 @@ static void weighted_stats(const std::vector<std::pair<size_t, double>>& data, d
 	stdev = sqrt(stdev / (total - 1));
 }
 
-// ABW_TIMING=1: wall-clock milestones on stderr (where the time of the drop-in program goes: CUDA start-up, text in, search, text out)
-static void milestone(const char* what)
-{
-	static const bool on = getenv("ABW_TIMING") != nullptr;
-	static auto t0 = std::chrono::steady_clock::now();
-	if(!on)
-		return;
-	const auto t1 = std::chrono::steady_clock::now();
-	fprintf(stderr, "[abw timing] %-28s %8.3f s\n", what, std::chrono::duration<double>(t1 - t0).count());
-	t0 = t1;
-}
-
 int main(int argc, const char** argv)
 {
 	milestone("start");
@@ -403,7 +388,8 @@ int main(int argc, const char** argv)
 		abw_default_params(&prm);
 		prm.min_reported_score = 0;                 // also report the best separation of terminal clusters, as the reference's log does
 		abw_search* search = nullptr;
-		ABWH_CHECK(ctx, abw_search_create(ctx, M.values.data(), 0, ABW_LAYOUT_COLMAJOR, N, N, nullptr, N, (uint32_t)D, M.dp2scaf.data(), (uint32_t)S, M.T.data(), M.len.data(),
+		// the search reads M.d_rows where it lies: it is freed after abw_search_destroy
+		ABWH_CHECK(ctx, abw_search_create(ctx, M.d_rows, 1, ABW_LAYOUT_ROWMAJOR, D, N, nullptr, N, (uint32_t)D, M.dp2scaf.data(), (uint32_t)S, M.T.data(), M.len.data(),
 		                                  M.scgmask.data(), M.W, &prm, P.strategy, &search));
 		std::vector<abw_cluster_rec> recs(2 * N / std::max<uint32_t>(prm.cluster_ndps_threshold, 1) + 64);
 		std::vector<uint32_t> dp2cluster(N), scaf2cluster(S);
@@ -415,7 +401,6 @@ int main(int argc, const char** argv)
 			return -1;
 		}
 		recs.resize(nrec);
-		abw_search_destroy(search);
 		milestone("search");
 
 		// membership of every evaluated cluster: terminal bins bubble up to their ancestors
@@ -424,47 +409,11 @@ int main(int argc, const char** argv)
 		std::map<uint32_t, std::vector<uint32_t>> dps_of;      // 0-based datapoints, ascending
 		for(size_t i = 0; i < N; i++)
 			for(uint32_t c = dp2cluster[i]; c != 0; c = parent_of[c]) dps_of[c].push_back((uint32_t)i);
-		// the data lines of the cluster dumps: "<dp+1>" and "\t%lf" per value (ClusterWriter.cpp:81-98), made on the device in pieces of at most LRN_CHUNK bytes
-		const uint64_t LRN_CHUNK = (uint64_t)64 << 20;
+		// scratch of the cluster dumps (write_lrn)
 		char* d_text = nullptr;
 		ABWH_CHECK(ctx, abw_device_alloc(ctx, LRN_CHUNK, (void**)&d_text));
 		std::vector<char> text;
 		std::vector<uint64_t> rows;
-		auto write_lrn = [&](uint32_t id, const std::vector<uint32_t>& dps) {
-			FILE* fp = fopen((P.cluster_dir + "/" + std::to_string(id) + ".lrn").c_str(), "w");
-			if(!fp) { std::cerr << "Fatal error: could write to file " << P.cluster_dir << "/" << id << ".lrn" << std::endl << std::endl; exit(-1); }
-			fprintf(fp, "%c %lu\n", '%', (unsigned long)dps.size());
-			fprintf(fp, "%c %lu\n", '%', (unsigned long)(D + 1));
-			fprintf(fp, "%c 9", '%');
-			for(size_t d = 0; d < D; d++) fprintf(fp, "\t1");
-			fprintf(fp, "\n%c Key", '%');
-			for(size_t d = 0; d < D; d++) fprintf(fp, "\t%s", M.dim_names[d].c_str());
-			fprintf(fp, "\n");
-			rows.assign(dps.begin(), dps.end());     // the reference writes these rows in unordered_set order (quirk Q9); here ascending dp id
-			for(uint64_t line0 = 0; line0 < rows.size();) {
-				uint64_t done = 0, nbytes = 0;
-				ABWH_CHECK(ctx, abw_format_lrn(ctx, M.d_rows, D, 0, (uint32_t)D, rows.data(), 0, line0, rows.size(), ABW_TEXT_LF, d_text, LRN_CHUNK, &done, &nbytes));
-				text.resize(std::max<size_t>(text.size(), nbytes));
-				ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
-				if(fwrite(text.data(), 1, nbytes, fp) != nbytes) { std::cerr << "Fatal error: could write to file " << P.cluster_dir << "/" << id << ".lrn" << std::endl << std::endl; exit(-1); }
-				line0 += done;
-			}
-			fclose(fp);
-		};
-		// SCG tallies of an arbitrary scaffold list on the host (SCGdb.cpp:6-18,41-55); the terminal ones also come back from the device
-		auto scg_of = [&](const std::vector<uint32_t>& assigned, double& nunique, double& avg) {
-			std::vector<uint64_t> un(M.W, 0);
-			size_t copies = 0;
-			for(uint32_t s : assigned)
-				for(uint32_t w = 0; w < M.W; w++) {
-					un[w] |= M.scgmask[(size_t)s * M.W + w];
-					copies += (size_t)__builtin_popcountll(M.scgmask[(size_t)s * M.W + w]);
-				}
-			size_t u = 0;
-			for(uint32_t w = 0; w < M.W; w++) u += (size_t)__builtin_popcountll(un[w]);
-			nunique = (double)u;
-			avg = (copies == 0)? 0 : (double)copies / (double)u;
-		};
 		auto gc_cvg_of = [&](const std::vector<uint32_t>& assigned, double& avg_gc, double& sd_gc, double& avg_cvg, double& sd_cvg) {
 			std::vector<std::pair<size_t, double>> gc, cvg;
 			for(uint32_t s : assigned) {
@@ -508,18 +457,14 @@ int main(int argc, const char** argv)
 							fa << up.substr(i, 60) << std::endl;
 					}
 				}
-				double nunique, avg_copies, avg_gc, sd_gc, avg_cvg = -1, sd_cvg = -1;
-				scg_of(assigned, nunique, avg_copies);
-				// ClusterQuality::gc / cvg of the bin come back with its record (abw_search_set_scaffold_stats)
-				avg_gc = r.gc_avg; sd_gc = r.gc_sd; avg_cvg = r.cvg_avg; sd_cvg = r.cvg_sd;
-				summary << r.id << '\t' << assigned.size() << '\t' << cur_dps.size() << '\t' << r.total_size << '\t' << int(1000 * avg_gc) / 10.0 << '\t' << int(1000 * sd_gc) / 100.0
-				        << '\t' << int(10 * avg_cvg) / 10.0 << '\t' << int(10 * sd_cvg) / 10.0 << '\t' << nunique << '\t' << int(100 * avg_copies) / 100.0 << std::endl;
+				// ClusterQuality::scg, gc and cvg of the bin come back with its record (gc and cvg: abw_search_set_scaffold_stats)
+				summary << r.id << '\t' << assigned.size() << '\t' << cur_dps.size() << '\t' << r.total_size << '\t' << int(1000 * r.gc_avg) / 10.0 << '\t' << int(1000 * r.gc_sd) / 100.0
+				        << '\t' << int(10 * r.cvg_avg) / 10.0 << '\t' << int(10 * r.cvg_sd) / 10.0 << '\t' << r.scg_unique << '\t' << int(100 * r.scg_avg) / 100.0 << std::endl;
 				continue;
 			}
 			// the split: raw sides on the winning dimension, then the vote (ClusterSeparator.cpp:25-54,82-134)
-			const double* col = &M.values[(size_t)(r.best.dim - 1) * N];
 			std::vector<uint32_t> low, high;
-			for(uint32_t dp : cur_dps) (col[dp] <= r.best.value? low : high).push_back(dp);
+			for(uint32_t dp : cur_dps) (M.rows[M.row_of_dp[dp] * D + r.best.dim - 1] <= r.best.value? low : high).push_back(dp);
 			const bool swapped = high.size() < low.size();
 			const std::vector<uint32_t>& raw1 = swapped? high : low;
 			const std::vector<uint32_t>& raw2 = swapped? low : high;
@@ -545,7 +490,18 @@ int main(int argc, const char** argv)
 			const std::vector<uint32_t>* raw[2] = {&raw1, &raw2};
 			for(int ch = 0; ch < 2; ch++) {
 				const std::vector<uint32_t>& cdps = dps_of[child[ch]];
-				write_lrn(child[ch], cdps);
+				// <id>.lrn: "<dp+1>" and "\t%lf" per value (ClusterWriter.cpp:81-98); the reference writes the rows in unordered_set order (quirk Q9), here
+				// ascending dp id
+				{
+					const std::string path = P.cluster_dir + "/" + std::to_string(child[ch]) + ".lrn";
+					FILE* fp = fopen(path.c_str(), "w");
+					rows.assign(cdps.begin(), cdps.end());
+					if(!fp || !write_lrn(ctx, fp, M.dim_names, M.d_rows, D, rows.data(), rows.size(), ABW_TEXT_LF, d_text, text)) {
+						std::cerr << "Fatal error: could write to file " << path << std::endl << std::endl;
+						exit(-1);
+					}
+					fclose(fp);
+				}
 				// <id>.scaf-stats.txt (ClusterWriter.cpp:35-66) and <id>.scaf-cluster.txt (:22-32)
 				{
 					std::map<uint32_t, size_t> in, out;
@@ -565,8 +521,9 @@ int main(int argc, const char** argv)
 					for(uint32_t s : *assigned[ch]) fprintf(fp, "%s\t%u\n", M.scaf_names[s].c_str(), child[ch]);
 					fclose(fp);
 				}
-				double nunique, avg_copies, avg_gc, sd_gc, avg_cvg, sd_cvg;
-				scg_of(*assigned[ch], nunique, avg_copies);
+				uint32_t nunique;
+				double avg_copies, avg_gc, sd_gc, avg_cvg, sd_cvg;
+				ABWH_CHECK(ctx, abw_cluster_scg(ctx, search, assigned[ch]->data(), (uint32_t)assigned[ch]->size(), &nunique, &avg_copies));
 				gc_cvg_of(*assigned[ch], avg_gc, sd_gc, avg_cvg, sd_cvg);
 				for(std::ostream* os : {(std::ostream*)&std::cerr, (std::ostream*)&log})
 					*os << '[' << get_time() << ']' << " Cluster " << child[ch] << ", " << cdps.size() << " datapoints, " << nunique << " unique SCGs (" << avg_copies
@@ -574,6 +531,7 @@ int main(int argc, const char** argv)
 			}
 		}
 		ABWH_CHECK(ctx, abw_device_free(ctx, d_text));
+		abw_search_destroy(search);
 		ABWH_CHECK(ctx, abw_device_free(ctx, M.d_rows));
 		milestone("logs, fasta and cluster dumps");
 		// dp2cluster.txt has a row for dp 0 as well (abawaca.cpp:199, quirk Q10)

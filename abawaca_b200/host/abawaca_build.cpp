@@ -4,16 +4,15 @@
 //                                      file abw_twobit_scan / abw_twobit_pack (the file goes to the device as it is)
 //   Scaf::Scaf                      -> abw_segment
 //   Scaf_segment::Scaf_segment      -> abw_kmer_features
-//   Scaf::add_mapped_read           -> abw_coverage (one call per SAM file, reads in file order)
+//   Scaf::add_mapped_read           -> abw_coverage (one call per sample file, reads in file order)
 //   SAMReader / ReadMapping(line)   -> abw_parse_sam (SAM text goes to the device in 64 MB chunks cut at line boundaries), or for a BAM file
 //                                      abw_bam_feed / abw_bam_finish (the file goes to the device in 64 MB reads, inflated and parsed there)
-//   the "%.3lf" rows of abawaca.lrn   -> abw_format_lrn (text made on the device in 64 MB pieces, written with fwrite)
+//   the "%.3lf" rows of abawaca.lrn   -> abw_format_lrn through abwh::write_lrn (text made on the device in 64 MB pieces, written with fwrite)
 // The other text writers stay on the host.  Not ported (out of the hot path, SURVEY.md section 2):
 // paired-end link counting (abawaca.links is written empty: `abawaca` only checks that it exists) and the calls to
 // the external gene predictor / SCG script.
 #include "abw_host.h"
 #include <algorithm>
-#include <chrono>
 #include <ctime>
 #include <iostream>
 #include <memory>
@@ -27,18 +26,6 @@ static std::string stamp()
 	char b[32];
 	snprintf(b, sizeof(b), "[%02u:%02u:%02u]\t", t / 3600, (t % 3600) / 60, t % 60);
 	return b;
-}
-
-// ABW_TIMING=1: wall-clock milestones on stderr (CUDA start-up, text in, features, text out)
-static void milestone(const std::string& what)
-{
-	static const bool on = getenv("ABW_TIMING") != nullptr;
-	static auto t0 = std::chrono::steady_clock::now();
-	if(!on)
-		return;
-	const auto t1 = std::chrono::steady_clock::now();
-	fprintf(stderr, "[abw timing] %-28s %8.3f s\n", what.c_str(), std::chrono::duration<double>(t1 - t0).count());
-	t0 = t1;
 }
 
 static void usage(const char* prog)
@@ -68,6 +55,82 @@ static std::vector<std::string> kmer_names()
 				seen[mer] = it->second;
 		}
 	return names;
+}
+
+static const size_t CHUNK = (size_t)64 << 20;          // bytes per read of a sample file
+
+// the reads of one sample file as device records, in file order
+struct SampleReads {
+	std::shared_ptr<const abw_read> d_reads;    // its deleter releases the records in the order of the context stream, after what is queued on them
+	uint64_t n = 0;
+	bool bam = false;
+};
+
+// A BAM file goes to the device in CHUNK-byte reads (blocks, header and records may be cut anywhere: the reader carries what is unfinished); SAM
+// text in chunks cut at line boundaries, parsed there (abw_parse_sam).  buf: room for CHUNK + 1 bytes, grown for a SAM line longer than that.
+static SampleReads sample_reads(abw_ctx* ctx, const abw_names* names, const std::string& path, std::vector<char>& buf)
+{
+	FILE* fp = fopen(path.c_str(), "rb");
+	if(!fp)
+		throw std::runtime_error("Failed to open SAM file " + path);
+	std::unique_ptr<FILE, int (*)(FILE*)> file(fp, fclose);
+	SampleReads out;
+	if(is_bgzf(fp)) {
+		abw_bam* bam_raw = nullptr;
+		ABWH_CHECK(ctx, abw_bam_create(ctx, names, &bam_raw));
+		std::unique_ptr<abw_bam, void (*)(abw_bam*)> bam(bam_raw, abw_bam_destroy);
+		size_t n;
+		while((n = fread(buf.data(), 1, CHUNK, fp)) > 0)
+			if(abw_bam_feed(ctx, bam.get(), buf.data(), n) != ABW_OK)
+				throw std::runtime_error(std::string("abw_bam_feed failed on ") + path + ": " + abw_last_error(ctx));
+		file.reset();
+		const abw_read* d_reads = nullptr;
+		if(abw_bam_finish(ctx, bam.get(), &d_reads, &out.n) != ABW_OK)
+			throw std::runtime_error(std::string("abw_bam_finish failed on ") + path + ": " + abw_last_error(ctx));
+		// the records are the reader's: it goes once the device has read them
+		out.d_reads = std::shared_ptr<const abw_read>(d_reads, [ctx, b = bam.release()](const abw_read*) { abw_ctx_synchronize(ctx); abw_bam_destroy(b); });
+		out.bam = true;
+		return out;
+	}
+	// a record line has at least 11 fields, i.e. at least 10 tabs and a newline: the file size bounds the number of records
+	fseek(fp, 0, SEEK_END);
+	const uint64_t nlines = (uint64_t)ftell(fp) / 11 + 2;
+	rewind(fp);
+	abw_read* d_reads = nullptr;
+	ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<uint64_t>(nlines, 1) * sizeof(abw_read), (void**)&d_reads));
+	out.d_reads = std::shared_ptr<const abw_read>(d_reads, [ctx](const abw_read* p) { abw_device_free(ctx, (void*)p); });
+	size_t have = 0;                                       // bytes of an unfinished line carried over from the previous chunk
+	for(;;) {
+		if(have == buf.size() - 1)
+			buf.resize(2 * buf.size());                    // a line longer than the chunk
+		const size_t n = fread(buf.data() + have, 1, buf.size() - 1 - have, fp);
+		const size_t total = have + n;
+		if(total == 0)
+			break;
+		size_t cut = total;
+		if(n > 0) {                                        // not at the end of the file: cut after the last complete line
+			while(cut > 0 && buf[cut - 1] != '\n')
+				cut--;
+			if(cut == 0) {
+				have = total;
+				continue;
+			}
+		}
+		uint64_t got = 0;
+		int prc = abw_parse_sam(ctx, names, buf.data(), cut, 0, d_reads + out.n, nlines - out.n, &got);
+		if(prc == ABW_ERR_ILLEGAL_DNA) {
+			std::cerr << "Fatal error, attempted to initialize DNAString with illegal string: " << abw_last_error(ctx) << std::endl;
+			exit(-1);
+		}
+		if(prc != ABW_OK)
+			throw std::runtime_error(std::string("abw_parse_sam failed on ") + path + ": " + abw_last_error(ctx));
+		out.n += got;
+		have = total - cut;
+		memmove(buf.data(), buf.data() + cut, have);
+		if(n == 0)
+			break;
+	}
+	return out;
 }
 
 int main(int argc, const char* argv[])
@@ -190,81 +253,15 @@ int main(int argc, const char* argv[])
 			}
 			ABWH_CHECK(ctx, abw_names_create(ctx, blob.data(), noff.data(), nscaf, &names));
 		}
-		const size_t CHUNK = (size_t)64 << 20;
 		std::vector<char> buf(CHUNK + 1);
 		for(size_t j = 0; j < sam_files.size(); j++) {
 			std::cerr << stamp() << "Reading SAM file " << sam_files[j] << std::endl;
 			const bool is_this_sample = (sam_files[j] == this_sample_str);
-			FILE* fp = fopen(sam_files[j].c_str(), "rb");
-			if(!fp)
-				throw std::runtime_error("Failed to open SAM file " + sam_files[j]);
-			if(is_bgzf(fp)) {
-				// BAM: the file in 64 MB reads; blocks, header and records may be cut anywhere, the reader carries what is unfinished
-				std::unique_ptr<FILE, int (*)(FILE*)> file(fp, fclose);
-				abw_bam* bam_raw = nullptr;
-				ABWH_CHECK(ctx, abw_bam_create(ctx, names, &bam_raw));
-				std::unique_ptr<abw_bam, void (*)(abw_bam*)> bam(bam_raw, abw_bam_destroy);
-				size_t n;
-				while((n = fread(buf.data(), 1, CHUNK, fp)) > 0)
-					if(abw_bam_feed(ctx, bam.get(), buf.data(), n) != ABW_OK)
-						throw std::runtime_error(std::string("abw_bam_feed failed on ") + sam_files[j] + ": " + abw_last_error(ctx));
-				file.reset();
-				const abw_read* d_reads = nullptr;
-				uint64_t nreads = 0;
-				if(abw_bam_finish(ctx, bam.get(), &d_reads, &nreads) != ABW_OK)
-					throw std::runtime_error(std::string("abw_bam_finish failed on ") + sam_files[j] + ": " + abw_last_error(ctx));
-				ABWH_CHECK(ctx, abw_coverage(ctx, sg, d_reads, nreads, 1, max_snps, ABW_FEAT_TRUNC3, d_rows, ld, (uint32_t)(179 + j), is_this_sample? d_nbps : nullptr));
-				ABWH_CHECK(ctx, abw_ctx_synchronize(ctx));      // the records are the reader's: coverage has read them before it goes
-				bam.reset();
-				milestone("BAM " + std::to_string(j));
-				if(is_this_sample) {
-					FILE* fl = fopen(links_file.c_str(), "w");
-					if(fl) fclose(fl);
-				}
-				continue;
-			}
-			// a record line has at least 11 fields, i.e. at least 10 tabs and a newline: the file size bounds the number of records
-			fseek(fp, 0, SEEK_END);
-			const uint64_t nlines = (uint64_t)ftell(fp) / 11 + 2;
-			rewind(fp);
-			abw_read* d_reads = nullptr;
-			ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<uint64_t>(nlines, 1) * sizeof(abw_read), (void**)&d_reads));
-			uint64_t nreads = 0;
-			size_t have = 0;                                       // bytes of an unfinished line carried over from the previous chunk
-			for(;;) {
-				if(have == buf.size() - 1)
-					buf.resize(2 * buf.size());                    // a line longer than the chunk
-				const size_t n = fread(buf.data() + have, 1, buf.size() - 1 - have, fp);
-				const size_t total = have + n;
-				if(total == 0)
-					break;
-				size_t cut = total;
-				if(n > 0) {                                        // not at the end of the file: cut after the last complete line
-					while(cut > 0 && buf[cut - 1] != '\n')
-						cut--;
-					if(cut == 0) {
-						have = total;
-						continue;
-					}
-				}
-				uint64_t got = 0;
-				int prc = abw_parse_sam(ctx, names, buf.data(), cut, 0, d_reads + nreads, nlines - nreads, &got);
-				if(prc == ABW_ERR_ILLEGAL_DNA) {
-					std::cerr << "Fatal error, attempted to initialize DNAString with illegal string: " << abw_last_error(ctx) << std::endl;
-					return -1;
-				}
-				if(prc != ABW_OK)
-					throw std::runtime_error(std::string("abw_parse_sam failed on ") + sam_files[j] + ": " + abw_last_error(ctx));
-				nreads += got;
-				have = total - cut;
-				memmove(buf.data(), buf.data() + cut, have);
-				if(n == 0)
-					break;
-			}
-			fclose(fp);
-			ABWH_CHECK(ctx, abw_coverage(ctx, sg, d_reads, nreads, 1, max_snps, ABW_FEAT_TRUNC3, d_rows, ld, (uint32_t)(179 + j), is_this_sample? d_nbps : nullptr));
-			ABWH_CHECK(ctx, abw_device_free(ctx, d_reads));
-			milestone("SAM " + std::to_string(j));
+			SampleReads reads = sample_reads(ctx, names, sam_files[j], buf);
+			ABWH_CHECK(ctx, abw_coverage(ctx, sg, reads.d_reads.get(), reads.n, 1, max_snps, ABW_FEAT_TRUNC3, d_rows, ld, (uint32_t)(179 + j),
+			                             is_this_sample? d_nbps : nullptr));
+			reads.d_reads.reset();
+			milestone((reads.bam? "BAM " : "SAM ") + std::to_string(j));
 			if(is_this_sample) {
 				FILE* fl = fopen(links_file.c_str(), "w");     // scaffold-end links are not computed (SURVEY.md section 2, row 5); the file must exist
 				if(fl) fclose(fl);
@@ -288,28 +285,15 @@ int main(int argc, const char* argv[])
 		if(!flrn) { std::cerr << "Could not write to " << lrn_file << std::endl << std::endl; return -1; }
 		if(!finfo) { std::cerr << "Could not write to " << info_file << std::endl << std::endl; return -1; }
 		fprintf(fout, "%c %lu\n", '%', (unsigned long)ndps);
-		fprintf(flrn, "%c %lu\n", '%', (unsigned long)ndps);
-		fprintf(flrn, "%c %lu\n", '%', (unsigned long)(180 + sam_files.size()));     // 180 + samples: the unwritten "A" and the key column cancel
-		fprintf(flrn, "%c 9", '%');
-		for(uint64_t c = 0; c < ld; c++) fprintf(flrn, "\t1");
-		fprintf(flrn, "\n%c Key", '%');
-		const std::vector<std::string> kn = kmer_names();
-		for(size_t d = 1; d < kn.size(); d++) fprintf(flrn, "\t%s", kn[d].c_str());
-		for(auto& sf : sam_files) fprintf(flrn, "\t%s", sf.c_str());
-		fprintf(flrn, "\n");
 		{
-			// the data lines: "<g+1>" and "\t%.3lf" per value, made on the device in pieces of at most LRN_CHUNK bytes
-			const uint64_t LRN_CHUNK = (uint64_t)64 << 20;
+			// the columns: the k-mers but the first ("A", which the reference does not write) and one per sample; "%.3lf" values
+			std::vector<std::string> cols = kmer_names();
+			cols.erase(cols.begin());
+			cols.insert(cols.end(), sam_files.begin(), sam_files.end());
 			char* d_text = nullptr;
 			ABWH_CHECK(ctx, abw_device_alloc(ctx, LRN_CHUNK, (void**)&d_text));
-			std::vector<char> text(LRN_CHUNK);
-			for(uint64_t line0 = 0; line0 < ndps;) {
-				uint64_t done = 0, nbytes = 0;
-				ABWH_CHECK(ctx, abw_format_lrn(ctx, d_rows, ld, 0, (uint32_t)ld, nullptr, 0, line0, ndps, ABW_TEXT_3LF, d_text, LRN_CHUNK, &done, &nbytes));
-				ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
-				if(fwrite(text.data(), 1, nbytes, flrn) != nbytes) { std::cerr << "Could not write to " << lrn_file << std::endl << std::endl; return -1; }
-				line0 += done;
-			}
+			std::vector<char> text;
+			if(!write_lrn(ctx, flrn, cols, d_rows, ld, nullptr, ndps, ABW_TEXT_3LF, d_text, text)) { std::cerr << "Could not write to " << lrn_file << std::endl << std::endl; return -1; }
 			ABWH_CHECK(ctx, abw_device_free(ctx, d_text));
 		}
 		fclose(flrn);

@@ -2,6 +2,8 @@
 // Everything here is parsing and formatting at the on-disk boundary (SURVEY.md appendix A); all computation
 // goes through the C ABI of libabawaca_b200.so.  Written from the format descriptions, not from the reference code.
 #pragma once
+#include <algorithm>
+#include <chrono>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -149,43 +151,50 @@ inline std::vector<std::string> glob_files(const std::string& pattern)
 	return out;
 }
 
-// num_snps() of a SAM line as ReadMapping::determine_snps counts them (ReadMapping.cpp:78-185): without an MD:Z field 0; otherwise one
-// per mismatch letter, one per deleted reference base (after '^'), plus one per insertion operation of the CIGAR string.
-inline uint32_t count_snps(const std::string& cigar, const std::string& mdz /* starts with MD:Z: or empty */)
-{
-	if(mdz.empty())
-		return 0;
-	if(mdz.compare(0, 5, "MD:Z:") != 0)
-		throw std::runtime_error("Illegal SNPs description, expected MD:Z: at the beginning: " + mdz);
-	uint32_t n = 0;
-	size_t i = 5;
-	while(i < mdz.size() && isdigit((unsigned char)mdz[i])) i++;
-	while(i < mdz.size()) {
-		if(mdz[i] == '^') {
-			i++;
-			while(i < mdz.size() && !isdigit((unsigned char)mdz[i])) { n++; i++; }
-		}
-		else if(mdz[i] >= 'A' && mdz[i] <= 'Z') {
-			n++;
-			i++;
-		}
-		else
-			throw std::runtime_error("Illegal SNPs description: " + mdz);
-		if(i >= mdz.size() || !isdigit((unsigned char)mdz[i]))
-			throw std::runtime_error("Illegal SNPs description: " + mdz);
-		while(i < mdz.size() && isdigit((unsigned char)mdz[i])) i++;
-	}
-	for(char c : cigar)
-		if(c == 'I')
-			n++;
-	return n;
-}
-
 #define ABWH_CHECK(ctx, call)                                                                           \
 	do {                                                                                                \
 		int rc__ = (call);                                                                              \
 		if(rc__ != ABW_OK)                                                                              \
 			throw std::runtime_error(std::string(#call) + " failed: " + abw_last_error(ctx));           \
 	} while(0)
+
+// ABW_TIMING=1: wall-clock milestones on stderr, each with the time since the one before (where the time of a command line goes)
+inline void milestone(const std::string& what)
+{
+	static const bool on = getenv("ABW_TIMING") != nullptr;
+	static auto t0 = std::chrono::steady_clock::now();
+	if(!on)
+		return;
+	const auto t1 = std::chrono::steady_clock::now();
+	fprintf(stderr, "[abw timing] %-28s %8.3f s\n", what.c_str(), std::chrono::duration<double>(t1 - t0).count());
+	t0 = t1;
+}
+
+// the data lines of a .lrn file are made on the device (abw_format_lrn) in pieces of at most LRN_CHUNK bytes
+const uint64_t LRN_CHUNK = (uint64_t)64 << 20;
+
+// Writes a .lrn file (ClusterData.cpp:27-168 reads it back): the header "% <nlines>", "% <columns + 1>", "% 9" and "\t1" per column, "% Key" and
+// the column names; then line i = "<r+1>" and the values of row r = rows[i] (r = i when rows is NULL; rows in host memory) of the row-major device
+// matrix d_values (row stride ld), printed as fmt (ABW_TEXT_*).  d_text (LRN_CHUNK bytes of device memory) and text are scratch, kept from file to
+// file.  false when fp takes fewer bytes than it is given.
+inline bool write_lrn(abw_ctx* ctx, FILE* fp, const std::vector<std::string>& names, const double* d_values, uint64_t ld, const uint64_t* rows, uint64_t nlines,
+                      int fmt, char* d_text, std::vector<char>& text)
+{
+	fprintf(fp, "%% %lu\n%% %lu\n%% 9", (unsigned long)nlines, (unsigned long)(names.size() + 1));
+	for(size_t c = 0; c < names.size(); c++) fprintf(fp, "\t1");
+	fprintf(fp, "\n%% Key");
+	for(const std::string& n : names) fprintf(fp, "\t%s", n.c_str());
+	fprintf(fp, "\n");
+	for(uint64_t line0 = 0; line0 < nlines;) {
+		uint64_t done = 0, nbytes = 0;
+		ABWH_CHECK(ctx, abw_format_lrn(ctx, d_values, ld, 0, (uint32_t)names.size(), rows, 0, line0, nlines, fmt, d_text, LRN_CHUNK, &done, &nbytes));
+		text.resize(std::max<size_t>(text.size(), nbytes));
+		ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
+		if(fwrite(text.data(), 1, nbytes, fp) != nbytes)
+			return false;
+		line0 += done;
+	}
+	return true;
+}
 
 }  // namespace abwh

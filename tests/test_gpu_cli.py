@@ -20,8 +20,8 @@ def _norm_lrn(text):
 
 
 @pytest.mark.parametrize("name", ["tiny_clean", "tiny_noisy"])
-def test_command_lines_reproduce_reference_files(tmp_path, name):
-    from abawaca_b200 import synth
+def test_command_lines_reproduce_reference_files(tmp_path, name, oracle):
+    from abawaca_b200 import hostio, synth
     subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "abawaca_b200", "host")], check=True)
     g = load_set(name)
     wd = str(tmp_path)
@@ -55,3 +55,17 @@ def test_command_lines_reproduce_reference_files(tmp_path, name):
             assert os.path.exists(os.path.join(out, "clusters", f"{cid}.{ext}"))
     # dp2cluster.txt keeps the reference's spurious row for datapoint 0 (quirk Q10)
     assert open(os.path.join(out, "dp2cluster.txt")).readline() == "0\t0\n"
+    # the SCG tallies of every child cluster in the log: the oracle's over the scaffolds of <id>.scaf-cluster.txt, printed as std::ostream prints
+    # a uint32_t and a double
+    prob = hostio.load_search_problem(os.path.join(build, "abawaca.names"), os.path.join(build, "abawaca.lrn"), paths["fasta"], paths["gene2scg"])
+    search = oracle.Search(prob["values"], prob["dp2scaf"], prob["T"], prob["len"], prob["scgmask"])
+    scaf_id = {s: i for i, s in enumerate(prob["scaf_names"])}
+    child_lines = [(int(m.group(1)), m.group(0)) for m in re.finditer(r"Cluster (\d+), \d+ datapoints, \d+ unique SCGs \(\S+ copies\)", open(os.path.join(out, "log")).read())]
+    assert sorted(cid for cid, _ in child_lines) == list(range(2, 2 + 2 * nsplits))
+    for cid, line in child_lines:
+        with open(os.path.join(out, "clusters", f"{cid}.scaf-cluster.txt")) as f:
+            scafs = [scaf_id[l.split("\t")[0]] for l in f.read().splitlines()]
+        with open(os.path.join(out, "clusters", f"{cid}.lrn")) as f:
+            ndps = int(f.readline().split()[1])
+        u, avg = search.cluster_scg(scafs)
+        assert line == f"Cluster {cid}, {ndps} datapoints, {u} unique SCGs ({avg:g} copies)"
