@@ -36,6 +36,7 @@ constexpr int BAM_ERR_INFLATE = 1, BAM_ERR_CRC = 2, BAM_ERR_AUX = 4, BAM_ERR_MDZ
 __global__ void __launch_bounds__(INF_WARPS * 32, 8) k_bgzf_inflate(const uint8_t* __restrict__ comp, const BlockDesc* __restrict__ blk, uint32_t nblk,
                                                                  uint8_t* __restrict__ out, int* __restrict__ err, uint32_t* __restrict__ err_blk)
 {
+	abw_grid_wait();
 	__shared__ abw_inflate::Tables tables[INF_WARPS];
 	__shared__ uint32_t crc_table[256];
 	for(int i = threadIdx.x; i < 256; i += blockDim.x)
@@ -92,6 +93,7 @@ __host__ __device__ __forceinline__ bool fixed_fields_ok(uint32_t bs, const uint
 // 1 where a complete record whose fixed fields agree with its block_size starts at position p (relative to `start`)
 __global__ void k_bam_candidates(const uint8_t* __restrict__ s, uint64_t start, uint64_t len, int32_t n_ref, uint32_t* __restrict__ cand)
 {
+	abw_grid_wait();
 	const uint64_t n = len - start;
 	for(uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
 		const uint64_t p = start + i;
@@ -112,6 +114,7 @@ constexpr uint32_t NXT_LAST = 0xFFFFFFFEu;     // the next position holds no com
 __global__ void k_bam_links(const uint8_t* __restrict__ s, uint64_t start, uint64_t len, const uint32_t* __restrict__ cand, const uint64_t* __restrict__ idx,
                             uint64_t* __restrict__ pos, uint32_t* __restrict__ nxt)
 {
+	abw_grid_wait();
 	const uint64_t n = len - start;
 	for(uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
 		if(!cand[i])
@@ -127,6 +130,7 @@ __global__ void k_bam_links(const uint8_t* __restrict__ s, uint64_t start, uint6
 // marked, after it those up to 2^(k+1) - 1 (a node marked early by a concurrent thread is on the chain too, so that race only adds chain nodes).
 __global__ void k_bam_chain_round(const uint32_t* __restrict__ jin, uint32_t* __restrict__ jout, uint32_t* mark, uint32_t m)
 {
+	abw_grid_wait();
 	for(uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
 		const uint32_t j = jin[i];
 		if(j < m && mark[i])
@@ -152,6 +156,7 @@ struct RecArgs {
 // one thread per marked record: the abw_read abw_parse_sam makes of the line `samtools view` prints for it
 __global__ void __launch_bounds__(128) k_bam_records(RecArgs a)
 {
+	abw_grid_wait();
 	for(uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < a.m; i += gridDim.x * blockDim.x) {
 		if(!a.mark[i])
 			continue;
@@ -273,6 +278,7 @@ __global__ void k_bam_ref_names(const char* __restrict__ blob, const uint64_t* _
                                 const uint32_t* __restrict__ slot_index, uint32_t nslots, const char* __restrict__ name_blob, const uint64_t* __restrict__ name_off,
                                 uint32_t* __restrict__ ref_scaf)
 {
+	abw_grid_wait();
 	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
 	if(i < n)
 		ref_scaf[i] = abw_name_probe(blob + off[i], off[i + 1] - off[i], slot_hash, slot_index, nslots, name_blob, name_off);

@@ -6,6 +6,7 @@
 #include <string>
 #include <vector>
 #include <map>
+#include <utility>
 #include <cstdio>
 #include "../../include/abawaca_b200.h"
 
@@ -86,12 +87,47 @@ inline int abw_fail(abw_ctx* ctx, int code, const std::string& msg)
 			return r__;                                                                                              \
 	} while(0)
 
-// every launch goes through this so that abw_kernel_launches() is an honest count
+// Programmatic dependent launch.  Kernels on the context stream are launched with programmatic stream serialization: the next grid is launched
+// while the previous one drains, and its CTAs stop in abw_grid_wait() until the previous grid has completed and its memory is visible.  So every
+// __global__ function of the library calls abw_grid_wait() first, before any early return, any read of data an earlier kernel wrote and any global
+// store.  The chain is only transitive that way: a grid that returned without waiting would let the grid after it overlap the grid before it.
+// (tests/test_pdl_sass.py checks that every kernel of the built library holds the wait.)  In a grid launched without the attribute the wait
+// returns at once.  abw_launch_dependents() lets the dependent grid be scheduled once every CTA of this grid has called it or exited; where it
+// sits never affects correctness, since the dependent still waits for this whole grid.
+__device__ __forceinline__ void abw_grid_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void abw_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// The attribute only relaxes the dependency on the previous operation of the stream when that operation is a kernel, and only as far as that kernel
+// allows (launch_dependents or exit).  After a memset, a copy or a cudaStreamWaitEvent (a side-stream join) the launch is ordered as a plain one:
+// cudaLaunchAttributeProgrammaticStreamSerialization, CUDA Runtime API, "overlap with the previous kernel in the stream, if that kernel requests
+// the overlap".  A kernel of another library on the stream (NCCL, torch) never requests it, so a kernel of ours after it starts once it has
+// exited, and still waits for its memory in abw_grid_wait().  Therefore every launch carries the attribute, whatever precedes it.
+template <typename... Params, typename... Args>
+inline cudaError_t abw_launch_pdl(void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args)
+{
+	cudaLaunchAttribute attr[1];
+	attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+	attr[0].val.programmaticStreamSerializationAllowed = 1;
+	cudaLaunchConfig_t cfg = {};
+	cfg.gridDim = grid;
+	cfg.blockDim = block;
+	cfg.dynamicSmemBytes = smem;
+	cfg.stream = stream;
+	cfg.attrs = attr;
+	cfg.numAttrs = 1;
+	return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
+
+// every launch goes through this so that abw_kernel_launches() is an honest count.  Profiling brackets each launch with events and waits for it,
+// so those launches stay plain: the per-kernel times remain comparable with profiles taken before launches overlapped.
 #define ABW_LAUNCH(ctx, kernel, grid, block, smem, ...)                                                              \
 	do {                                                                                                             \
-		if((ctx)->profiling)                                                                                         \
+		if((ctx)->profiling) {                                                                                       \
 			cudaEventRecord((ctx)->ev_a, (ctx)->stream);                                                             \
-		kernel<<<(grid), (block), (smem), (ctx)->stream>>>(__VA_ARGS__);                                             \
+			kernel<<<(grid), (block), (smem), (ctx)->stream>>>(__VA_ARGS__);                                         \
+		}                                                                                                            \
+		else                                                                                                         \
+			abw_launch_pdl(kernel, (grid), (block), (smem), (ctx)->stream, __VA_ARGS__);                             \
 		(ctx)->launches++;                                                                                           \
 		ABW_CUDA((ctx), cudaGetLastError());                                                                         \
 		if((ctx)->profiling) {                                                                                       \

@@ -30,6 +30,7 @@ int redzone_mode()
 
 __global__ void k_redzone_check(const unsigned char* __restrict__ front, const unsigned char* __restrict__ back, size_t nback, unsigned long long* bad)
 {
+	abw_grid_wait();
 	// bad[0], bad[1]: damaged bytes before / after the block; bad[2], bad[3]: offset of the first one (atomicMin)
 	for(size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < RZ + nback; i += (size_t)gridDim.x * blockDim.x) {
 		const bool is_front = i < RZ;
@@ -125,6 +126,7 @@ cudaError_t abw_arena_alloc(abw_ctx* ctx, size_t bytes, void** out)
 // bytes from src to dst, one of them mapped pinned host memory; word-wise when both are 4-byte aligned
 __global__ void k_copy_small(unsigned char* __restrict__ dst, const unsigned char* __restrict__ src, size_t bytes)
 {
+	abw_grid_wait();
 	const size_t i0 = (size_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (size_t)gridDim.x * blockDim.x;
 	if(((reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(src)) & 3u) == 0) {
 		const size_t words = bytes >> 2;
@@ -142,7 +144,7 @@ __global__ void k_copy_small(unsigned char* __restrict__ dst, const unsigned cha
 static cudaError_t copy_small(abw_ctx* ctx, void* dst, const void* src, size_t bytes)
 {
 	const unsigned int blocks = (unsigned int)std::min<size_t>(64, (bytes / 4 + 255) / 256 + 1);
-	k_copy_small<<<blocks, 256, 0, ctx->stream>>>((unsigned char*)dst, (const unsigned char*)src, bytes);
+	abw_launch_pdl(k_copy_small, blocks, 256, 0, ctx->stream, (unsigned char*)dst, (const unsigned char*)src, bytes);      // in the middle of the chain of ABW_LAUNCH kernels
 	ctx->launches++;
 	return cudaGetLastError();
 }

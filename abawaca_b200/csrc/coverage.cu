@@ -194,6 +194,7 @@ __global__ void __launch_bounds__(COV_THREADS, 4) k_cov_sum(const ReadSrc src, u
                                                            const uint64_t* __restrict__ seg_end, unsigned long long* __restrict__ sum_ov,
                                                            uint2* __restrict__ tile_range, unsigned long long* __restrict__ scaf_nbps)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm_acc[CS_RANGE];
 	__shared__ uint32_t sm_nb[NBPS? CS_SCAFS : 1];
 	__shared__ uint32_t sm_min, sm_max, sm_smin;
@@ -337,6 +338,7 @@ __global__ void __launch_bounds__(256) k_cov_quotient(const unsigned long long* 
                                                       const uint64_t* __restrict__ seg_end, double* __restrict__ rows, uint64_t ld, uint32_t col0,
                                                       uint32_t* __restrict__ flag_bits, uint32_t nwords, uint32_t* __restrict__ nflagged)
 {
+	abw_grid_wait();
 	const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	const uint32_t sample = blockIdx.y;
 	bool f = false;
@@ -375,6 +377,7 @@ __global__ void __launch_bounds__(256) k_cov_tile_filter(const ReadSrc* __restri
                                                          uint32_t nwords, const uint32_t* __restrict__ nflagged, const uint2* __restrict__ tile_range, int all,
                                                          uint32_t* __restrict__ tile_counts, uint2* __restrict__ list, uint32_t* __restrict__ nlist)
 {
+	abw_grid_wait();
 	const uint32_t flat = blockIdx.x * blockDim.x + threadIdx.x;
 	bool go = false;
 	uint32_t sample = 0;
@@ -423,6 +426,7 @@ __global__ void __launch_bounds__(COV_THREADS) k_cov_pairs(const ReadSrc* __rest
                                                           const uint64_t* __restrict__ tile_offs, uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
                                                           unsigned long long* __restrict__ scaf_nbps, int nbps_sample)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[COV_THREADS / 32];
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 	const uint32_t n = *nlist;
@@ -537,6 +541,7 @@ __global__ void __launch_bounds__(128) k_cov_accumulate(const uint32_t* __restri
                                                         const uint64_t* __restrict__ seg_start, const uint64_t* __restrict__ seg_end, double* __restrict__ rows,
                                                         uint64_t ld, uint32_t col0)
 {
+	abw_grid_wait();
 	const uint64_t i0 = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(i0 >= npairs)
 		return;
@@ -577,6 +582,7 @@ __global__ void __launch_bounds__(128) k_cov_accumulate(const uint32_t* __restri
 
 __global__ void k_cov_zero_columns(double* __restrict__ rows, uint64_t nseg, uint64_t ld, uint32_t col0, uint32_t ncols)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(i < nseg * ncols)
 		rows[(i / ncols) * ld + col0 + (i % ncols)] = 0.0;

@@ -89,6 +89,7 @@ __global__ void __launch_bounds__(256) k_pack(const unsigned char* __restrict__ 
                                               uint32_t* __restrict__ nmask, unsigned long long* __restrict__ countN, unsigned long long* __restrict__ countGC,
                                               int* __restrict__ err)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t s = warp0; s < nscaf; s += nwarps) {
@@ -151,6 +152,7 @@ __device__ __forceinline__ void window_plan(uint64_t len, uint64_t nN, uint64_t 
 
 __global__ void k_seg_count(const uint64_t* __restrict__ len, const unsigned long long* __restrict__ countN, uint32_t nscaf, uint64_t window, uint64_t* __restrict__ counts)
 {
+	abw_grid_wait();
 	uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
 	if(s < nscaf) {
 		uint64_t nbps, count;
@@ -165,6 +167,7 @@ __global__ void __launch_bounds__(256) k_seg_fill(const uint64_t* __restrict__ l
                                                   uint32_t* __restrict__ seg_scaf, uint64_t* __restrict__ seg_start, uint64_t* __restrict__ seg_end,
                                                   uint64_t* __restrict__ seg_nonN, uint64_t* __restrict__ seg_gbase, uint4* __restrict__ scaf_info)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t s = warp0; s < nscaf; s += nwarps) {
@@ -267,6 +270,7 @@ __global__ void __launch_bounds__(KM_WARPS * 32) k_kmer(const uint32_t* __restri
                                                         const uint64_t* __restrict__ seg_start, const uint64_t* __restrict__ seg_end, uint64_t nseg, int skip_A,
                                                         double* __restrict__ rows, uint64_t ld, uint32_t col0)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm_dim_tab[ABW_NKMER_DIMS];
 	__shared__ KmWarpSmem sm_warp[KM_WARPS];
 	KmWarpSmem* sm = sm_warp + (threadIdx.x >> 5);
@@ -420,6 +424,7 @@ template <typename OutT>
 __global__ void __launch_bounds__(256) k_rows_milli(const double* __restrict__ rows, uint64_t nrows, uint64_t ld, uint32_t col0, uint32_t ncols, OutT* __restrict__ out,
                                                     int* __restrict__ inexact)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	bool bad = false;
 	if(i < nrows * ncols) {

@@ -28,6 +28,7 @@ constexpr int LN_TILE = LN_THREADS * LN_BYTES_PER_THREAD;      // 4 KB of text p
 
 __global__ void __launch_bounds__(LN_THREADS) k_line_count(const char* __restrict__ text, uint64_t nbytes, uint32_t* __restrict__ tile_counts)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[LN_THREADS / 32];
 	const uint64_t i0 = (uint64_t)blockIdx.x * LN_TILE + (uint64_t)threadIdx.x * LN_BYTES_PER_THREAD;
 	uint32_t c = 0;
@@ -56,6 +57,7 @@ __global__ void __launch_bounds__(LN_THREADS) k_line_count(const char* __restric
 // line l (l >= 1) starts after the l-th newline; line 0 starts at 0.  A final newline opens an empty last line, which is not a record.
 __global__ void __launch_bounds__(LN_THREADS) k_line_starts(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ tile_offs, uint64_t* __restrict__ line_start)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[LN_THREADS / 32];
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 	const uint64_t i0 = (uint64_t)blockIdx.x * LN_TILE + (uint64_t)threadIdx.x * LN_BYTES_PER_THREAD;
@@ -141,6 +143,7 @@ __device__ __forceinline__ bool dev_isspace(char c) { return c == ' ' || (c >= '
 __global__ void k_line_select(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines, char skip, bool trim_space,
                               uint32_t* __restrict__ keep)
 {
+	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines)
 		return;
@@ -189,6 +192,7 @@ __global__ void __launch_bounds__(128) k_sam_parse(const char* __restrict__ text
                                                    const uint32_t* __restrict__ slot_index, uint32_t nslots, const char* __restrict__ name_blob,
                                                    const uint64_t* __restrict__ name_off, abw_read* __restrict__ out, uint64_t cap, int* __restrict__ err)
 {
+	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines || !is_record[l])
 		return;
@@ -277,6 +281,7 @@ constexpr int FA_ERR_NO_HEADER = 1, FA_ERR_EMPTY_ID = 2;
 __global__ void k_fa_classify(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, uint64_t nlines, uint64_t* __restrict__ line_a,
                               uint32_t* __restrict__ line_len, uint32_t* __restrict__ is_header, uint32_t* __restrict__ id_len, int* __restrict__ err)
 {
+	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines)
 		return;
@@ -310,6 +315,7 @@ __global__ void k_fa_records(const uint64_t* __restrict__ line_a, const uint32_t
                              const uint64_t* __restrict__ hdr_before, const uint64_t* __restrict__ chars_before, uint64_t nlines, uint64_t nrec,
                              uint64_t* __restrict__ rec_id_off, uint32_t* __restrict__ rec_id_len, uint64_t* __restrict__ rec_chars0, int* __restrict__ err)
 {
+	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines)
 		return;
@@ -328,6 +334,7 @@ __global__ void __launch_bounds__(256) k_fa_copy(const char* __restrict__ text, 
                                                  const uint64_t* __restrict__ hdr_before, const uint64_t* __restrict__ chars_before, uint64_t nlines,
                                                  const uint64_t* __restrict__ rec_chars0, const uint64_t* __restrict__ rec_dst, char* __restrict__ out)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t l = warp0; l < nlines; l += nwarps) {
@@ -434,6 +441,7 @@ __global__ void __launch_bounds__(128) k_lrn_parse(const char* __restrict__ text
                                                    uint64_t* __restrict__ keys, double* __restrict__ values, LrnFallback* __restrict__ fb, uint32_t fb_cap,
                                                    uint32_t* __restrict__ fb_count, int* __restrict__ err)
 {
+	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(l >= nlines || !is_row[l])
 		return;
@@ -476,6 +484,7 @@ __global__ void __launch_bounds__(128) k_lrn_parse(const char* __restrict__ text
 __global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ src, uint64_t ld_src, double* __restrict__ dst, uint64_t ld_dst, uint32_t ncols,
                                                      const uint64_t* __restrict__ rows, uint64_t nrows)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < nrows; i += nwarps) {

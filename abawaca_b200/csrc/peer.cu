@@ -30,6 +30,7 @@ struct PeerDst {
 // windows a scaffold keeps: ScafDpData drops scaffolds with a single datapoint (ScafDpData.cpp:92-93)
 __global__ void k_kept_windows(const uint64_t* __restrict__ seg_first, uint32_t nscaf, uint32_t* __restrict__ kept)
 {
+	abw_grid_wait();
 	const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
 	if(s < nscaf) {
 		const uint64_t c = seg_first[s + 1] - seg_first[s];
@@ -46,6 +47,7 @@ __global__ void __launch_bounds__(PX_THREADS) k_scatter_columns(const double* __
                                                                 uint64_t row0, const PeerDst dst, int* __restrict__ inexact, const uint32_t* __restrict__ seg_scaf,
                                                                 const uint64_t* __restrict__ seg_first, const uint64_t* __restrict__ kept_before)
 {
+	abw_grid_wait();
 	extern __shared__ uint32_t tile[];         // [PX_ROWS][ncols]
 	__shared__ unsigned long long dst_row[PX_ROWS];
 	__shared__ double milli[1001];             // k / 1000.0 for the k-mer frequencies (k <= 1000): the exactness test without a division per value

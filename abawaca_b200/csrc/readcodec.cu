@@ -61,6 +61,7 @@ __device__ __forceinline__ Seg block_seg_scan(Seg x, Seg carry, Seg* total, Seg*
 
 __global__ void __launch_bounds__(256) k_sorted_run_counts(const abw_read_run* __restrict__ runs, uint64_t nruns, uint32_t* __restrict__ counts)
 {
+	abw_grid_wait();
 	const uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(r < nruns)
 		counts[r] = __ldg(&runs[r].count);
@@ -81,6 +82,7 @@ __device__ __forceinline__ uint32_t run_search(const uint64_t* __restrict__ firs
 __global__ void __launch_bounds__(256) k_sorted_tile_runs(const uint64_t* __restrict__ first, uint32_t nruns, const uint64_t* __restrict__ d_total, uint64_t n,
                                                           uint32_t ntiles, uint32_t* __restrict__ tile_run)
 {
+	abw_grid_wait();
 	const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
 	if(t >= ntiles)
 		return;
@@ -136,6 +138,7 @@ __global__ void __launch_bounds__(RC_THREADS) k_sorted_summary(const uint16_t* _
                                                                const uint64_t* __restrict__ d_total, const uint32_t* __restrict__ tile_run, uint32_t ntiles,
                                                                uint4* __restrict__ summary)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm_esc, sm_code, sm_before, sm_add;
 	if(threadIdx.x == 0) {
 		sm_esc = 0; sm_code = 0; sm_before = 0; sm_add = 0;
@@ -188,6 +191,7 @@ __device__ __forceinline__ uint32_t exc_at(const uint32_t* __restrict__ exc, uin
 __global__ void __launch_bounds__(RC_CARRY_THREADS) k_sorted_carry(const uint4* __restrict__ summary, uint32_t ntiles, const uint32_t* __restrict__ exc, uint64_t nexc,
                                                                    uint2* __restrict__ carry)
 {
+	abw_grid_wait();
 	__shared__ Seg sm[RC_CARRY_THREADS / 32];
 	Seg esc_carry{0, 0}, pos_carry{0, 0};
 	for(uint32_t c0 = 0; c0 < ntiles; c0 += RC_CARRY_THREADS * RC_CARRY_TILES) {
@@ -230,6 +234,7 @@ __global__ void __launch_bounds__(RC_THREADS, 4) k_sorted_write(const uint16_t* 
                                                              uint64_t nexc, const uint32_t* __restrict__ tile_run, uint32_t ntiles, const uint2* __restrict__ carry,
                                                              abw_read8* __restrict__ out)
 {
+	abw_grid_wait();
 	__shared__ Seg sm[RC_THREADS / 32];
 	Items it;
 	load_items(delta, n, first, nruns, nruns? *d_total : 0, tile_run, ntiles, it);

@@ -57,11 +57,13 @@ __global__ void __launch_bounds__(SCAN_THREADS) k_scan_onepass(const Tin* __rest
                                                               uint32_t* __restrict__ status, unsigned long long* __restrict__ aggs, unsigned long long* __restrict__ prefixes,
                                                               uint32_t* __restrict__ failed)
 {
+	abw_grid_wait();
 	__shared__ uint64_t sm[33];
 	__shared__ unsigned long long sm_tile, sm_carry;
 	if(threadIdx.x == 0)
 		sm_tile = atomicAdd(ticket, 1ull) - ticket_base;
 	__syncthreads();
+	abw_launch_dependents();                               // tile drawn: once every CTA has one, the next kernel may take the slots they free
 	const uint64_t tile = sm_tile;
 	const uint64_t base = tile * SCAN_TILE + (uint64_t)threadIdx.x * SCAN_ITEMS;
 	uint64_t v[SCAN_ITEMS];
@@ -162,6 +164,7 @@ constexpr int RS_TILE = RS_THREADS * RS_ITEMS;     // 4096
 template <typename K>
 __global__ void __launch_bounds__(RS_THREADS) k_rs_or_and(const K* __restrict__ keys, uint64_t n, uint64_t stride, unsigned long long* __restrict__ or_and)
 {
+	abw_grid_wait();
 	const K* a = keys + (uint64_t)blockIdx.y * stride;
 	unsigned long long o = 0, an = ~0ull;
 	for(uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) {
@@ -184,6 +187,7 @@ __global__ void __launch_bounds__(RS_THREADS) k_rs_or_and(const K* __restrict__ 
 template <typename K, int BITS>
 __global__ void __launch_bounds__(RS_THREADS) k_rs_hist(const K* __restrict__ keys, uint64_t n, uint64_t stride, int shift, uint32_t* __restrict__ hist)
 {
+	abw_grid_wait();
 	constexpr int NB = 1 << BITS;
 	__shared__ uint32_t sh[NB];
 	const K* a = keys + (uint64_t)blockIdx.y * stride;
@@ -206,6 +210,7 @@ template <typename K, int BITS>
 __global__ void __launch_bounds__(RS_THREADS) k_rs_scatter(const K* __restrict__ keys_in, const uint32_t* __restrict__ vals_in, K* __restrict__ keys_out,
                                                           uint32_t* __restrict__ vals_out, uint64_t n, uint64_t stride, int shift, const uint64_t* __restrict__ offsets)
 {
+	abw_grid_wait();
 	constexpr int NB = 1 << BITS;
 	__shared__ uint32_t cnt[RS_WARPS][NB + 1];
 	__shared__ uint64_t digit_base[NB];

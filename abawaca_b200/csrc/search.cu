@@ -277,6 +277,7 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep_split_scafs(const uint3
                                                                     SweepParams prm, uint32_t epoch, uint32_t* __restrict__ status, AggSlot* __restrict__ aggs,
                                                                     AggSlot* __restrict__ prefixes, CandRec* __restrict__ out)
 {
+	abw_grid_wait();
 	__shared__ Agg sm_agg[SW_THREADS / 32 + 1];
 	__shared__ CandRec sm_best[SW_THREADS / 32];
 	__shared__ unsigned long long sm_w;
@@ -290,8 +291,10 @@ __global__ void __launch_bounds__(SW_THREADS, 3) k_sweep_split_scafs(const uint3
 			sm_w = atomicAdd(&ctl->tickets[1], 1ull);
 		__syncthreads();
 		const uint64_t w = sm_w;
-		if(w >= items)
+		if(w >= items) {
+			abw_launch_dependents();        // no ticket left for this CTA: the next level kernel may take its slot
 			break;
+		}
 		const uint32_t d = (uint32_t)(w / TT);
 		const uint2 te = __ldg(tile_tab + (uint32_t)(w - (uint64_t)d * TT));
 		const uint32_t c = te.x, tile = te.y;
@@ -396,6 +399,7 @@ __global__ void __launch_bounds__(SW_THREADS, FLIP_CTAS) k_flip_prefix(const uin
                                                               AggSlot* __restrict__ prefixes, uint2* __restrict__ F8, uint32_t* __restrict__ FC, uint32_t* __restrict__ scg_k,
                                                               uint64_t Kstride, uint2* __restrict__ klohi, uint32_t Cstride, unsigned long long scg_min_size)
 {
+	abw_grid_wait();
 	__shared__ uint4 sm_r[FP_TILE];                        // {T (0: no entry), n | SCG flag << 31, length}
 	__shared__ Agg sm_agg[SW_THREADS / 32];
 	__shared__ unsigned long long sm_w;
@@ -408,8 +412,10 @@ __global__ void __launch_bounds__(SW_THREADS, FLIP_CTAS) k_flip_prefix(const uin
 			sm_w = atomicAdd(&ctl->tickets[0], 1ull);
 		__syncthreads();
 		const uint64_t w = sm_w;
-		if(w >= items)
+		if(w >= items) {
+			abw_launch_dependents();        // no ticket left for this CTA: the next level kernel may take its slot
 			break;
+		}
 		const uint32_t d = (uint32_t)(w / FTT);
 		const uint2 te = __ldg(ftile_tab + (uint32_t)(w - (uint64_t)d * FTT));
 		const uint32_t tile = te.y;
@@ -509,6 +515,7 @@ __global__ void __launch_bounds__(SW_THREADS, SWEEP_CTAS) k_sweep_ss(const uint3
                                                            const uint2* __restrict__ klohi, uint32_t Cstride, uint64_t Sf, const uint8_t* __restrict__ pass_tab,
                                                            SweepParams prm, uint32_t epoch, unsigned long long* __restrict__ lookback, CandRec* __restrict__ out)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm_warp[SW_THREADS / 32];
 	__shared__ CandRec sm_best[SW_THREADS / 32];
 	__shared__ unsigned long long sm_w;
@@ -521,8 +528,10 @@ __global__ void __launch_bounds__(SW_THREADS, SWEEP_CTAS) k_sweep_ss(const uint3
 			sm_w = atomicAdd(&ctl->tickets[1], 1ull);
 		__syncthreads();
 		const uint64_t w = sm_w;
-		if(w >= items)
+		if(w >= items) {
+			abw_launch_dependents();        // no ticket left for this CTA: the next level kernel may take its slot
 			break;
+		}
 		const uint32_t d = (uint32_t)(w / TT);
 		const uint2 te = __ldg(tile_tab + (uint32_t)(w - (uint64_t)d * TT));
 		const uint32_t tile = te.y;
@@ -665,6 +674,7 @@ template <int STRATEGY>
 __global__ void __launch_bounds__(RB_THREADS) k_reduce_best(const CandRec* __restrict__ per_item, uint32_t D, const LevelCtl* __restrict__ ctl,
                                                     const LevelCluster* __restrict__ clusters, uint32_t dim_offset, uint32_t dim_stride, CandRec* __restrict__ out)
 {
+	abw_grid_wait();
 	__shared__ CandRec sm[RB_THREADS];
 	const uint32_t C = ctl->C, TT = ctl->TT;
 	for(uint32_t c = blockIdx.x; c < C; c += gridDim.x) {
@@ -706,6 +716,7 @@ __global__ void __launch_bounds__(PT_WARPS * 32) k_pass_table(const uint32_t* __
                              const LevelCtl* __restrict__ ctl, const uint64_t* __restrict__ scgmask, uint32_t W, double overlap_thr, uint64_t* __restrict__ suffix_tmp,
                              uint8_t* __restrict__ tab, uint32_t D, uint2* __restrict__ klohi, uint32_t Cstride, unsigned long long scg_min_size)
 {
+	abw_grid_wait();
 	__shared__ unsigned long long chunk_or[PT_WARPS][SCG_WMAX];
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 	const uint32_t C = ctl->C;
@@ -925,6 +936,7 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_jobs(const LevelBufs B, in
                                                          uint32_t dim_offset, uint32_t dim_stride, uint32_t Dlocal, const uint32_t* __restrict__ E, uint64_t N,
                                                          ChildStats* __restrict__ stats, unsigned long long* __restrict__ value_key, uint64_t* __restrict__ child_never, uint32_t W)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[33];
 	__shared__ unsigned long long sm_el;
 	LevelCtl* const ctl = B.ctl;
@@ -1033,6 +1045,7 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_jobs(const LevelBufs B, in
 __global__ void __launch_bounds__(256) k_count_low(const uint32_t* __restrict__ E, uint64_t N, const LevelBufs B, int cur, uint32_t dim_offset, uint32_t dim_stride,
                                                   uint32_t* __restrict__ low)
 {
+	abw_grid_wait();
 	const LevelCluster* __restrict__ cls = B.cl[cur];
 	const uint32_t items = B.ctl->CL_items;
 	for(uint32_t it = blockIdx.x; it < items; it += gridDim.x) {
@@ -1074,6 +1087,7 @@ __global__ void __launch_bounds__(SS_CHUNK) k_scaf_sides(const uint32_t* __restr
                              const uint64_t* __restrict__ scgmask, uint32_t W, int strategy, double fraction_in, uint8_t* __restrict__ side, uint8_t* __restrict__ new_assigned,
                              ChildStats* __restrict__ stats, uint64_t* __restrict__ child_never, unsigned long long* __restrict__ value_key)
 {
+	abw_grid_wait();
 	const LevelCluster* __restrict__ cls = B.cl[cur];
 	const uint32_t items = B.ctl->SS_items;
 	const int lane = threadIdx.x & 31;
@@ -1171,6 +1185,7 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_decide(const LevelBufs B, 
                                                            int build_next, const ChildStats* __restrict__ stats, const unsigned long long* __restrict__ value_key,
                                                            const uint64_t* __restrict__ child_never)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[33];
 	__shared__ unsigned long long sm_el;
 	LevelCtl* const ctl = B.ctl;
@@ -1341,6 +1356,7 @@ __global__ void __launch_bounds__(LV_THREADS) k_level_decide(const LevelBufs B, 
 // pending clusters become bins without being evaluated (abw_search_set_max_levels): the children of the last level that was run
 __global__ void __launch_bounds__(LV_THREADS) k_pending_jobs(const LevelBufs B, int cur, uint32_t W)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[33];
 	LevelCtl* const ctl = B.ctl;
 	const LevelCluster* __restrict__ cls = B.cl[cur];
@@ -1371,6 +1387,7 @@ __global__ void __launch_bounds__(128) k_finalize_terminal(const uint32_t* __res
                                     const uint8_t* __restrict__ assigned, const uint64_t* __restrict__ scgmask, uint32_t W, uint32_t* __restrict__ scaf_member,
                                     uint32_t* __restrict__ scaf_final, const double* __restrict__ x_gc, const double* __restrict__ x_cvg)
 {
+	abw_grid_wait();
 	__shared__ int sm_last;
 	LevelCtl* const ctl = B.ctl;
 	const uint32_t items = ctl->TM_items, Tn = ctl->Tn;
@@ -1491,6 +1508,7 @@ __global__ void __launch_bounds__(SW_THREADS, PART_CTAS) k_partition2(const Part
                                                              const uint2* __restrict__ tab_all, const uint8_t* __restrict__ side, const uint8_t* __restrict__ new_assigned,
                                                              uint8_t* __restrict__ assigned, uint32_t epoch, unsigned long long* __restrict__ lookback)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm_cnt[SW_THREADS / 32];
 	__shared__ uint32_t sm_ht[SW_THREADS / 32];
 	__shared__ unsigned long long sm_w;
@@ -1501,8 +1519,10 @@ __global__ void __launch_bounds__(SW_THREADS, PART_CTAS) k_partition2(const Part
 			sm_w = atomicAdd(&ctl->tickets[2], 1ull);
 		__syncthreads();
 		const uint64_t w = sm_w;
-		if(w >= end3)
+		if(w >= end3) {
+			abw_launch_dependents();        // no ticket left for this CTA: the next level kernel may take its slot
 			break;
+		}
 		const int pl = (w >= end0) + (w >= end1) + (w >= end2);
 		const uint64_t wl = w - ((pl == 0)? 0ull : (pl == 1)? end0 : (pl == 2)? end1 : end2);
 		const uint32_t TT = ctl->part_TT[pl];
@@ -1673,6 +1693,7 @@ __global__ void __launch_bounds__(SW_THREADS, PART_CTAS) k_partition2(const Part
 __global__ void k_scg_tally(const uint32_t* __restrict__ list, uint32_t n, const uint64_t* __restrict__ scgmask, uint32_t W, TermStats* __restrict__ stats,
                             uint64_t* __restrict__ union_mask)
 {
+	abw_grid_wait();
 	for(uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
 		const uint32_t s = list[i];
 		uint32_t copies = 0;
@@ -1690,6 +1711,7 @@ __global__ void k_scg_tally(const uint32_t* __restrict__ list, uint32_t n, const
 
 __global__ void k_dp_bins(const uint32_t* __restrict__ dp2scaf, const uint32_t* __restrict__ scaf_member, uint64_t N, uint32_t* __restrict__ dp2cluster)
 {
+	abw_grid_wait();
 	uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(i < N)
 		dp2cluster[i] = scaf_member[dp2scaf[i]];
@@ -1708,6 +1730,7 @@ template <bool MILLI, typename KeyT>
 __global__ void __launch_bounds__(256) k_keys(const ValSrc v, uint64_t N, uint32_t d0, uint32_t nd, KeyT* __restrict__ keys, uint32_t* __restrict__ vals,
                                               int* __restrict__ flag)
 {
+	abw_grid_wait();
 	__shared__ KeyT tile[32][33];
 	const uint64_t r0 = (uint64_t)blockIdx.x * 32;
 	const uint32_t c0 = blockIdx.y * 32;
@@ -1766,6 +1789,7 @@ __global__ void __launch_bounds__(256) k_keys(const ValSrc v, uint64_t N, uint32
 
 __global__ void k_fill_or_and(uint32_t* __restrict__ or_and, uint32_t n)
 {
+	abw_grid_wait();
 	const uint32_t d = blockIdx.x * blockDim.x + threadIdx.x;
 	if(d < n) {
 		or_and[2 * d] = 0u;
@@ -1780,6 +1804,7 @@ __global__ void __launch_bounds__(256) k_rank_class(const KeyT* __restrict__ key
                                                     const uint64_t* __restrict__ dp_first, const ScafRow* __restrict__ rows, const uint8_t* __restrict__ has_scg, int strategy,
                                                     double fraction_in, uint8_t* __restrict__ cls_out, uint32_t* __restrict__ or_and)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	const uint32_t d = blockIdx.y;
 	if(or_and != nullptr) {
@@ -1835,6 +1860,7 @@ template <typename KeyT>
 __global__ void k_pack_elements(const KeyT* __restrict__ keys, const uint32_t* __restrict__ vals, uint64_t N, uint32_t nd, const uint32_t* __restrict__ dp2scaf,
                                 const uint8_t* __restrict__ cls, uint32_t* __restrict__ E, const uint32_t* __restrict__ scg_index, uint32_t* __restrict__ flip_pos, uint64_t K)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	const uint32_t d = blockIdx.y;
 	if(i >= N || d >= nd)
@@ -1862,6 +1888,7 @@ struct RootStats {
 // one thread per datapoint: dp2scaf must be non-decreasing, below S and without gaps; first[s] = first datapoint of scaffold s
 __global__ void k_tab_runs(const uint32_t* __restrict__ dp2scaf, uint64_t N, uint32_t S, uint64_t* __restrict__ first, RootStats* __restrict__ rs)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	if(i >= N)
 		return;
@@ -1896,6 +1923,7 @@ __global__ void k_tab_runs(const uint32_t* __restrict__ dp2scaf, uint64_t N, uin
 // dp2scaf of a matrix that holds every datapoint of every scaffold (n == T, the reference's own flow): datapoints [first[s], first[s+1]) belong to s
 __global__ void k_tab_fill_dp2scaf(const uint64_t* __restrict__ first, uint32_t S, uint64_t N, uint32_t* __restrict__ dp2scaf)
 {
+	abw_grid_wait();
 	const uint32_t sidx = blockIdx.x * blockDim.x + threadIdx.x;
 	if(sidx >= S)
 		return;
@@ -1909,6 +1937,7 @@ __global__ void __launch_bounds__(256) k_tab_scaffolds(const uint64_t* __restric
                                                        const uint64_t* __restrict__ scgmask, uint32_t S, uint32_t W, double fraction_in, ScafRow* __restrict__ rows,
                                                        uint4* __restrict__ frow, uint8_t* __restrict__ has_scg, uint32_t* __restrict__ scg_flag, uint32_t* __restrict__ scaf_iota, RootStats* __restrict__ rs)
 {
+	abw_grid_wait();
 	const uint32_t sidx = blockIdx.x * blockDim.x + threadIdx.x;
 	const bool active = sidx < S;
 	uint32_t t = 0, n = 0, err = 0;
@@ -1961,6 +1990,7 @@ __global__ void __launch_bounds__(256) k_tab_scaffolds(const uint64_t* __restric
 // SCG-carrying scaffolds that can flip, in scaffold order, and the index of each in that list
 __global__ void k_tab_scg(const uint32_t* __restrict__ scg_flag, const uint64_t* __restrict__ scg_before, uint32_t S, uint32_t* __restrict__ scg_index, uint32_t* __restrict__ scg_scafs)
 {
+	abw_grid_wait();
 	const uint32_t sidx = blockIdx.x * blockDim.x + threadIdx.x;
 	if(sidx >= S)
 		return;
@@ -1974,6 +2004,7 @@ __global__ void k_tab_scg(const uint32_t* __restrict__ scg_flag, const uint64_t*
 // pass 1: class-1 elements per tile of SW_TILE; pass 2: a tile finds its offset by summing the counts of the tiles before it.
 __global__ void __launch_bounds__(256) k_flip_count(const uint32_t* __restrict__ E, uint64_t N, uint32_t tiles, uint32_t* __restrict__ counts)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[8];
 	const uint32_t d = blockIdx.y, t = blockIdx.x;
 	const uint32_t* __restrict__ seg = E + (uint64_t)d * N;
@@ -1992,6 +2023,7 @@ __global__ void __launch_bounds__(256) k_flip_count(const uint32_t* __restrict__
 __global__ void __launch_bounds__(256) k_flip_write(const uint32_t* __restrict__ E, uint64_t N, uint32_t tiles, const uint32_t* __restrict__ counts, uint32_t* __restrict__ list,
                                                    uint64_t Sf)
 {
+	abw_grid_wait();
 	__shared__ uint32_t sm[9];
 	const uint32_t d = blockIdx.y, t = blockIdx.x;
 	const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -2033,6 +2065,7 @@ __global__ void __launch_bounds__(256) k_flip_write(const uint32_t* __restrict__
 __global__ void k_iota_pairs(unsigned long long* __restrict__ keys, const uint32_t* __restrict__ flip_pos, uint32_t* __restrict__ vals, const uint32_t* __restrict__ scg_scafs,
                              uint64_t K, uint32_t nd)
 {
+	abw_grid_wait();
 	const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
 	const uint32_t d = blockIdx.y;
 	if(i < K && d < nd) {
@@ -2357,6 +2390,7 @@ int search_build(abw_ctx* ctx, abw_search* s, const double* values, int values_o
 // one thread per scaffold of the assembly: windows per scaffold, and whether ScafDpData keeps it (at least two windows, ScafDpData.cpp:92-93)
 __global__ void k_feat_counts(const uint64_t* __restrict__ seg_first, uint32_t nscaf, uint32_t* __restrict__ keep, uint32_t* __restrict__ cnt)
 {
+	abw_grid_wait();
 	const uint32_t sidx = blockIdx.x * blockDim.x + threadIdx.x;
 	if(sidx >= nscaf)
 		return;
@@ -2370,6 +2404,7 @@ __global__ void k_feat_gather(const uint64_t* __restrict__ seg_first, uint32_t n
                               uint32_t W, uint32_t* __restrict__ T_out, uint64_t* __restrict__ len_out, uint64_t* __restrict__ mask_out, uint64_t* __restrict__ rowidx,
                               uint32_t* __restrict__ kept_out)
 {
+	abw_grid_wait();
 	const uint32_t sidx = blockIdx.x * blockDim.x + threadIdx.x;
 	if(sidx >= nscaf || !keep[sidx])
 		return;

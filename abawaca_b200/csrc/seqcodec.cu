@@ -52,6 +52,7 @@ __global__ void __launch_bounds__(256) k_2bit_decode(const uint8_t* __restrict__
                                                      uint32_t* __restrict__ packed, uint32_t* __restrict__ valid, uint32_t* __restrict__ nmask,
                                                      unsigned long long* __restrict__ countN, unsigned long long* __restrict__ countGC)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t s = warp0; s < nscaf; s += nwarps) {
@@ -112,6 +113,7 @@ __global__ void __launch_bounds__(256) k_2bit_runs(const abw_base_run* __restric
                                                    const uint64_t* __restrict__ base, uint32_t nscaf, uint32_t* __restrict__ packed,
                                                    uint32_t* __restrict__ valid, uint32_t* __restrict__ nmask, uint32_t* __restrict__ touched)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t r = warp0; r < nruns; r += nwarps) {
@@ -144,6 +146,7 @@ __global__ void __launch_bounds__(256) k_2bit_recount(const uint32_t* __restrict
                                                       const uint32_t* __restrict__ packed, const uint32_t* __restrict__ nmask,
                                                       unsigned long long* __restrict__ countN, unsigned long long* __restrict__ countGC)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t s = warp0; s < nscaf; s += nwarps) {

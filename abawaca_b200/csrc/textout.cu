@@ -88,6 +88,7 @@ __global__ void __launch_bounds__(TX_WARPS * 32) k_lrn_text_len(const double* __
                                                                uint32_t* __restrict__ line_len, TxFallback* __restrict__ fb, uint32_t fb_cap,
                                                                uint32_t* __restrict__ fb_count)
 {
+	abw_grid_wait();
 	const int lane = threadIdx.x & 31;
 	const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
 	for(uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < nlines; i += nwarps) {
@@ -118,6 +119,7 @@ __global__ void __launch_bounds__(TX_WARPS * 32) k_lrn_text_len(const double* __
 
 __global__ void k_lrn_text_fb_len(const uint64_t* __restrict__ fb_key, const uint32_t* __restrict__ fb_len, uint32_t nfb, uint32_t ncols, uint32_t* __restrict__ line_len)
 {
+	abw_grid_wait();
 	const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
 	if(k < nfb)
 		atomicAdd(&line_len[fb_key[k] / ncols], fb_len[k]);
@@ -126,6 +128,7 @@ __global__ void k_lrn_text_fb_len(const uint64_t* __restrict__ fb_key, const uin
 // cut[0] = whole lines that fit cap bytes, cut[1] = their bytes, cut[2] = bytes of line 0
 __global__ void k_lrn_text_cut(const uint64_t* __restrict__ offs, const uint64_t* __restrict__ total, uint64_t nlines, uint64_t cap, uint64_t* __restrict__ cut)
 {
+	abw_grid_wait();
 	const uint64_t tot = *total;
 	auto end_of = [&](uint64_t k) { return k + 1 < nlines? offs[k + 1] : tot; };      // end of line k
 	uint64_t lo = 0, hi = nlines;                                                       // lines [0, lo) fit; lines [0, hi + 1) do not
@@ -189,6 +192,7 @@ __global__ void __launch_bounds__(TX_WARPS * 32, 4) k_lrn_text_write(const doubl
                                                                  const uint64_t* __restrict__ fb_off, const uint32_t* __restrict__ fb_len, uint32_t nfb,
                                                                  const char* __restrict__ fb_text, char* __restrict__ out)
 {
+	abw_grid_wait();
 	__shared__ __align__(16) unsigned char smem[TX_WARPS][TX_BUF];
 	const int lane = threadIdx.x & 31;
 	unsigned char* buf = smem[threadIdx.x >> 5];
