@@ -86,6 +86,7 @@ EXPORTS = [
     "abw_names_create", "abw_names_destroy", "abw_parse_sam", "abw_fasta_scan", "abw_fasta_destroy", "abw_fasta_count", "abw_fasta_get", "abw_fasta_pack", "abw_nccl_unique_id", "abw_nccl_collectives_create", "abw_nccl_collectives_destroy", "abw_peer_buffer_create", "abw_peer_buffer_destroy", "abw_peer_group_create", "abw_peer_group_destroy",
     "abw_scatter_columns_milli", "abw_parse_lrn", "abw_gather_rows", "abw_format_lrn", "abw_search_set_scaffold_stats",
     "abw_pack_2bit", "abw_twobit_scan", "abw_twobit_destroy", "abw_twobit_count", "abw_twobit_get", "abw_twobit_decode", "abw_twobit_pack",
+    "abw_fasta_format", "abw_twobit_format", "abw_fasta_base_counts", "abw_twobit_base_counts",
     "abw_bam_create", "abw_bam_feed", "abw_bam_finish", "abw_bam_destroy",
 ]
 
@@ -164,6 +165,11 @@ def load():
     L.abw_twobit_get.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.abw_twobit_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     L.abw_twobit_pack.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]
+    L.abw_fasta_format.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+    L.abw_twobit_format.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64),
+                                    C.POINTER(C.c_uint64)]
+    L.abw_fasta_base_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.abw_twobit_base_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     L.abw_bam_create.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
     L.abw_bam_feed.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64]
     L.abw_bam_finish.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]

@@ -1,6 +1,7 @@
 // Text parsers on the device (SURVEY.md section 8f: host text parsing is > 80 % of abawaca-build):
 //   SAM    (abw_parse_sam)    -> the abw_read record stream abw_coverage consumes, in file order
-//   FASTA  (abw_fasta_scan)   -> records with their ids and trimmed sequence lines, packed by abw_fasta_pack
+//   FASTA  (abw_fasta_scan)   -> records with their ids and trimmed sequence lines, packed by abw_fasta_pack, counted by abw_fasta_base_counts and
+//                                written back as abawaca prints them by abw_fasta_format (fastaout.cu)
 //   .lrn   (abw_parse_lrn)    -> keys and a row-major matrix of doubles
 //
 // The three share one line index (line_index): newline positions are counted per 4 KB tile and scanned, which gives every line its index, and a
@@ -15,6 +16,7 @@
 //   scafs.find(ref_name)               abawaca-build.cpp:549         (reference name -> scaffold index; unknown names give index 0xFFFFFFFF)
 #include "common.cuh"
 #include "reads.cuh"
+#include "fastaout.cuh"
 #include <algorithm>
 #include <cstring>
 #include <cstdlib>
@@ -310,10 +312,13 @@ __global__ void k_fa_classify(const char* __restrict__ text, uint64_t nbytes, co
 	id_len[l] = idl;
 }
 
-// per line: its record (headers seen so far - 1); header lines publish where the record starts in the running sum of sequence characters
-__global__ void k_fa_records(const uint64_t* __restrict__ line_a, const uint32_t* __restrict__ line_len, const uint32_t* __restrict__ is_header, const uint32_t* __restrict__ id_len,
+// per line: its record (headers seen so far - 1); header lines publish where the record starts in the running sum of sequence characters, and
+// their description: the header after the id and the white space that follows it, up to the trimmed end of the line (SeqIORead_fasta.h:57-76)
+__global__ void k_fa_records(const char* __restrict__ text, uint64_t nbytes, const uint64_t* __restrict__ line_start, const uint64_t* __restrict__ line_a,
+                             const uint32_t* __restrict__ line_len, const uint32_t* __restrict__ is_header, const uint32_t* __restrict__ id_len,
                              const uint64_t* __restrict__ hdr_before, const uint64_t* __restrict__ chars_before, uint64_t nlines, uint64_t nrec,
-                             uint64_t* __restrict__ rec_id_off, uint32_t* __restrict__ rec_id_len, uint64_t* __restrict__ rec_chars0, int* __restrict__ err)
+                             uint64_t* __restrict__ rec_id_off, uint32_t* __restrict__ rec_id_len, uint64_t* __restrict__ rec_chars0,
+                             uint64_t* __restrict__ rec_desc_off, uint32_t* __restrict__ rec_desc_len, int* __restrict__ err)
 {
 	abw_grid_wait();
 	const uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -324,6 +329,13 @@ __global__ void k_fa_records(const uint64_t* __restrict__ line_a, const uint32_t
 		rec_id_off[r] = line_a[l] + 1;
 		rec_id_len[r] = id_len[l];
 		rec_chars0[r] = chars_before[l];
+		uint64_t b = line_extent(line_start, nlines, nbytes, l).b, q = line_a[l] + 1 + id_len[l];
+		while(b > q && dev_isspace(text[b - 1]))
+			b--;
+		while(q < b && dev_isspace(text[q]))
+			q++;
+		rec_desc_off[r] = q;
+		rec_desc_len[r] = (uint32_t)min((uint64_t)0xFFFFFFFFu, b - q);
 	}
 	else if(line_len[l] && hdr_before[l] == 0)
 		atomicOr(err, FA_ERR_NO_HEADER);                  // sequence text before the first header line (:58-62)
@@ -352,6 +364,37 @@ __global__ void __launch_bounds__(256) k_fa_copy(const char* __restrict__ text, 
 	}
 }
 
+
+// one warp per sequence line: N (either case) and C/G (either case) of its characters, added to its record's counts
+__global__ void __launch_bounds__(256) k_fa_base_counts(const char* __restrict__ text, const uint64_t* __restrict__ line_a, const uint32_t* __restrict__ line_len,
+                                                        const uint64_t* __restrict__ hdr_before, uint64_t nlines, unsigned long long* __restrict__ countN,
+                                                        unsigned long long* __restrict__ countGC)
+{
+	abw_grid_wait();
+	const int lane = threadIdx.x & 31;
+	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+	for(uint64_t l = warp0; l < nlines; l += nwarps) {
+		const uint32_t len = line_len[l];
+		if(len == 0)
+			continue;
+		const char* __restrict__ src = text + line_a[l];
+		uint32_t nN = 0, nGC = 0;
+		for(uint32_t i = lane; i < len; i += 32) {
+			const uint32_t c = (unsigned char)src[i] | 0x20u;            // 'N' and 'n' -> 'n', 'C' / 'c' -> 'c', 'G' / 'g' -> 'g'; no other byte maps there
+			nN += c == 'n';
+			nGC += c == 'c' || c == 'g';
+		}
+		nN = __reduce_add_sync(0xffffffffu, nN);
+		nGC = __reduce_add_sync(0xffffffffu, nGC);
+		if(lane == 0) {
+			const uint64_t r = hdr_before[l] - 1;
+			if(nN)
+				atomicAdd(countN + r, (unsigned long long)nN);
+			if(nGC)
+				atomicAdd(countGC + r, (unsigned long long)nGC);
+		}
+	}
+}
 
 // ---------------------------------------------------------------------------------------------------
 // .lrn data lines -> keys and a row-major matrix of doubles (ClusterData::ClusterData, ClusterData.cpp:110-168: one line per datapoint,
@@ -498,11 +541,13 @@ __global__ void __launch_bounds__(256) k_gather_rows(const double* __restrict__ 
 }  // namespace
 
 struct abw_fasta {
-	LineIndex lines;                          // the text; its line starts are released once the lines are classified
+	LineIndex lines;                          // the text; its line starts are released once the records are found
 	uint64_t nrec = 0;
-	DevBuf<uint64_t> line_a, hdr_before, chars_before, rec_id_off, rec_chars0;
-	DevBuf<uint32_t> line_len, rec_id_len;
-	std::vector<uint64_t> h_seq_len;
+	DevBuf<uint64_t> line_a, hdr_before, chars_before, rec_id_off, rec_chars0, rec_desc_off;
+	DevBuf<uint32_t> line_len, rec_id_len, rec_desc_len;
+	// per record: sequence length, and what abw_fasta_format lays the text out with (id, description, first sequence character)
+	std::vector<uint64_t> h_seq_len, h_id_off, h_desc_off, h_chars0;
+	std::vector<uint32_t> h_id_len, h_desc_len;
 };
 
 extern "C" {
@@ -615,7 +660,6 @@ int abw_fasta_scan(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_
 		ABW_CUDA(ctx, f->hdr_before.alloc(nlines));
 		ABW_CUDA(ctx, f->chars_before.alloc(nlines));
 		ABW_LAUNCH(ctx, k_fa_classify, abw_div_up(nlines, 256), 256, 0, li.text, nbytes, li.start.p, nlines, f->line_a.p, f->line_len.p, is_header.p, id_len.p, d_err.p);
-		li.start.release();
 		// hdr_before[l] = header lines strictly before l; a header line itself gets its own record index, a sequence line index + 1 of its record
 		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, is_header.p, f->hdr_before.p, nlines, total.p));
 		ABW_CHECK(abw_exclusive_scan_u32_to_u64(ctx, f->line_len.p, f->chars_before.p, nlines, total.p + 1));
@@ -627,19 +671,32 @@ int abw_fasta_scan(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_
 		ABW_CUDA(ctx, f->rec_id_off.alloc(nrec));
 		ABW_CUDA(ctx, f->rec_id_len.alloc(nrec));
 		ABW_CUDA(ctx, f->rec_chars0.alloc(nrec + 1));
-		ABW_LAUNCH(ctx, k_fa_records, abw_div_up(nlines, 256), 256, 0, f->line_a.p, f->line_len.p, is_header.p, id_len.p, f->hdr_before.p, f->chars_before.p, nlines, nrec,
-		           f->rec_id_off.p, f->rec_id_len.p, f->rec_chars0.p, d_err.p);
+		ABW_CUDA(ctx, f->rec_desc_off.alloc(nrec));
+		ABW_CUDA(ctx, f->rec_desc_len.alloc(nrec));
+		ABW_LAUNCH(ctx, k_fa_records, abw_div_up(nlines, 256), 256, 0, li.text, nbytes, li.start.p, f->line_a.p, f->line_len.p, is_header.p, id_len.p, f->hdr_before.p,
+		           f->chars_before.p, nlines, nrec, f->rec_id_off.p, f->rec_id_len.p, f->rec_chars0.p, f->rec_desc_off.p, f->rec_desc_len.p, d_err.p);
+		li.start.release();
 		ABW_CUDA(ctx, cudaMemcpyAsync(f->rec_chars0.p + nrec, &nchars, sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
 		int h_err = 0;
 		ABW_CUDA(ctx, abw_fetch(ctx, &h_err, d_err.p, sizeof(int)));
-		std::vector<uint64_t> c0(nrec + 1);
-		ABW_CUDA(ctx, abw_fetch(ctx, c0.data(), f->rec_chars0.p, sizeof(uint64_t) * (nrec + 1)));
+		f->h_chars0.resize(nrec + 1);
+		f->h_id_off.resize(nrec);
+		f->h_id_len.resize(nrec);
+		f->h_desc_off.resize(nrec);
+		f->h_desc_len.resize(nrec);
+		ABW_CUDA(ctx, abw_fetch(ctx, f->h_chars0.data(), f->rec_chars0.p, sizeof(uint64_t) * (nrec + 1)));
+		if(nrec) {
+			ABW_CUDA(ctx, abw_fetch(ctx, f->h_id_off.data(), f->rec_id_off.p, sizeof(uint64_t) * nrec));
+			ABW_CUDA(ctx, abw_fetch(ctx, f->h_id_len.data(), f->rec_id_len.p, sizeof(uint32_t) * nrec));
+			ABW_CUDA(ctx, abw_fetch(ctx, f->h_desc_off.data(), f->rec_desc_off.p, sizeof(uint64_t) * nrec));
+			ABW_CUDA(ctx, abw_fetch(ctx, f->h_desc_len.data(), f->rec_desc_len.p, sizeof(uint32_t) * nrec));
+		}
 		ABW_CUDA(ctx, abw_sync(ctx));
 		if(h_err)
 			return abw_fail(ctx, ABW_ERR_ARG, "Bad_file: was expecting a header line for the next sequence in a fasta file but got something else (SeqIORead_fasta.h:58-62)");
 		f->h_seq_len.resize(nrec);
 		for(uint64_t r = 0; r < nrec; r++)
-			f->h_seq_len[r] = c0[r + 1] - c0[r];
+			f->h_seq_len[r] = f->h_chars0[r + 1] - f->h_chars0[r];
 		// from here on a sequence line looks its record up as hdr_before - 1
 		return ABW_OK;
 	}();
@@ -697,6 +754,49 @@ int abw_fasta_pack(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_order, ui
 	}
 	ABW_CUDA(ctx, abw_sync(ctx));      // rec_dst is a local
 	return abw_pack_sequences(ctx, ascii.p, 1, offsets.data(), nout, out);
+}
+
+int abw_fasta_format(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_recs, uint64_t nrecs, uint64_t byte0, char* d_text, uint64_t cap, uint64_t* total_bytes,
+                     uint64_t* nbytes)
+{
+	if(!ctx || !f || !total_bytes || !nbytes || (!h_recs && nrecs))
+		return abw_fail(ctx, ABW_ERR_ARG, "abw_fasta_format: null argument");
+	ABW_ENTER(ctx);
+	*total_bytes = 0;
+	*nbytes = 0;
+	std::vector<FaRecord> recs(nrecs);
+	for(uint64_t i = 0; i < nrecs; i++) {
+		const uint32_t r = h_recs[i];
+		if(r >= f->nrec)
+			return abw_fail(ctx, ABW_ERR_ARG, "abw_fasta_format: record index out of range");
+		recs[i] = FaRecord{f->h_id_off[r], f->h_desc_off[r], f->h_chars0[r], f->h_seq_len[r], 0, 0, f->h_id_len[r], f->h_desc_len[r]};
+	}
+	FaSource src;
+	src.kind = FA_SRC_TEXT;
+	src.text = f->lines.text;
+	src.line_a = f->line_a.p;
+	src.line_len = f->line_len.p;
+	src.chars_before = f->chars_before.p;
+	src.nlines = f->lines.nlines;
+	return abw_fasta_text(ctx, src, recs, byte0, d_text, cap, total_bytes, nbytes);
+}
+
+int abw_fasta_base_counts(abw_ctx* ctx, const abw_fasta* f, uint64_t* h_count_N, uint64_t* h_count_GC)
+{
+	if(!ctx || !f || ((!h_count_N || !h_count_GC) && f->nrec))
+		return abw_fail(ctx, ABW_ERR_ARG, "abw_fasta_base_counts: null argument");
+	ABW_ENTER(ctx);
+	if(f->nrec == 0)
+		return ABW_OK;
+	DevBuf<unsigned long long> counts;
+	ABW_CUDA(ctx, counts.alloc(2 * f->nrec));
+	ABW_CUDA(ctx, cudaMemsetAsync(counts.p, 0, sizeof(unsigned long long) * 2 * f->nrec, ctx->stream));
+	const unsigned int blocks = (unsigned int)std::min<uint64_t>(abw_div_up(f->lines.nlines * 32, 256), (uint64_t)ctx->sm_count * 16);
+	ABW_LAUNCH(ctx, k_fa_base_counts, blocks, 256, 0, f->lines.text, f->line_a.p, f->line_len.p, f->hdr_before.p, f->lines.nlines, counts.p, counts.p + f->nrec);
+	ABW_CUDA(ctx, abw_fetch(ctx, h_count_N, counts.p, sizeof(uint64_t) * f->nrec));
+	ABW_CUDA(ctx, abw_fetch(ctx, h_count_GC, counts.p + f->nrec, sizeof(uint64_t) * f->nrec));
+	ABW_CUDA(ctx, abw_sync(ctx));
+	return ABW_OK;
 }
 
 int abw_parse_lrn(abw_ctx* ctx, const char* text, uint64_t nbytes, int text_on_device, uint32_t D, uint64_t* d_keys, double* d_values, uint64_t cap_rows, uint64_t* nrows)

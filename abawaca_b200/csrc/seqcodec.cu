@@ -1,5 +1,6 @@
 // Assembly in 2 bits per base: abw_pack_2bit decodes UCSC-order codes plus runs of non-ACGT characters into the abw_seqset layout of
-// features.cu (see the comment at its top), and the abw_twobit_* entry points read UCSC .2bit files into that form.
+// features.cu (see the comment at its top), and the abw_twobit_* entry points read UCSC .2bit files into that form, count their bases
+// (k_2bit_base_gc) and write them back as FASTA text (abw_twobit_format, fastaout.cu).
 //
 // Three kernels, in stream order:
 //   k_2bit_decode  one warp per scaffold, 64 bases (16 code bytes) per lane and step: packed words, valid = every position < len, nmask = 0,
@@ -14,6 +15,7 @@
 #include <cstring>
 
 #include "features.cuh"
+#include "fastaout.cuh"
 
 namespace {
 
@@ -168,6 +170,34 @@ __global__ void __launch_bounds__(256) k_2bit_recount(const uint32_t* __restrict
 	}
 }
 
+// One warp per record of a .2bit file: C+G = the C/G codes (UCSC C = 1, G = 3: the low bit) of its bases, less those under its N blocks.
+__global__ void __launch_bounds__(256) k_2bit_base_gc(const uint8_t* __restrict__ file, const uint64_t* __restrict__ dna_off, const uint64_t* __restrict__ len,
+                                                      const uint64_t* __restrict__ nblk0, const uint2* __restrict__ nblocks, uint64_t nrec,
+                                                      unsigned long long* __restrict__ countGC)
+{
+	abw_grid_wait();
+	const int lane = threadIdx.x & 31;
+	const uint64_t warp0 = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+	for(uint64_t r = warp0; r < nrec; r += nwarps) {
+		const uint64_t L = len[r];
+		const uint8_t* __restrict__ dna = file + dna_off[r];
+		int64_t nGC = 0;
+		for(uint64_t i = lane; i < (L + 3) >> 2; i += 32) {
+			const uint32_t keep = (4 * i + 4 <= L)? 0xFFu : (0xFFu << (2 * (4 * i + 4 - L))) & 0xFFu;      // codes of bases past L are padding
+			nGC += __popc((uint32_t)dna[i] & keep & 0x55u);
+		}
+		for(uint64_t k = nblk0[r]; k < nblk0[r + 1]; k++) {
+			const uint2 nb = nblocks[k];
+			for(uint64_t p = (uint64_t)nb.x + lane; p < (uint64_t)nb.x + nb.y; p += 32)
+				nGC -= (dna[p >> 2] >> (6 - 2 * (p & 3))) & 1u;
+		}
+		for(int o = 16; o > 0; o >>= 1)
+			nGC += __shfl_down_sync(0xffffffffu, nGC, o);
+		if(lane == 0)
+			countGC[r] = (unsigned long long)nGC;
+	}
+}
+
 int pack_2bit_impl(abw_ctx* ctx, abw_seqset* s, const abw_2bit_assembly* in, uint32_t nscaf)
 {
 	s->nscaf = nscaf;
@@ -236,6 +266,7 @@ struct abw_twobit {
 	std::vector<uint32_t> name_len;
 	std::vector<uint64_t> nblk0, mblk0;      // [nrec + 1]: the record's blocks in nblocks / mblocks
 	std::vector<Block> nblocks, mblocks;
+	DevBuf<uint2> d_nblocks;                 // nblocks on the device {start, size}, for abw_twobit_format / abw_twobit_base_counts
 };
 
 namespace {
@@ -358,8 +389,19 @@ int abw_twobit_scan(abw_ctx* ctx, const void* h_file, uint64_t nbytes, abw_twobi
 {
 	if(!ctx || !out || (!h_file && nbytes))
 		return abw_fail(ctx, ABW_ERR_ARG, "abw_twobit_scan: null argument");
+	ABW_ENTER(ctx);
 	abw_twobit* t = new abw_twobit();
 	int rc = twobit_scan_impl(ctx, t, (const uint8_t*)h_file, nbytes);
+	if(rc == ABW_OK && !t->nblocks.empty()) {
+		static_assert(sizeof(Block) == sizeof(uint2), "N blocks go to the device as uint2");
+		const cudaError_t e = t->d_nblocks.alloc(t->nblocks.size());
+		if(e == cudaSuccess)
+			rc = abw_upload_small(ctx, t->d_nblocks.p, t->nblocks.data(), sizeof(Block) * t->nblocks.size()) == cudaSuccess? ABW_OK : ABW_ERR_CUDA;
+		else
+			rc = ABW_ERR_CUDA;
+		if(rc != ABW_OK)
+			abw_fail(ctx, rc, "abw_twobit_scan: could not copy the N blocks to the device");
+	}
 	if(rc != ABW_OK) {
 		delete t;
 		return rc;
@@ -456,6 +498,62 @@ int abw_twobit_pack(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint6
 		return rc;
 	}
 	*out = s;
+	return ABW_OK;
+}
+
+int abw_twobit_format(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, const uint32_t* h_recs, uint64_t nrecs, uint64_t byte0, char* d_text,
+                      uint64_t cap, uint64_t* total_bytes, uint64_t* nbytes)
+{
+	if(!ctx || !t || !total_bytes || !nbytes || (!h_recs && nrecs) || (!d_file && t->nbytes))
+		return abw_fail(ctx, ABW_ERR_ARG, "abw_twobit_format: null argument");
+	ABW_ENTER(ctx);
+	*total_bytes = 0;
+	*nbytes = 0;
+	const uint64_t nrec = t->seq_len.size();
+	std::vector<FaRecord> recs(nrecs);
+	for(uint64_t i = 0; i < nrecs; i++) {
+		const uint32_t r = h_recs[i];
+		if(r >= nrec)
+			return abw_fail(ctx, ABW_ERR_ARG, "abw_twobit_format: record index out of range");
+		recs[i] = FaRecord{t->name_off[r], 0, t->dna_off[r], t->seq_len[r], t->nblk0[r], t->nblk0[r + 1], t->name_len[r], 0};
+	}
+	ABW_CHECK(abw_wait_h2d(ctx, h2d_ticket));                      // on the device: the file image may still be on its way
+	FaSource src;
+	src.kind = FA_SRC_2BIT;
+	src.text = (const char*)d_file;
+	src.nblocks = t->d_nblocks.p;
+	return abw_fasta_text(ctx, src, recs, byte0, d_text, cap, total_bytes, nbytes);
+}
+
+int abw_twobit_base_counts(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, uint64_t* h_count_N, uint64_t* h_count_GC)
+{
+	const uint64_t nrec = t? t->seq_len.size() : 0;
+	if(!ctx || !t || ((!h_count_N || !h_count_GC) && nrec) || (!d_file && t->nbytes))
+		return abw_fail(ctx, ABW_ERR_ARG, "abw_twobit_base_counts: null argument");
+	ABW_ENTER(ctx);
+	ABW_CHECK(abw_wait_h2d(ctx, h2d_ticket));
+	if(nrec == 0)
+		return ABW_OK;
+	DevBuf<uint64_t> d_off, d_len, d_blk0;
+	DevBuf<unsigned long long> d_gc;
+	ABW_CUDA(ctx, d_off.alloc(nrec));
+	ABW_CUDA(ctx, d_len.alloc(nrec));
+	ABW_CUDA(ctx, d_blk0.alloc(nrec + 1));
+	ABW_CUDA(ctx, d_gc.alloc(nrec));
+	ABW_CUDA(ctx, abw_upload_small(ctx, d_off.p, t->dna_off.data(), sizeof(uint64_t) * nrec));
+	ABW_CUDA(ctx, abw_upload_small(ctx, d_len.p, t->seq_len.data(), sizeof(uint64_t) * nrec));
+	ABW_CUDA(ctx, abw_upload_small(ctx, d_blk0.p, t->nblk0.data(), sizeof(uint64_t) * (nrec + 1)));
+	const unsigned int blocks = (unsigned int)std::min<uint64_t>(abw_div_up(nrec * 32, 256), (uint64_t)ctx->sm_count * 16);
+	ABW_LAUNCH(ctx, k_2bit_base_gc, blocks, 256, 0, (const uint8_t*)d_file, d_off.p, d_len.p, d_blk0.p, t->d_nblocks.p, nrec, d_gc.p);
+	ABW_CUDA(ctx, abw_fetch(ctx, h_count_GC, d_gc.p, sizeof(uint64_t) * nrec));
+	ABW_CUDA(ctx, abw_sync(ctx));
+	// N: the sizes of the N blocks, a mask over them or not
+	for(uint64_t r = 0; r < nrec; r++) {
+		uint64_t n = 0;
+		for(uint64_t k = t->nblk0[r]; k < t->nblk0[r + 1]; k++)
+			n += t->nblocks[k].size;
+		h_count_N[r] = n;
+	}
 	return ABW_OK;
 }
 

@@ -4,7 +4,8 @@
 // The loaders below rebuild what ScafDpData (ScafDpData.cpp:11-120), ClusterData (ClusterData.cpp:27-168) and SCGdb
 // (SCGdb.cpp:58-120) build, as flat arrays; the writers reproduce log, summary.txt, dp2cluster.txt, scaf2cluster.txt,
 // final-clusters/<id>.fasta and clusters/<id>.{lrn,scaf-cluster.txt,scaf-stats.txt} from the records the device returns; the data lines of
-// clusters/<id>.lrn are printed on the device (abw_format_lrn).
+// clusters/<id>.lrn (abw_format_lrn) and the text of final-clusters/<id>.fasta (abw_fasta_format / abw_twobit_format) are made on the device, where the
+// assembly stays from loading to the last bin.
 #include "abw_host.h"
 #include <algorithm>
 #include <cmath>
@@ -124,7 +125,7 @@ static int read_params(Params& P, int argc, const char** argv)
 struct Model {
 	// scaffolds (1-based ids = index + 1, name order) and datapoints (1-based ids, (scaffold, dp name) order)
 	std::vector<std::string> scaf_names;
-	std::vector<const FastaRecord*> scaf_seq;
+	std::vector<uint32_t> scaf_rec;             // record of the scaffold in the assembly file
 	std::vector<double> scaf_cvg, scaf_gc;
 	std::vector<uint32_t> T;
 	std::vector<uint64_t> len;
@@ -137,7 +138,10 @@ struct Model {
 	std::vector<uint64_t> scgmask;              // [S][W]
 	uint32_t W = 1;
 	int total_num_scgs = 0;
-	std::vector<FastaRecord> fasta;
+	// the assembly on the device: FASTA text indexed by abw_fasta_scan, or a .2bit image (d_file) parsed by abw_twobit_scan
+	abw_fasta* fa = nullptr;
+	abw_twobit* tb = nullptr;
+	void* d_file = nullptr;
 	size_t N() const { return dp2scaf.size(); }
 	size_t S() const { return scaf_names.size(); }
 	size_t D() const { return dim_names.size(); }
@@ -201,40 +205,49 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 			dp_name2id[dpn] = M.dp2scaf.size();
 		}
 	}
-	// assembly
+	// assembly: read once, kept on the device for the bin files
 	{
 		std::string bytes = read_file(P.fasta_file);
-		if(is_twobit(bytes))
-			M.fasta = read_twobit(ctx, P.fasta_file, bytes);
+		const bool twobit = is_twobit(bytes);
+		if(twobit? abw_twobit_scan(ctx, bytes.data(), bytes.size(), &M.tb) != ABW_OK : abw_fasta_scan(ctx, bytes.data(), bytes.size(), 0, &M.fa) != ABW_OK)
+			throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + P.fasta_file + ")");
+		if(twobit) {
+			ABWH_CHECK(ctx, abw_device_alloc(ctx, std::max<size_t>(bytes.size(), 1), &M.d_file));
+			ABWH_CHECK(ctx, abw_copy_to_device(ctx, M.d_file, bytes.data(), bytes.size()));
+		}
+		const uint64_t nrec = twobit? abw_twobit_count(M.tb) : abw_fasta_count(M.fa);
+		std::vector<uint64_t> id_off(nrec), rec_len(nrec), count_N(nrec), count_GC(nrec);
+		std::vector<uint32_t> id_len(nrec);
+		if(twobit) {
+			ABWH_CHECK(ctx, abw_twobit_get(ctx, M.tb, id_off.data(), id_len.data(), rec_len.data()));
+			ABWH_CHECK(ctx, abw_twobit_base_counts(ctx, M.tb, M.d_file, 0, count_N.data(), count_GC.data()));
+		}
 		else {
-			std::string().swap(bytes);
-			M.fasta = read_fasta(P.fasta_file);
+			ABWH_CHECK(ctx, abw_fasta_get(ctx, M.fa, id_off.data(), id_len.data(), rec_len.data()));
+			ABWH_CHECK(ctx, abw_fasta_base_counts(ctx, M.fa, count_N.data(), count_GC.data()));
 		}
-	}
-	M.scaf_seq.assign(M.S(), nullptr);
-	M.scaf_cvg.assign(M.S(), 0);
-	for(auto& r : M.fasta) {
-		auto it = scaf_name2id.find(r.id);
-		if(it != scaf_name2id.end()) {                 // a repeated id overwrites the earlier record (scafs[id] = Seq(...), ScafDpData.cpp:110)
-			M.scaf_seq[it->second - 1] = &r;
-			auto ci = name2cvg.find(r.id);
-			M.scaf_cvg[it->second - 1] = (ci == name2cvg.end())? 0 : ci->second;
+		const uint32_t none = 0xFFFFFFFFu;
+		M.scaf_rec.assign(M.S(), none);
+		M.scaf_cvg.assign(M.S(), 0);
+		for(uint64_t i = 0; i < nrec; i++) {
+			const std::string id = bytes.substr(id_off[i], id_len[i]);
+			auto it = scaf_name2id.find(id);
+			if(it != scaf_name2id.end()) {                 // a repeated id overwrites the earlier record (scafs[id] = Seq(...), ScafDpData.cpp:110)
+				M.scaf_rec[it->second - 1] = (uint32_t)i;
+				auto ci = name2cvg.find(id);
+				M.scaf_cvg[it->second - 1] = (ci == name2cvg.end())? 0 : ci->second;
+			}
 		}
-	}
-	M.len.resize(M.S());
-	M.scaf_gc.resize(M.S());
-	for(size_t s = 0; s < M.S(); s++) {
-		if(!M.scaf_seq[s])
-			throw std::invalid_argument("scaffold " + M.scaf_names[s] + " is not in " + P.fasta_file);
-		const std::string& q = M.scaf_seq[s]->seq;
-		M.len[s] = q.size();
-		size_t gc = 0, Ns = 0;                      // Bio::gc after DNAString upper-casing (String.cpp:114-131)
-		for(char ch : q) {
-			char u = (char)toupper((unsigned char)ch);
-			if(u == 'N') Ns++;
-			else if(u == 'C' || u == 'G') gc++;
+		M.len.resize(M.S());
+		M.scaf_gc.resize(M.S());
+		for(size_t s = 0; s < M.S(); s++) {
+			const uint32_t r = M.scaf_rec[s];
+			if(r == none)
+				throw std::invalid_argument("scaffold " + M.scaf_names[s] + " is not in " + P.fasta_file);
+			M.len[s] = rec_len[r];
+			// Bio::gc after DNAString upper-casing (String.cpp:114-131)
+			M.scaf_gc[s] = (rec_len[r] == count_N[r])? 0 : (double)count_GC[r] / (double)(rec_len[r] - count_N[r]);
 		}
-		M.scaf_gc[s] = (q.size() == Ns)? 0 : (double)gc / (double)(q.size() - Ns);
 	}
 	// .lrn (ClusterData.cpp:27-168)
 	{
@@ -345,6 +358,26 @@ static void load_model(const Params& P, Model& M, abw_ctx* ctx)
 	}
 }
 
+// The FASTA text of the assembly records `recs` (abw_fasta_format / abw_twobit_format) in windows of LRN_CHUNK bytes: d_text (LRN_CHUNK bytes of device
+// memory) and text are scratch, kept from file to file.  false when fp takes fewer bytes than it is given.
+static bool write_fasta(abw_ctx* ctx, FILE* fp, const Model& M, const std::vector<uint32_t>& recs, char* d_text, std::vector<char>& text)
+{
+	for(uint64_t byte0 = 0, total = 1; byte0 < total;) {
+		uint64_t nbytes = 0;
+		if(M.tb)
+			ABWH_CHECK(ctx, abw_twobit_format(ctx, M.tb, M.d_file, 0, recs.data(), recs.size(), byte0, d_text, LRN_CHUNK, &total, &nbytes));
+		else
+			ABWH_CHECK(ctx, abw_fasta_format(ctx, M.fa, recs.data(), recs.size(), byte0, d_text, LRN_CHUNK, &total, &nbytes));
+		text.resize(std::max<size_t>(text.size(), nbytes));
+		if(nbytes)
+			ABWH_CHECK(ctx, abw_copy_to_host(ctx, text.data(), d_text, nbytes));
+		if(fwrite(text.data(), 1, nbytes, fp) != nbytes)
+			return false;
+		byte0 += nbytes;
+	}
+	return true;
+}
+
 // size-weighted mean and standard deviation in scaffold-id order (ClusterQuality.cpp:6-27)
 static void weighted_stats(const std::vector<std::pair<size_t, double>>& data, double& mean, double& stdev)
 {
@@ -409,11 +442,12 @@ int main(int argc, const char** argv)
 		std::map<uint32_t, std::vector<uint32_t>> dps_of;      // 0-based datapoints, ascending
 		for(size_t i = 0; i < N; i++)
 			for(uint32_t c = dp2cluster[i]; c != 0; c = parent_of[c]) dps_of[c].push_back((uint32_t)i);
-		// scratch of the cluster dumps (write_lrn)
+		// scratch of the cluster dumps (write_lrn) and the bin files (write_fasta)
 		char* d_text = nullptr;
 		ABWH_CHECK(ctx, abw_device_alloc(ctx, LRN_CHUNK, (void**)&d_text));
 		std::vector<char> text;
 		std::vector<uint64_t> rows;
+		std::vector<uint32_t> recs_of_bin;
 		auto gc_cvg_of = [&](const std::vector<uint32_t>& assigned, double& avg_gc, double& sd_gc, double& avg_cvg, double& sd_cvg) {
 			std::vector<std::pair<size_t, double>> gc, cvg;
 			for(uint32_t s : assigned) {
@@ -445,17 +479,18 @@ int main(int argc, const char** argv)
 				std::cerr << '[' << get_time() << ']' << " Cluster " << r.id << " is a terminal cluster" << std::endl;
 				log << '[' << get_time() << ']' << " Cluster " << r.id << " is a terminal cluster" << std::endl;
 				const std::vector<uint32_t>& assigned = assigned_of[r.id];
-				// final-clusters/<id>.fasta: 60 columns, one more (possibly empty) line when the length is a multiple of 60 (SeqIOWrite_fasta.h:40-51)
+				// final-clusters/<id>.fasta: 60 columns, one more (possibly empty) line when the length is a multiple of 60 (SeqIOWrite_fasta.h:40-51),
+				// made on the device in windows of the dump scratch
 				{
-					std::ofstream fa((P.fasta_dir + "/" + std::to_string(r.id) + ".fasta").c_str());
-					for(uint32_t s : assigned) {
-						const FastaRecord& q = *M.scaf_seq[s];
-						std::string up = q.seq;
-						for(char& ch : up) ch = (char)toupper((unsigned char)ch);
-						fa << '>' << q.id << ' ' << q.desc << std::endl;
-						for(size_t i = 0; i <= up.size(); i += 60)
-							fa << up.substr(i, 60) << std::endl;
+					const std::string path = P.fasta_dir + "/" + std::to_string(r.id) + ".fasta";
+					FILE* fp = fopen(path.c_str(), "w");
+					recs_of_bin.clear();
+					for(uint32_t s : assigned) recs_of_bin.push_back(M.scaf_rec[s]);
+					if(!fp || !write_fasta(ctx, fp, M, recs_of_bin, d_text, text)) {
+						std::cerr << "Fatal error: could write to file " << path << std::endl << std::endl;
+						exit(-1);
 					}
+					fclose(fp);
 				}
 				// ClusterQuality::scg, gc and cvg of the bin come back with its record (gc and cvg: abw_search_set_scaffold_stats)
 				summary << r.id << '\t' << assigned.size() << '\t' << cur_dps.size() << '\t' << r.total_size << '\t' << int(1000 * r.gc_avg) / 10.0 << '\t' << int(1000 * r.gc_sd) / 100.0
@@ -533,6 +568,10 @@ int main(int argc, const char** argv)
 		ABWH_CHECK(ctx, abw_device_free(ctx, d_text));
 		abw_search_destroy(search);
 		ABWH_CHECK(ctx, abw_device_free(ctx, M.d_rows));
+		abw_fasta_destroy(M.fa);
+		abw_twobit_destroy(M.tb);
+		if(M.d_file)
+			ABWH_CHECK(ctx, abw_device_free(ctx, M.d_file));
 		milestone("logs, fasta and cluster dumps");
 		// dp2cluster.txt has a row for dp 0 as well (abawaca.cpp:199, quirk Q10)
 		ofs_dp << 0 << "\t0" << std::endl;

@@ -19,54 +19,6 @@
 
 namespace abwh {
 
-struct FastaRecord { std::string id, desc, seq; };
-
-// FASTA as SeqIORead_fasta<DNASequence>::next_seq reads it (SeqIORead_fasta.h:51-103): blank lines skipped, id = first token after
-// '>', the rest of the header is the description, sequence lines trimmed on both sides and concatenated.
-inline std::vector<FastaRecord> read_fasta(const std::string& path)
-{
-	FILE* fp = fopen(path.c_str(), "r");
-	if(!fp)
-		throw std::runtime_error("Failed to open file " + path);
-	std::vector<FastaRecord> out;
-	char* line = nullptr;
-	size_t cap = 0;
-	ssize_t n;
-	while((n = getline(&line, &cap, fp)) >= 0) {
-		char *b = line, *e = line + n;
-		while(b < e && isspace((unsigned char)*b)) b++;
-		while(e > b && isspace((unsigned char)e[-1])) e--;
-		if(b == e)
-			continue;
-		if(*b == '>') {
-			FastaRecord r;
-			char* p = b + 1;
-			char* q = p;
-			while(q < e && !isspace((unsigned char)*q)) q++;
-			r.id.assign(p, q);
-			while(q < e && isspace((unsigned char)*q)) q++;
-			r.desc.assign(q, e);
-			if(r.id.empty()) {
-				free(line);
-				fclose(fp);
-				throw std::runtime_error("Was expecting a header line for the next sequence in fasta file " + path);
-			}
-			out.push_back(r);
-		}
-		else {
-			if(out.empty()) {
-				free(line);
-				fclose(fp);
-				throw std::runtime_error("Was expecting a header line for the next sequence in fasta file " + path);
-			}
-			out.back().seq.append(b, e);
-		}
-	}
-	free(line);
-	fclose(fp);
-	return out;
-}
-
 inline std::string read_file(const std::string& path)
 {
 	std::string text;
@@ -92,28 +44,6 @@ inline bool is_twobit(const std::string& bytes)
 		return false;
 	const unsigned char* b = (const unsigned char*)bytes.data();
 	return (b[0] == 0x43 && b[1] == 0x27 && b[2] == 0x41 && b[3] == 0x1A) || (b[0] == 0x1A && b[1] == 0x41 && b[2] == 0x27 && b[3] == 0x43);
-}
-
-// the records of a .2bit file as twoBitToFa prints them (abw_twobit_scan / _get / _decode), with an empty description
-inline std::vector<FastaRecord> read_twobit(abw_ctx* ctx, const std::string& path, const std::string& bytes)
-{
-	abw_twobit* t = nullptr;
-	if(abw_twobit_scan(ctx, bytes.data(), bytes.size(), &t) != ABW_OK)
-		throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + path + ")");
-	const uint64_t n = abw_twobit_count(t);
-	std::vector<uint64_t> name_off(n), len(n);
-	std::vector<uint32_t> name_len(n);
-	std::vector<FastaRecord> out(n);
-	int rc = abw_twobit_get(ctx, t, name_off.data(), name_len.data(), len.data());
-	for(uint64_t i = 0; i < n && rc == ABW_OK; i++) {
-		out[i].id = bytes.substr(name_off[i], name_len[i]);
-		out[i].seq.resize(len[i]);
-		rc = abw_twobit_decode(ctx, t, i, bytes.data(), &out[i].seq[0]);
-	}
-	abw_twobit_destroy(t);
-	if(rc != ABW_OK)
-		throw std::runtime_error(std::string(abw_last_error(ctx)) + " (" + path + ")");
-	return out;
 }
 
 // a BAM file starts with a BGZF block header (gzip magic 1f 8b); no SAM file starts with byte 0x1F.  Leaves the file at its start.

@@ -194,6 +194,90 @@ def twobit_to_seqset(ctx, data):
         L.abw_twobit_destroy(t)
 
 
+def is_twobit(data) -> bool:
+    """a UCSC .2bit file starts with the signature 0x1A412743 in the byte order of the file"""
+    return bytes(data[:4]) in (b"\x43\x27\x41\x1A", b"\x1A\x41\x27\x43")
+
+
+class AssemblyFile:
+    """An assembly file held on the device for the FASTA writer and the base counts: FASTA text indexed by abw_fasta_scan, or a UCSC .2bit image
+    (told apart by its signature) parsed by abw_twobit_scan and copied to the device as it is.  d_text: the FASTA text is already in device memory
+    there (data is its host copy, which only gives the ids); it must stay alive until close()."""
+
+    def __init__(self, ctx, data, d_text=None):
+        self.ctx, self.data = ctx, data
+        L = ctx.lib
+        arr, p = _host_bytes(data)
+        self.twobit = is_twobit(arr)
+        self.h = C.c_void_p()
+        self.d_file = None
+        if self.twobit:
+            ctx.check(L.abw_twobit_scan(ctx.h, p, arr.size, C.byref(self.h)))
+            self.d_file = ctx.alloc(max(arr.size, 1))
+            ctx.to_device(self.d_file, arr)
+            self.count = int(L.abw_twobit_count(self.h))
+        else:
+            ctx.check(L.abw_fasta_scan(ctx.h, p if d_text is None else C.c_void_p(d_text), arr.size, 0 if d_text is None else 1, C.byref(self.h)))
+            self.count = int(L.abw_fasta_count(self.h))
+
+    def records(self):
+        """(ids as bytes, sequence lengths) per record in file order"""
+        off, idl, sl = np.zeros(self.count, np.uint64), np.zeros(self.count, np.uint32), np.zeros(self.count, np.uint64)
+        get = self.ctx.lib.abw_twobit_get if self.twobit else self.ctx.lib.abw_fasta_get
+        self.ctx.check(get(self.ctx.h, self.h, capi._p(off), capi._p(idl), capi._p(sl)))
+        return [bytes(self.data[int(a):int(a) + int(n)]) for a, n in zip(off, idl)], sl
+
+    def format_window(self, recs, byte0, d_text, cap):
+        """abw_*_format of the records `recs` (uint32 array): bytes [byte0, byte0 + cap) of their FASTA text to d_text -> (total bytes, bytes written)"""
+        total, n = C.c_uint64(), C.c_uint64()
+        L, ctx = self.ctx.lib, self.ctx
+        pr = capi._p(recs) if recs.size else None
+        if self.twobit:
+            ctx.check(L.abw_twobit_format(ctx.h, self.h, C.c_void_p(self.d_file), 0, pr, recs.size, byte0, C.c_void_p(d_text), cap, C.byref(total), C.byref(n)))
+        else:
+            ctx.check(L.abw_fasta_format(ctx.h, self.h, pr, recs.size, byte0, C.c_void_p(d_text), cap, C.byref(total), C.byref(n)))
+        return int(total.value), int(n.value)
+
+    def close(self):
+        if self.h:
+            (self.ctx.lib.abw_twobit_destroy if self.twobit else self.ctx.lib.abw_fasta_destroy)(self.h)
+            self.h = None
+        if self.d_file is not None:
+            self.ctx.free(self.d_file)
+            self.d_file = None
+
+
+def format_fasta(ctx, asm: AssemblyFile, recs, cap=64 << 20) -> bytes:
+    """The FASTA text abawaca writes for the records `recs` (file-order indices, in list order) of an AssemblyFile, made on the device in windows of
+    at most `cap` bytes (abw_fasta_format / abw_twobit_format) and concatenated."""
+    recs = np.ascontiguousarray(recs, dtype=np.uint32)
+    d_text = ctx.alloc(max(cap, 1))
+    out, byte0 = [], 0
+    try:
+        while True:                  # at least one call, so that an empty list goes through the library too
+            total, n = asm.format_window(recs, byte0, d_text, cap)
+            buf = np.empty(n, dtype=np.uint8)
+            if n:
+                ctx.to_host(buf, d_text)
+            out.append(buf.tobytes())
+            byte0 += n
+            if byte0 >= total:
+                break
+    finally:
+        ctx.free(d_text)
+    return b"".join(out)
+
+
+def base_counts(ctx, asm: AssemblyFile):
+    """(N, C+G) per record of an AssemblyFile in file order, uint64 arrays, after upper-casing (abw_fasta_base_counts / abw_twobit_base_counts)"""
+    cn, cgc = np.zeros(max(asm.count, 1), np.uint64), np.zeros(max(asm.count, 1), np.uint64)
+    if asm.twobit:
+        ctx.check(ctx.lib.abw_twobit_base_counts(ctx.h, asm.h, C.c_void_p(asm.d_file), 0, capi._p(cn), capi._p(cgc)))
+    else:
+        ctx.check(ctx.lib.abw_fasta_base_counts(ctx.h, asm.h, capi._p(cn), capi._p(cgc)))
+    return cn[:asm.count], cgc[:asm.count]
+
+
 class PackedAssembly:
     """An assembly in 2 bits per base (abw_2bit_assembly): UCSC-order codes with every scaffold starting at a byte of its own, plus runs of the
     characters that are not A/C/G/T (capi.BASE_RUN_DTYPE, kind BASE_N for 'N', BASE_OTHER for the rest)."""

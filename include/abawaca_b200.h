@@ -272,6 +272,27 @@ int      abw_twobit_get(abw_ctx* ctx, const abw_twobit* t, uint64_t* h_name_off,
 int      abw_twobit_decode(abw_ctx* ctx, const abw_twobit* t, uint64_t record, const void* h_file, char* h_out);
 int      abw_twobit_pack(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, const uint32_t* h_order, uint32_t nout, abw_seqset** out);
 
+/* ---- records -> FASTA text on the device (abawaca's final-clusters/<id>.fasta) ------------------------------------------------------
+ * Replaces SeqIOWrite_fasta as abawaca uses it (abawaca.cpp:141-142).  The text of the records h_recs[0 .. nrecs) (file-order indices, in list order,
+ * a record may be listed more than once) is, per record, the header '>' id ' ' desc '\n' and the sequence upper-cased byte by byte as the C locale's
+ * toupper does (only a-z change), in lines of 60 characters: floor(L / 60) + 1 lines, the last holding L % 60 characters (an empty line when L is a
+ * multiple of 60, or 0).  FASTA: id as abw_fasta_get has it, desc the rest of the header line after the white space that follows the id, trimmed at
+ * its end (interior white space kept); the sequence as abw_fasta_pack reads it (interior white space of sequence lines kept, other bytes unchanged).
+ * .2bit: desc is empty (the header ends "id \n"); the codes as TCAG, N blocks as 'N', mask blocks ignored.
+ * Records can be far larger than any buffer, so the text is cut at a byte offset: the call writes bytes [byte0, min(byte0 + cap, total)) to d_text
+ * (device memory, any byte address), sets *total_bytes to the size of the whole text and *nbytes to the bytes written; nothing is written when
+ * byte0 >= total.  A record index >= the record count gives ABW_ERR_ARG.  There is no illegal-DNA check (a lower-case 'n' is written as 'N').  One
+ * wait on the host per call; abw_twobit_format waits for h2d_ticket on the device, d_file being the file image abw_twobit_pack takes. */
+int abw_fasta_format(abw_ctx* ctx, const abw_fasta* f, const uint32_t* h_recs, uint64_t nrecs, uint64_t byte0, char* d_text, uint64_t cap, uint64_t* total_bytes,
+                     uint64_t* nbytes);
+int abw_twobit_format(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, const uint32_t* h_recs, uint64_t nrecs, uint64_t byte0, char* d_text,
+                      uint64_t cap, uint64_t* total_bytes, uint64_t* nbytes);
+/* Per record in file order, host arrays [count]: the N and the C+G count of its sequence after upper-casing ('N' / 'n'; 'C', 'c', 'G', 'g'), what
+ * abawaca computes %G+C from (abawaca.cpp:231-237).  Unlike abw_*_pack followed by abw_seqset_stats there is no illegal-DNA check, so a lower-case
+ * 'n' counts as N.  .2bit: N = the sizes of the N blocks, C+G = the C/G codes outside them. */
+int abw_fasta_base_counts(abw_ctx* ctx, const abw_fasta* f, uint64_t* h_count_N, uint64_t* h_count_GC);
+int abw_twobit_base_counts(abw_ctx* ctx, const abw_twobit* t, const void* d_file, uint64_t h2d_ticket, uint64_t* h_count_N, uint64_t* h_count_GC);
+
 /* ---- .lrn data lines -> matrix on the device ---------------------------------------------------------------------------------
  * Replaces the datapoint loop of ClusterData::ClusterData (ClusterData.cpp:110-168) for the text after the four header lines: every line that is
  * not empty and does not start with '%' is "<key>\t<v1>\t...\t<vD>"; keys are read with atoi, values with atof (:151,159).  Row r of the
